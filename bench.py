@@ -31,6 +31,11 @@ cpu_baseline  the oracle (CPU restatement of the reference, PyTorch-CPU fp32) on
 
     --image-size 608 --batch 32    BASELINE.json configs[3] (19x19 grid) instead of the headline 416 / 64
     --no-graph                     eager launches (for ncu launch lists);  --no-cpu-baseline skips the CPU leg
+    --dump-outputs DIR             after the K timed steps, write what the last one computed (rank 0, --precision mode) as
+                                   DIR/<name>.npy: infer -> net, boxes, scores, keep_idx, keep_count (what Yolo2Engine.infer
+                                   returns); train -> loss_terms (what Yolo2Trainer.step returns) and params_strided (every
+                                   k-th weight after the update).  Inputs and weights are seeded, so the same arguments give
+                                   the same inputs on every run and two builds can be compared output for output.
 """
 import argparse
 import json
@@ -106,6 +111,39 @@ def load_peaks():
         return dict(burst=d.get('bf16_tflops', 1590.0), sustained=d.get('bf16_tflops_sustained', 1400.0),
                     hbm=d.get('hbm_gbs', 6650.0), which='measured (MEASURED_PEAKS.json)')
     return dict(burst=1590.0, sustained=1400.0, hbm=6650.0, which='fallback (B200_PROFILING.md)')
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, batch_major=True):
+    """Write arrays as out_dir/<name>.npy: floating ones as float32, integer ones as float64 (exact for int32).  When
+    batch-major arrays together exceed DUMP_LIMIT_BYTES, the same seeded sample of images (rows of axis 0) is kept from
+    each, and its row numbers are written as sampled_rows.npy."""
+    import numpy as np
+    arrays = {k: a.astype(np.float32 if np.issubdtype(a.dtype, np.floating) else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if batch_major and total > DUMP_LIMIT_BYTES:
+        n = next(iter(arrays.values())).shape[0]
+        keep = max(1, n * DUMP_LIMIT_BYTES // (total + 8 * n))
+        rows = np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays['sampled_rows'] = rows.astype(np.float64)
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
+def engine_outputs(eng):
+    """What Yolo2Engine.infer() hands its caller, as numpy.  Slots of keep_idx past keep_count still hold what an earlier
+    step left there, so they are written as -1."""
+    import numpy as np
+    out = {k: t.cpu().numpy() for k, t in dict(net=eng.net_out, boxes=eng.boxes, scores=eng.scores, keep_idx=eng.keep_idx,
+                                                keep_count=eng.keep_count).items()}
+    slot = np.arange(out['keep_idx'].shape[-1])
+    out['keep_idx'] = np.where(slot < out['keep_count'][..., None], out['keep_idx'], -1)
+    return out
 
 
 class ClockSampler:
@@ -274,6 +312,8 @@ def measure_mode(precision, args, world, rank, dev, dist, sampler_index):
     ms_per_step = t_ms / args.steps
     cand = int((eng.scores > 0).sum().item())
     kept = int(eng.keep_count.sum().item())
+    if args.dump_outputs and rank == 0 and precision == args.precision:
+        dump_outputs(args.dump_outputs, engine_outputs(eng))
 
     # ---- e2e: pinned host uint8 -> H2D -> step -> D2H (keep lists + boxes of the batch) ----
     res_host = dict(keep_idx=torch.empty(eng.keep_idx.shape, dtype=torch.int32).pin_memory(),
@@ -567,6 +607,11 @@ def run_train(args):
     t_ms = allmax(sum(a.elapsed_time(b) for a, b in evs))
     ms_per_step = t_ms / args.steps
     value = world * N * args.steps / (t_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        params = tr.params.cpu().numpy()
+        stride = -(-params.size // (4 << 20))                 # at most 4 Mi weights (16 MiB)
+        dump_outputs(args.dump_outputs, dict(loss_terms=tr.terms.cpu().numpy(), params_strided=params[::stride]),
+                     batch_major=False)
 
     # ---- e2e: pinned host images (+ labels) -> H2D -> step -> D2H of the five loss terms, every step ----
     terms_host = torch.empty((5,), dtype=torch.float32).pin_memory()
@@ -699,7 +744,13 @@ def main():
     ap.add_argument('--no-graph', action='store_true', help='eager launches (for ncu launch lists)')
     ap.add_argument('--image-size', type=int, default=None, help='416 (headline, BASELINE configs[1]) or 608 (configs[3])')
     ap.add_argument('--batch', type=int, default=None, help='images per GPU (default 64; configs[3] uses 32 at 608)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, <= 64 MiB in all)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours)')
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     global IMAGE_SIZE, BATCH_PER_GPU
     if args.image_size:
         IMAGE_SIZE = args.image_size

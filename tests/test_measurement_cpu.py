@@ -39,6 +39,35 @@ def test_bench_config_follows_image_size(bench):
     assert cfg['image_size'] == 608 and cfg['global_batch'] == 32 and '608x608' in cfg['workload'] and 'configs[3]' in cfg['workload']
 
 
+def test_dump_outputs_dtypes_and_size_cap(bench, tmp_path, monkeypatch):
+    """--dump-outputs: float arrays as float32, integer ones as float64; past the cap the same seeded rows of every array."""
+    import numpy as np
+    import torch
+    eng = type('Eng', (), {})()
+    eng.net_out = torch.randn(6, 2, 2, 25)
+    eng.boxes, eng.scores = torch.rand(6, 20, 4), torch.rand(6, 20, 20)
+    eng.keep_idx = torch.randint(0, 20, (6, 20, 4), dtype=torch.int32)
+    eng.keep_count = torch.randint(-1, 6, (6, 20), dtype=torch.int32)
+    out = bench.engine_outputs(eng)
+    kc = eng.keep_count.numpy()
+    for j in range(4):
+        assert np.array_equal(out['keep_idx'][..., j] == -1, kc <= j)
+    bench.dump_outputs(str(tmp_path / 'all'), out)
+    got = {k: np.load(str(tmp_path / 'all' / (k + '.npy'))) for k in out}
+    assert got['net'].dtype == np.float32 and got['keep_idx'].dtype == np.float64
+    assert np.array_equal(got['net'], eng.net_out.numpy()) and np.array_equal(got['keep_count'], kc)
+    monkeypatch.setattr(bench, 'DUMP_LIMIT_BYTES', 10000)     # 18720 bytes in all
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), out)
+    files = sorted(os.listdir(str(tmp_path / 'a')))
+    assert files == sorted(k + '.npy' for k in list(out) + ['sampled_rows']) and files == sorted(os.listdir(str(tmp_path / 'b')))
+    rows = np.load(str(tmp_path / 'a' / 'sampled_rows.npy')).astype(int)
+    assert 0 < len(rows) < 6 and sum(os.path.getsize(str(tmp_path / 'a' / f)) - 128 for f in files) <= 10000
+    for f in files:
+        assert np.array_equal(np.load(str(tmp_path / 'a' / f)), np.load(str(tmp_path / 'b' / f)))
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'scores.npy')), eng.scores.numpy()[rows])
+
+
 def test_launch_list_condenser(tmp_path):
     """tools/ncu_launch_list.py: one step = flush memset .. next flush memset; conv DRAM bytes and share of the step."""
     hdr = '"ID","Process ID","Process Name","Host Name","Kernel Name","Context","Stream","Block Size","Grid Size","Device","CC","Section Name","Metric Name","Metric Unit","Metric Value"'
