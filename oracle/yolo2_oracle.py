@@ -8,7 +8,8 @@ What it is: a restatement in NumPy / PyTorch-CPU of the reference's algorithm fo
 (reference = /root/reference, a Python-2 / TensorFlow-1.x repo that cannot run in this image).
 Every function cites the reference file:line it follows.  TensorFlow primitive semantics (SAME
 padding, BN defaults eps=1e-3 / momentum=0.99, max/min gradient tie rules) are *TF knowledge*,
-not code in the reference tree.
+not code in the reference tree.  Max-pool ties: the gradient of a 2x2 window goes whole to its first
+maximum in the order (0,0), (0,1), (1,0), (1,1) (max_pool_2x2), as the training kernels route it.
 
 Pinning status (see DESIGN.md "Oracle"):
   * get_iou / get_loss / decode / label encoder / darknet19 builders are pinned against golden
@@ -95,10 +96,17 @@ def conv2d_same(x_nhwc, w_hwio, dtype=None):
 
 
 def max_pool_2x2(x_nhwc):
-    """darknet.py:24-25: tf.nn.max_pool 2x2 stride 2 SAME (even maps -> no padding)."""
+    """darknet.py:24-25: tf.nn.max_pool 2x2 stride 2 SAME (even maps -> no padding).
+    Gradient: the whole incoming gradient goes to the FIRST maximum of each window in the order (0,0), (0,1), (1,0),
+    (1,1) [TF-knowledge: MaxPoolGrad routes to the arg-max the forward recorded, the first one it met], never split
+    between tied entries (torch's amax would split it evenly)."""
     n, h, w, c = x_nhwc.shape
     assert h % 2 == 0 and w % 2 == 0
-    return x_nhwc.reshape(n, h // 2, 2, w // 2, 2, c).amax(dim=(2, 4))
+    win = x_nhwc.reshape(n, h // 2, 2, w // 2, 2, c).permute(0, 1, 3, 5, 2, 4).reshape(n, h // 2, w // 2, c, 4)
+    v = win.detach()
+    pos = torch.arange(4, device=v.device)
+    first = torch.where(v == v.amax(dim=-1, keepdim=True), pos, 4).amin(dim=-1, keepdim=True)
+    return win.gather(-1, first).squeeze(-1)
 
 
 def batch_norm(h, gamma, beta, moving_mean, moving_var, training):

@@ -209,3 +209,34 @@ def test_resize_restatement_pinned_to_cv2(golden_dir):
         np.testing.assert_array_equal(O.resize_bilinear_u8(im, IS, IS), cv2.resize(im, (IS, IS)))
     im = cases[0][0]
     np.testing.assert_array_equal(O.resize_bilinear_u8(im, 300, 200), cv2.resize(im, (300, 200)))     # non-square target
+
+
+def test_max_pool_routes_ties_to_first_maximum():
+    """max_pool_2x2's gradient goes whole to the first maximum of each window, in the order (0,0), (0,1), (1,0), (1,1), like
+    the training kernels' arg-max routing (constant image regions give bit-identical pre-BN values, so exact ties are common);
+    the forward value is the plain maximum."""
+    x = torch.zeros((1, 4, 6, 2), dtype=torch.float64)
+    wins = {(0, 0): [[5, 5], [5, 5]],          # four-way tie -> (0,0)
+            (0, 1): [[1, 7], [7, 7]],          # three-way tie after the first entry -> (0,1)
+            (0, 2): [[2, 3], [9, 9]],          # tie in the bottom row -> (1,0)
+            (1, 0): [[-4, -4], [-4, -4]],      # negative ties
+            (1, 1): [[0, 2], [1, 3]],          # no tie -> (1,1)
+            (1, 2): [[6, 1], [6, 0]]}          # tie down the first column -> (0,0)
+    for (i, j), w in wins.items():
+        x[0, 2 * i:2 * i + 2, 2 * j:2 * j + 2, 0] = torch.tensor(w, dtype=torch.float64)
+        x[0, 2 * i:2 * i + 2, 2 * j:2 * j + 2, 1] = -torch.tensor(w, dtype=torch.float64)   # channel 1: the mirror image
+    x.requires_grad_(True)
+    y = O.max_pool_2x2(x)
+    np.testing.assert_array_equal(y.detach().numpy(), x.detach().reshape(1, 2, 2, 3, 2, 2).amax(dim=(2, 4)).numpy())
+    dy = torch.arange(1, 13, dtype=torch.float64).reshape(1, 2, 3, 2)
+    (y * dy).sum().backward()
+    want = torch.zeros_like(x)
+    xd = x.detach()
+    for i in range(2):
+        for j in range(3):
+            for c in range(2):
+                w = xd[0, 2 * i:2 * i + 2, 2 * j:2 * j + 2, c].reshape(4)
+                k = int(next(k for k in range(4) if w[k] == w.max()))
+                want[0, 2 * i + k // 2, 2 * j + k % 2, c] = dy[0, i, j, c]
+    np.testing.assert_array_equal(x.grad.numpy(), want.numpy())
+    assert want[0, 0, 0, 0] == dy[0, 0, 0, 0] and want[0, 0, 3, 0] == dy[0, 0, 1, 0] and want[0, 1, 4, 0] == dy[0, 0, 2, 0]
