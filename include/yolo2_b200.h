@@ -41,7 +41,8 @@ const char* y2_last_error(void);
 /* Number of kernels this library has launched from the calling process since load (all threads).
  * bench.py reports the delta over the timed region as "gpu_launches". */
 unsigned long long y2_launch_count(void);
-/* The Y2_* environment switches (A/B and debug knobs of the launchers) are read once per process; this re-reads them. */
+/* The Y2_* environment switches (reference paths for tests and tools, INTEGRATION.md section 5) are read once per process;
+   this re-reads them. */
 int y2_reload_env(void);
 
 /* ---- a10: input preprocessing ------------------------------------------------------------

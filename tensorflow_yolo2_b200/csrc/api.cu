@@ -19,40 +19,17 @@ static std::atomic<int> g_env_state{0};     // 0 = not read, 1 = being read, 2 =
 
 static void env_read() {
   auto on = [](const char* k) { return getenv(k) != nullptr; };
-  auto num = [](const char* k, int dflt) { const char* e = getenv(k); return e ? atoi(e) : dflt; };
   EnvSwitches e;
   e.bn_bwd_generic = on("Y2_BN_BWD_GENERIC");
-  e.conv_no_streamk = on("Y2_CONV_NO_STREAMK");
-  e.conv_streamk_1cta = on("Y2_CONV_STREAMK_1CTA");
-  e.conv_streamk_512 = on("Y2_CONV_STREAMK_512");
-  e.conv_force_streamk = on("Y2_CONV_FORCE_STREAMK");
-  e.conv_force_tiled = on("Y2_CONV_FORCE_TILED");
-  e.conv_no_patch = on("Y2_CONV_NO_PATCH");
-  e.conv_force_patch = on("Y2_CONV_FORCE_PATCH");
-  e.conv_no_cta2 = on("Y2_CONV_NO_CTA2");
-  e.conv_no_cta2_generic = on("Y2_CONV_NO_CTA2_GENERIC");
-  e.conv_cluster = on("Y2_CONV_CLUSTER");
-  e.conv_no_bstat = on("Y2_CONV_NO_BSTAT");
-  e.conv_no_kwmerge = on("Y2_CONV_NO_KWMERGE");
-  e.conv_no_tma_store = on("Y2_CONV_NO_TMA_STORE");
-  e.conv_tma_store_split = num("Y2_CONV_TMA_STORE_SPLIT", 0);
-  e.conv_is_no_tma_store = on("Y2_CONV_IS_NO_TMA_STORE");
-  e.conv_no_tma_store_f32 = on("Y2_CONV_NO_TMA_STORE_F32");
-  e.conv1_no_tma_store = on("Y2_CONV1_NO_TMA_STORE");
-  e.bn_stats_unr4 = on("Y2_BN_STATS_UNR4");
-  e.bn_stats_variant = num("Y2_BN_STATS_VARIANT", 0);
-  e.bn_bwd_minb = num("Y2_BN_BWD_MINB", 4);
   e.affine_generic = on("Y2_AFFINE_GENERIC");
   e.no_pdl = on("Y2_NO_PDL");
-  e.conv_streamk_x3_generic = on("Y2_CONV_STREAMK_X3_GENERIC");
-  e.wgrad_cta2 = on("Y2_WGRAD_CTA2");
-  e.wgrad_no_group = on("Y2_WGRAD_NO_GROUP");
+  e.conv_no_streamk = on("Y2_CONV_NO_STREAMK");
+  e.conv_force_streamk = on("Y2_CONV_FORCE_STREAMK");
+  e.conv_force_tiled = on("Y2_CONV_FORCE_TILED");
+  e.conv_no_cta2 = on("Y2_CONV_NO_CTA2");
   e.conv_no_is = on("Y2_CONV_NO_IS");
   e.conv_force_is = on("Y2_CONV_FORCE_IS");
-  e.conv_streamk_min_ksteps = num("Y2_CONV_STREAMK_MIN_KSTEPS", -1);
-  e.conv_block_n = num("Y2_CONV_BLOCK_N", 0);
-  e.conv1_debug = num("Y2_CONV1_DEBUG", 0);
-  e.wgrad_splits = num("Y2_WGRAD_SPLITS", 0);
+  e.conv_no_tma_store_f32 = on("Y2_CONV_NO_TMA_STORE_F32");
   g_env = e;
 }
 

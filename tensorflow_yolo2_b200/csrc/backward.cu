@@ -86,9 +86,9 @@ __global__ void bn_bwd_reduce_kernel(const float* __restrict__ h, int ldh, const
 }
 
 // Vectorised pass 1 (C % 4 == 0): a thread owns 4 channels (16-byte loads of h, 8-byte loads of bf16 dy) and keeps
-// UNR units in flight; block = TX channel groups x (256/TX) unit lanes.
-template <bool POOL, int TX, int MINB>
-__global__ void __launch_bounds__(256, MINB) bn_bwd_reduce_v4_kernel(
+// UNR units in flight; block = TX channel groups x (256/TX) unit lanes.  Four blocks resident per SM.
+template <bool POOL, int TX>
+__global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
     const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, const float* __restrict__ mean,
     const float* __restrict__ var, const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float alpha,
     int leaky_on, int H, int W, int C, size_t units, size_t units_per_split, double* __restrict__ part) {
@@ -692,25 +692,17 @@ int y2_bn_leaky_pool_bwd(const float* h_raw, int ldh, const void* dy, int dy_dty
   splits = (int)((units + ups - 1) / ups);
   if (C % 4 == 0 && ldh % 4 == 0 && (((uintptr_t)h_raw) & 15) == 0 && (((uintptr_t)dy) & 15) == 0) {
     const int cg = C / 4;
-    const int minb = env().bn_bwd_minb;
     {   // one wave of blocks (see bn_stats_impl); tiles are dealt round-robin, so any number of splits is balanced
       const int tx = cg <= 8 ? 8 : (cg <= 16 ? 16 : 32);
-      const int wave = num_sms() * (minb == 1 ? 2 : minb) / ((cg + tx - 1) / tx);
+      const int wave = num_sms() * 4 / ((cg + tx - 1) / tx);
       if (splits > wave) splits = wave > 1 ? wave : 1;
     }
-#define Y2_LAUNCH_RED1(POOL_, TX_, MB_)                                                                               \
-  bn_bwd_reduce_v4_kernel<POOL_, TX_, MB_><<<dim3((cg + TX_ - 1) / TX_, splits), 256, 0, st>>>(                       \
-      h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on, H, W, C, units, ups, (double*)workspace)
 #define Y2_LAUNCH_RED(POOL_, TX_)                                                                                     \
-  do {                                                                                                                \
-    if (minb == 1) Y2_LAUNCH_RED1(POOL_, TX_, 1);                                                                     \
-    else if (minb == 4) Y2_LAUNCH_RED1(POOL_, TX_, 4);                                                                \
-    else Y2_LAUNCH_RED1(POOL_, TX_, 3);                                                                               \
-  } while (0)
+  bn_bwd_reduce_v4_kernel<POOL_, TX_><<<dim3((cg + TX_ - 1) / TX_, splits), 256, 0, st>>>(                            \
+      h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on, H, W, C, units, ups, (double*)workspace)
     if (pool) { if (cg <= 8) Y2_LAUNCH_RED(true, 8); else if (cg <= 16) Y2_LAUNCH_RED(true, 16); else Y2_LAUNCH_RED(true, 32); }
     else      { if (cg <= 8) Y2_LAUNCH_RED(false, 8); else if (cg <= 16) Y2_LAUNCH_RED(false, 16); else Y2_LAUNCH_RED(false, 32); }
 #undef Y2_LAUNCH_RED
-#undef Y2_LAUNCH_RED1
   } else {
     dim3 grid((C + 31) / 32, splits), block(32, 8);
     bn_bwd_reduce_kernel<<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on,

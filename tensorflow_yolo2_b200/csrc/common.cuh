@@ -14,19 +14,12 @@ namespace y2 {
 void set_error(const char* fmt, ...);
 void count_launch(int n = 1);
 
-// Debug / A-B switches (environment variables Y2_*), read ONCE per process (a launch used to pay ~10 getenv() calls);
-// y2_reload_env() re-reads them (tests and A/B runs that flip a switch inside one process).
+// Switches (environment variables Y2_*) that select a reference path for tests and tools, or take PDL out of the
+// picture.  Read ONCE per process (a launch used to pay ~10 getenv() calls); y2_reload_env() re-reads them (tests that
+// flip a switch inside one process).
 struct EnvSwitches {
-  bool bn_bwd_generic, conv_no_streamk, conv_streamk_1cta, conv_streamk_512, conv_force_streamk, conv_force_tiled,
-      conv_no_patch, conv_force_patch, conv_no_cta2, conv_no_cta2_generic, conv_cluster, conv_no_bstat, conv_no_kwmerge,
-      conv_no_tma_store, conv_is_no_tma_store, conv_no_tma_store_f32, conv1_no_tma_store, bn_stats_unr4, affine_generic, no_pdl, conv_streamk_x3_generic, wgrad_cta2, wgrad_no_group, conv_no_is, conv_force_is;
-  int conv_streamk_min_ksteps;   // -1 = unset
-  int conv_block_n;              // 0 = unset
-  int conv1_debug;               // 0 = unset
-  int wgrad_splits;              // 0 = unset
-  int conv_tma_store_split;      // bf16x3 layer 3: 0 direct stores, 1 TMA box stores with two staging buffers per group, 2 with one
-  int bn_stats_variant;          // A/B bits: 1 = no streaming loads, 2 = four (not five) blocks per SM
-  int bn_bwd_minb;               // min resident blocks of bn_bwd_reduce_v4_kernel (1 / 3 / 4; default 3)
+  bool bn_bwd_generic, affine_generic, no_pdl, conv_no_streamk, conv_force_streamk, conv_force_tiled, conv_no_cta2,
+      conv_no_is, conv_force_is, conv_no_tma_store_f32;
 };
 const EnvSwitches& env();
 

@@ -82,9 +82,6 @@ struct Conv1Args {
   int tiles_w, tiles_per_img, total_tiles;
   uint32_t fd_img_mul, fd_img_shr, fd_w_mul, fd_w_shr;   // magic-number division by tiles_per_img / tiles_w
   float alpha;
-  int tma_store;         // the pooled tile leaves as one TMA box store from swizzled smem (0: 16-byte global stores per lane)
-  int debug;             // ablation knobs (env Y2_CONV1_DEBUG): 1 no raw loads, 2 no conversion, 4 no TMEM drain/stores, 8 no MMA,
-                         // 16 TMEM drain without the pooling math / output
 };
 
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t* v) {
@@ -164,7 +161,7 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
 
   if (warp >= C1_WARP_PRODUCER && warp < C1_WARP_MMA) {
     // =========================== raw uint8 patch: one TMA box per tile ===========================
-    if (lane == 0 && !(a.debug & 1)) {
+    if (lane == 0) {
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmImg)) : "memory");
       for (int it = warp - C1_WARP_PRODUCER;; it += C1_PROD_WARPS) {
         const int tile = first + it * step;
@@ -187,7 +184,7 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
       if (tile >= a.total_tiles) break;
       const int rs = it % C1_RAW_STAGES;
       const C1Tile t = c1_tile(a, tile);
-      if (!(a.debug & 1)) mbar_wait(&raw_full[rs], (uint32_t)(it / C1_RAW_STAGES) & 1u);
+      mbar_wait(&raw_full[rs], (uint32_t)(it / C1_RAW_STAGES) & 1u);
       mbar_wait(&a_empty[cw], ((uint32_t)(it / C1_A_STAGES) & 1u) ^ 1u);
       const uint8_t* raw = gen0 + (sRaw - sm0) + rs * C1_RAW_STAGE;
       const int row0 = 2 * t.ph0 - 1, col0 = 2 * t.pw0 - 1;
@@ -200,7 +197,7 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
       // byte loads (a second full row pass would issue 235 instructions for two active lanes)
       static_assert(C1_PROWS == 34 && C1_PCOLS == 18, "converter passes are laid out for a 34 x 18 patch");
 #pragma unroll 1
-      for (int pass = (a.debug & 2) ? 2 : 0; pass < 2; ++pass) {
+      for (int pass = 0; pass < 2; ++pass) {
         if (pass == 1 && lane >= 2 * (C1_PCOLS / 2)) break;
         const int pr = pass == 0 ? lane : 32 + lane / (C1_PCOLS / 2);
         const int jt = pass == 0 ? 0 : lane % (C1_PCOLS / 2);
@@ -291,7 +288,7 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
         const uint64_t ad = adesc0 + (uint32_t)((as * C1_A_STAGE) >> 4);
 #pragma unroll
         for (int ty = 0; ty < 4; ++ty)
-          if (!(a.debug & 8)) umma_bf16(tmem_d, ad + (uint32_t)((ty * C1_PITCH) >> 4), bdesc0 + (uint32_t)((ty * 4096) >> 4), idesc, ty > 0);
+          umma_bf16(tmem_d, ad + (uint32_t)((ty * C1_PITCH) >> 4), bdesc0 + (uint32_t)((ty * 4096) >> 4), idesc, ty > 0);
         if constexpr (SPLIT) {
 #pragma unroll
           for (int ty = 0; ty < 4; ++ty)          // the lo halves of the weights, same patch rows
@@ -305,12 +302,11 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
   } else {
     // =========================== epilogue: pool over the 4 column groups, +shift, leaky, store ===========================
     const int q = warp & 3, eg = warp >> 2;
-    const int r = q * 32 + lane, g = r >> 3, i = r & 7;
-    const int Ho = a.H >> 1, Wo = a.W >> 1;
+    const int r = q * 32 + lane;
     const float alpha = a.alpha;
-    const bool tma_st = a.tma_store != 0;
     const bool st_leader = q == 0 && lane == 0;
-    // my row of the staging box (row r = g * 8 + i, STG_ROW bytes); 16-byte unit u sits at u ^ swz (SWIZZLE_64B / _128B)
+    // my row of the staging box (pooled pixel (ph0 + (r >> 3), pw0 + (r & 7)), STG_ROW bytes); 16-byte unit u sits at u ^ swz
+    // (SWIZZLE_64B / _128B)
     const uint32_t stg_row = sStg + (uint32_t)eg * STG_BYTES + (uint32_t)r * STG_ROW;
     const uint32_t swz = SPLIT ? (uint32_t)(r & 7) : (uint32_t)((r >> 1) & 3);
     for (int it = eg;; it += C1_EPI_GROUPS) {
@@ -318,20 +314,11 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
       if (tile >= a.total_tiles) break;
       const int buf = it % C1_NBUF;
       const C1Tile t = c1_tile(a, tile);
-      uint4* dst = reinterpret_cast<uint4*>(a.y + ((size_t)((size_t)t.n * Ho + t.ph0 + g) * Wo + t.pw0 + i) * (SPLIT ? 2 * C1_COUT : C1_COUT));
       mbar_wait(&tmem_full[buf], (uint32_t)(it / C1_NBUF) & 1u);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * 128);
-      if (a.debug & 4) {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tmem_empty[buf]);
-        continue;
-      }
-      if (tma_st) {
-        if (st_leader) bulk_wait_group_read<0>();        // my group's previous box store has read the staging buffer
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + eg) : "memory");
-      }
+      if (st_leader) bulk_wait_group_read<0>();          // my group's previous box store has read the staging buffer
+      asm volatile("bar.sync %0, 128;" ::"r"(1 + eg) : "memory");
 #pragma unroll
       for (int ch = 0; ch < 4; ++ch) {                  // 8 output channels at a time
         uint32_t v0[8], v1[8], v2[8], v3[8];
@@ -345,7 +332,6 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
           __syncwarp();
           if (lane == 0) mbar_arrive(&tmem_empty[buf]);
         }
-        if (a.debug & 16) continue;                       // ablation: TMEM drain only (no pooling math, no output)
         const float4 sa = *reinterpret_cast<const float4*>(&s_shift[ch * 8]);
         const float4 sb = *reinterpret_cast<const float4*>(&s_shift[ch * 8 + 4]);
         const float shv[8] = {sa.x, sa.y, sa.z, sa.w, sb.x, sb.y, sb.z, sb.w};
@@ -368,12 +354,9 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
           __nv_bfloat162 h = __floats2bfloat162_rn(f[2 * e], f[2 * e + 1]);
           o[e] = *reinterpret_cast<uint32_t*>(&h);
         }
-        if (tma_st)
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg_row + (((uint32_t)ch ^ swz) << 4)), "r"(o[0]), "r"(o[1]),
-                       "r"(o[2]), "r"(o[3])
-                       : "memory");
-        else
-          dst[ch] = make_uint4(o[0], o[1], o[2], o[3]);
+        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg_row + (((uint32_t)ch ^ swz) << 4)), "r"(o[0]), "r"(o[1]),
+                     "r"(o[2]), "r"(o[3])
+                     : "memory");
         if constexpr (SPLIT) {
           uint32_t l[4];
 #pragma unroll
@@ -382,25 +365,20 @@ conv1_u8_pool_kernel(const __grid_constant__ CUtensorMap tmImg, const __grid_con
             __nv_bfloat162 h = __floats2bfloat162_rn(f[2 * e] - hf.x, f[2 * e + 1] - hf.y);
             l[e] = *reinterpret_cast<uint32_t*>(&h);
           }
-          if (tma_st)
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg_row + (((uint32_t)(4 + ch) ^ swz) << 4)), "r"(l[0]),
-                         "r"(l[1]), "r"(l[2]), "r"(l[3])
-                         : "memory");
-          else
-            dst[4 + ch] = make_uint4(l[0], l[1], l[2], l[3]);     // lo half: channels 32..63 of the row
+          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg_row + (((uint32_t)(4 + ch) ^ swz) << 4)), "r"(l[0]),
+                       "r"(l[1]), "r"(l[2]), "r"(l[3])
+                       : "memory");     // lo half: channels 32..63 of the row
         }
       }
-      if (tma_st) {
-        fence_proxy_async_smem();
-        asm volatile("bar.sync %0, 128;" ::"r"(1 + eg) : "memory");
-        if (st_leader) {
-          tma_store_4d(&tmY, sStg + (uint32_t)eg * STG_BYTES, 0, t.pw0, t.ph0, t.n);
-          bulk_commit_group();
-        }
+      fence_proxy_async_smem();
+      asm volatile("bar.sync %0, 128;" ::"r"(1 + eg) : "memory");
+      if (st_leader) {
+        tma_store_4d(&tmY, sStg + (uint32_t)eg * STG_BYTES, 0, t.pw0, t.ph0, t.n);
+        bulk_commit_group();
       }
       __syncwarp();
     }
-    if (tma_st && st_leader) bulk_wait_group_read<0>();   // smem must outlive the last box store's read
+    if (st_leader) bulk_wait_group_read<0>();             // smem must outlive the last box store's read
   }
 
   tc_fence_before();
@@ -498,8 +476,6 @@ static int conv1_u8_pool_launch(const uint8_t* img, const void* w_packed, const 
   Y2_ARG(total < (1ll << 31) - 1024);
   a.total_tiles = (int)total;
   a.alpha = alpha;
-  a.debug = env().conv1_debug;
-  a.tma_store = env().conv1_no_tma_store ? 0 : 1;
   CUtensorMap tmImg, tmY;
   {
     // pooled output [N, H/2, W/2, 32 | 64] bf16: boxes of one tile (8 x 16 pooled pixels, the whole row), swizzled rows

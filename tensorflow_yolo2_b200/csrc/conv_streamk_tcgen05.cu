@@ -1,48 +1,59 @@
 // conv_streamk_tcgen05.cu -- a1 + a2 (scale/shift, leaky) for the deep 3x3 layers on the small maps (26x26 and below):
-// the same implicit GEMM as conv_tcgen05.cu with 256 x 256 CTA tiles and a stream-K work split.
+// the same implicit GEMM as conv_tcgen05.cu with 256 x 256 tiles, each computed by a CTA PAIR (tcgen05 cta_group::2),
+// and a stream-K work split over the pairs.
 //
-// Why.  conv_tc_kernel on these layers is bound by the operand bytes the L2 can deliver into the SMs -- measured
-// 5 700 B/clk for the whole chip (l1tex__m_xbar2l1tex_read_bytes of L19: 2.41 GB in 215 us), not by the tensor pipe
-// (46 % busy).  A 128 x 256 tile needs 48 KB per 64-deep K step = 85 flop per delivered byte; a 256 x 256 tile
-// needs 64 KB for twice the flops = 128 flop/B, i.e. 1.5x fewer bytes for the same layer.  With K = 9 * 1024 the
-// accumulator (2 x 128 x 256 fp32 = all 512 TMEM columns, single-buffered) is drained once per ~150 k clk, so the
-// un-overlapped epilogue costs ~2 %.  But 256 x 256 tiles leave only 172 tiles for 148 SMs, so instead of whole
-// tiles each CTA takes an equal, contiguous range of (tile, K-step) units ("stream-K"): a CTA's range is the TAIL of
-// one tile (its first segment), whole tiles, and the HEAD of the next tile (its last segment).  Every range is at
-// least one tile long, so a tile is shared by at most two CTAs, c (head, done LAST in c's range) and c + 1 (tail,
-// done FIRST in c + 1's range):
-//   tail  -> the float32 partial goes to slot c + 1 of a workspace, then flag[c + 1] is released;
-//   head  -> CTA c waits for flag[c + 1] (in practice set ~150 k clk earlier), adds the partial to its own
+// Why 256 x 256.  conv_tc_kernel on these layers is bound by the operand bytes the L2 can deliver into the SMs --
+// measured 5 700 B/clk for the whole chip (l1tex__m_xbar2l1tex_read_bytes of L19: 2.41 GB in 215 us), not by the tensor
+// pipe (46 % busy).  A 128 x 256 tile needs 48 KB per 64-deep K step = 85 flop per delivered byte; a 256 x 256 tile
+// needs 64 KB for twice the flops = 128 flop/B, i.e. 1.5x fewer bytes for the same layer.
+//
+// Why a CTA pair.  With cta_group::1 every MMA fetches its whole A (128 x 16) and B (N x 16) slice from the issuing SM's
+// shared memory, and that operand path moves ~64 B/clk: 12 KB = 192 clk for a 128 x 256 x 16 MMA whose arithmetic takes
+// 128 clk.  ncu on the single-CTA kernels (profiles/r1c): 101 / 146 / 192 clk per MMA at N = 64 / 128 / 256, i.e.
+// (4096 + 32 N) / 64 -- the tensor pipe tops out at 67 % however the loop is written.  A pair computes one 256 x 256 tile
+// with M = 256 MMAs: each SM supplies its own 128 rows of A and HALF of the B rows (8 KB per MMA = the 128 clk of
+// arithmetic) and accumulates its 128 rows in its own TMEM.
+//   * both CTAs run a TMA producer (own A half, own B half) that signals the LEADER's full barrier (cta_group::2 loads,
+//     leader-mapped barrier address); the leader alone expects the 64 KB of both;
+//   * the leader's MMA warp issues tcgen05.mma.cta_group::2 and commits with a multicast arrive to the empty / tmem_full
+//     barriers of both CTAs; the follower's MMA warp only allocates / frees TMEM;
+//   * each CTA's 8 epilogue warps drain their own 128 x 256 accumulator and arrive on the leader's tmem_empty.
+// The accumulator is 256 of the 512 TMEM columns, so segments alternate between two buffers and the epilogue of one
+// segment overlaps the MMAs of the next.
+//
+// Stream-K.  256 x 256 tiles leave only 172 tiles for 74 pairs, so instead of whole tiles each pair takes an equal,
+// contiguous range of (tile, K-step) units: a pair's range is the TAIL of one tile (its first segment), whole tiles, and
+// the HEAD of the next tile (its last segment).  Every range is at least one tile long, so a tile is shared by at most two
+// pairs, c (head, done LAST in c's range) and c + 1 (tail, done FIRST in c + 1's range).  Per CTA (same rank: same rows):
+//   tail  -> the float32 partial goes to workspace slot blockIdx.x, then flag[blockIdx.x] is released;
+//   head  -> the CTA waits for flag[blockIdx.x + 2] (in practice set ~150 k clk earlier), adds the partial to its own
 //            accumulator and runs the full epilogue (scale/shift, leaky, float32 or bf16 store) -- the owner
 //            finalises, so the fused epilogue survives the K split, there are no atomics and no zero-fill, and the
 //            result is bit-reproducible (fixed order: head + tail).
 // No circular wait: a tail segment depends on nothing, and all CTAs are co-resident (grid <= #SMs, 1 CTA/SM).
 //
 // Scope: ksize 1 or 3, stride 1, SAME; Cin % 64 == 0; Cout % 256 == 0; no fused pool; maps smaller than 64x64;
-// >= 32 K steps.  Needs the workspace registered with y2_conv_set_workspace (y2_conv_workspace_bytes() bytes, one per
-// stream); without it, or for any other layer, y2_conv_fwd_bf16 stays on conv_tc_kernel.  Env Y2_CONV_NO_STREAMK=1
-// disables the path.
+// >= 18 K steps (bf16x3: 6); at least two SMs.  Needs the workspace registered with y2_conv_set_workspace
+// (y2_conv_workspace_bytes() bytes, one per stream); without it, or for any other layer, y2_conv_fwd_bf16 stays on
+// conv_tc_kernel.  Env Y2_CONV_NO_STREAMK=1 disables the path.
 #include "tc_common.cuh"
 
 namespace y2 {
 
 constexpr int SK_THREADS = 64 + 8 * 32;        // warps 0-7 epilogue (2 per TMEM lane quarter), 8 TMA, 9 MMA
-constexpr int SK_STAGES = 3;                   // 64 KB each: A 2 x (128 px x 128 B), B 256 x 128 B
-constexpr uint32_t SK_A_HALF = 128 * 128, SK_B_BYTES = 256 * 128, SK_STAGE = 2 * SK_A_HALF + SK_B_BYTES;
 constexpr int SK_MAX_UNITS = 1024;             // K steps per tile (bf16x3, 3x3, 1280 channels: 9 * 60 = 540)
 
 struct SkArgs {
   const float* scale;
   const float* shift;
   void* y;
-  float* ws_partial;                // [grid][2][128][256] float32 partial accumulators (slot = the tail CTA)
+  float* ws_partial;                // [grid][128][256] float32 partial accumulators (slot = the tail CTA)
   int* ws_flags;                    // [grid + 2], all zero between launches (a head resets the flag it consumed)
   float alpha;
   int leaky, out_f32;
   long long M;
   int H, W, ldy, pad;
   int cin_p, cchunks, ksteps;       // K steps per tile = taps * cchunks   (cin_p: K extent per tap of the B operand)
-  int a_wrap;                       // channel chunks of the A tensor (bf16x3: 2/3 of cchunks -- the K loop walks [hi | lo | hi])
   int split_out, lo_off;            // bf16x3 output: hi at column c, lo at column lo_off + c
   float* stats;                     // out_f32 only: per 32-row slab and column (k, sum(x - k), sum((x - k)^2)) of the stored rows,
   int cout;                         //   laid out [slab][3][cout] -- batch-norm statistics without a second pass over the rows
@@ -54,11 +65,11 @@ struct SkArgs {
 
 constexpr uint32_t SK_STG_WARP = 32 * 128;     // per-warp store staging: 32 rows x 32 floats (or bf16), 128B-swizzled
 
-// K step -> (filter tap, A channel coordinate, B K coordinate).  bf16x3: the third block of a tap re-reads the hi channels.
+// K step -> (filter tap, A channel coordinate, B K coordinate).  bf16x3 (X3): the hi chunks; the stage adds their lo partners.
 __device__ __forceinline__ void sk_unit(const SkArgs& a, int k, int& tap, int& a_c0, int& b_k) {
   tap = (int)fdiv((uint32_t)k, a.fd_cc_mul, a.fd_cc_shr);
   const int j = k - tap * a.cchunks;
-  a_c0 = (j < a.a_wrap ? j : j - a.a_wrap) * 64;
+  a_c0 = j * 64;
   b_k = tap * a.cin_p + j * 64;
 }
 
@@ -129,289 +140,29 @@ __device__ __forceinline__ void sk_store_chunk_bf16(const SkArgs& a, uint32_t st
   }
 }
 
-__global__ void __launch_bounds__(SK_THREADS, 1)
-conv_streamk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const SkArgs a) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  __shared__ __align__(8) uint64_t full_bar[SK_STAGES], empty_bar[SK_STAGES], tmem_full, tmem_empty;
-  __shared__ uint32_t s_tmem_base;
-  pdl_launch_dependents();                                      // persistent grid: the next kernel may take SMs as my CTAs retire
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t smem_base = (smem_u32(smem) + 1023u) & ~1023u;
-
-  // my contiguous range of (tile, K-step) units
-  const long long u_begin = a.units * blockIdx.x / gridDim.x, u_end = a.units * (blockIdx.x + 1) / gridDim.x;
-
-  if (warp == 8) {
-    if (lane == 0) {
-      asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-      asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
-      for (int s = 0; s < SK_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-      mbar_init(&tmem_full, 1);
-      mbar_init(&tmem_empty, 8);
-      fence_barrier_init();
-    }
-  }
-  if (warp == 9) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem_base)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = s_tmem_base;
-  pdl_wait();                                                   // everything above overlapped the previous kernel's tail
-
-  if (warp == 8) {
-    // =========================== TMA producer ===========================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      long long u = u_begin;
-      while (u < u_end) {
-        const uint32_t tile = (uint32_t)fdiv((uint32_t)u, a.fd_ks_mul, a.fd_ks_shr);       // units < 2^31 (host-checked)
-        const int k0 = (int)(u - (long long)tile * a.ksteps);
-        const int k1 = (int)min((long long)a.ksteps, k0 + (u_end - u));
-        const uint32_t mt = fdiv(tile, a.fd_nt_mul, a.fd_nt_shr);
-        const int nrow0 = (int)(tile - mt * (uint32_t)a.n_tiles) * 256;
-        int w0[2], h0[2], n0[2];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          uint32_t m = mt * 256u + (uint32_t)h * 128u;
-          if ((long long)m >= a.M) m = 0;                    // half tile entirely past the end: load valid pixels, rows are masked
-          const uint32_t row = fdiv(m, a.fd_w_mul, a.fd_w_shr);
-          w0[h] = (int)(m - row * (uint32_t)a.W);
-          const uint32_t img = fdiv(row, a.fd_h_mul, a.fd_h_shr);
-          h0[h] = (int)(row - img * (uint32_t)a.H);
-          n0[h] = (int)img;
-        }
-        for (int k = k0; k < k1; ++k) {
-          mbar_wait(&empty_bar[stage], phase ^ 1u);
-          mbar_expect_tx(&full_bar[stage], SK_STAGE);
-          int tap, a_c0, b_k;
-          sk_unit(a, k, tap, a_c0, b_k);
-          const int kh = a.pad ? (tap * 11) >> 5 : 0, kw = tap - kh * 3;       // tap / 3 for tap < 9 (1x1: tap == 0)
-          const uint32_t sA = smem_base + stage * SK_STAGE;
-          const uint32_t bar = smem_u32(&full_bar[stage]);
-          tma_load_im2col_4d(sA, &tmA, bar, a_c0, w0[0] - a.pad, h0[0] - a.pad, n0[0], (uint16_t)kw, (uint16_t)kh);
-          tma_load_im2col_4d(sA + SK_A_HALF, &tmA, bar, a_c0, w0[1] - a.pad, h0[1] - a.pad, n0[1], (uint16_t)kw, (uint16_t)kh);
-          tma_load_2d(sA + 2 * SK_A_HALF, &tmB, bar, b_k, nrow0);
-          if (++stage == SK_STAGES) { stage = 0; phase ^= 1u; }
-        }
-        u += k1 - k0;
-      }
-    }
-  } else if (warp == 9) {
-    // =========================== MMA issuer ===========================
-    uint32_t is_leader;
-    asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(is_leader));
-    constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-    const uint64_t adesc0 = make_smem_desc(smem_base, 16u, 8u * 128u, 2u);                    // SWIZZLE_128B, K-major
-    const uint64_t bdesc0 = make_smem_desc(smem_base + 2 * SK_A_HALF, 16u, 8u * 128u, 2u);
-    int stage = 0;
-    uint32_t phase = 0, seg = 0;
-    long long u = u_begin;
-    while (u < u_end) {
-      const uint32_t tile = (uint32_t)fdiv((uint32_t)u, a.fd_ks_mul, a.fd_ks_shr);
-      const int k0 = (int)(u - (long long)tile * a.ksteps);
-      const int k1 = (int)min((long long)a.ksteps, k0 + (u_end - u));
-      mbar_wait(&tmem_empty, (seg & 1u) ^ 1u);                 // the previous segment's accumulators are drained
-      tc_fence_after();
-      uint32_t accum = 0;
-      for (int k = k0; k < k1; ++k) {
-        mbar_wait(&full_bar[stage], phase);
-        tc_fence_after();
-        if (is_leader) {
-          const uint32_t soff = (uint32_t)(stage * SK_STAGE) >> 4;
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-            for (int h = 0; h < 2; ++h)
-              umma_bf16(tmem_base + (uint32_t)(h * 256), adesc0 + soff + (uint32_t)(h * (SK_A_HALF >> 4)) + (uint32_t)(ks * 2),
-                        bdesc0 + soff + (uint32_t)(ks * 2), idesc, accum);
-            accum = 1;
-          }
-          umma_commit(&empty_bar[stage]);
-        }
-        __syncwarp();
-        if (++stage == SK_STAGES) { stage = 0; phase ^= 1u; }
-      }
-      if (is_leader) umma_commit(&tmem_full);
-      __syncwarp();
-      u += k1 - k0;
-      ++seg;
-    }
-  } else {
-    // =========================== epilogue ===========================
-    const int q = warp & 3, chalf = warp >> 2;                 // TMEM lane quarter, column half of each accumulator
-    const int et = threadIdx.x;                                // 0..255
-    uint32_t seg = 0;
-    long long u = u_begin;
-    while (u < u_end) {
-      const uint32_t tile = (uint32_t)fdiv((uint32_t)u, a.fd_ks_mul, a.fd_ks_shr);
-      const int k0 = (int)(u - (long long)tile * a.ksteps);
-      const int k1 = (int)min((long long)a.ksteps, k0 + (u_end - u));
-      const bool tail = k0 > 0;                                // partial -> workspace slot blockIdx.x
-      const bool head = k0 == 0 && k1 < a.ksteps;              // owner: add the partial of CTA blockIdx.x + 1, finalise
-      const uint32_t mt = fdiv(tile, a.fd_nt_mul, a.fd_nt_shr);
-      const int col0 = (int)(tile - mt * (uint32_t)a.n_tiles) * 256 + chalf * 128;
-      if (head) {
-        if (et == 0) {
-          const int* f = a.ws_flags + blockIdx.x + 1;
-          int v;
-          long long t0 = clock64();
-          do {
-            asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(f) : "memory");
-            if (!v) {
-              __nanosleep(200);
-              if (clock64() - t0 > 6000000000ll) { printf("y2 conv_streamk: partial of CTA %d never arrived\n", blockIdx.x + 1); __trap(); }
-            }
-          } while (!v);
-          *const_cast<int*>(f) = 0;                             // consumed: the flags are all zero again when the kernel ends
-        }
-        asm volatile("bar.sync 1, 256;" ::: "memory");          // the 8 epilogue warps
-      }
-      mbar_wait(&tmem_full, seg & 1u);
-      tc_fence_after();
-      // Partials use a lane-major layout (float4 #i of lane l at [i * 32 + l]) so that both the tail's stores and the
-      // head's loads are fully coalesced; the final rows go through a per-warp 128B-swizzled smem tile so that one store
-      // instruction covers whole 128-byte (float32) / 64-byte (bf16) row segments instead of 32 scattered 16-byte pieces.
-      const uint32_t stg = smem_base + SK_STAGES * SK_STAGE + (uint32_t)warp * SK_STG_WARP;
-      float4* part = reinterpret_cast<float4*>(a.ws_partial + (size_t)(tail ? blockIdx.x : blockIdx.x + 1) * 65536) +
-                     (size_t)warp * 2048 + lane;                  // + (h * 4 + c/32) * 256 + i * 32
-      float4 pv[8];
-      if (head) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) pv[i] = __ldcg(part + i * 32);
-      }
-#pragma unroll 1
-      for (int hc = 0; hc < 8; ++hc) {
-        const int h = hc >> 2, c = (hc & 3) * 32;
-        const int row0 = h * 128 + q * 32;                        // first tile row of this warp's 32-row slab
-        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(h * 256 + chalf * 128 + c);
-        uint32_t v[32];
-        tmem_ld32(taddr, v);
-        tmem_ld_wait();
-        if (hc == 7) {                                         // my last chunk is in registers
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tmem_empty);
-        }
-        if (tail) {
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            __stcg(part + hc * 256 + i * 32, make_float4(__uint_as_float(v[4 * i]), __uint_as_float(v[4 * i + 1]),
-                                                         __uint_as_float(v[4 * i + 2]), __uint_as_float(v[4 * i + 3])));
-          continue;
-        }
-        float f[32];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          float4 sc = make_float4(1.f, 1.f, 1.f, 1.f), sh = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (a.scale) sc = __ldg(reinterpret_cast<const float4*>(a.scale + col0 + c) + i);
-          if (a.shift) sh = __ldg(reinterpret_cast<const float4*>(a.shift + col0 + c) + i);
-          const float4 p4 = head ? pv[i] : make_float4(0.f, 0.f, 0.f, 0.f);
-          f[4 * i + 0] = fmaf(__uint_as_float(v[4 * i + 0]) + p4.x, sc.x, sh.x);
-          f[4 * i + 1] = fmaf(__uint_as_float(v[4 * i + 1]) + p4.y, sc.y, sh.y);
-          f[4 * i + 2] = fmaf(__uint_as_float(v[4 * i + 2]) + p4.z, sc.z, sh.z);
-          f[4 * i + 3] = fmaf(__uint_as_float(v[4 * i + 3]) + p4.w, sc.w, sh.w);
-        }
-        if (head && hc < 7) {                                  // prefetch the next chunk's partial behind this chunk's stores
-#pragma unroll
-          for (int i = 0; i < 8; ++i) pv[i] = __ldcg(part + (hc + 1) * 256 + i * 32);
-        }
-        if (a.leaky) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) f[i] = fmaxf(f[i], a.alpha * f[i]);
-        }
-        const long long grow0 = (long long)mt * 256 + row0;       // global row of slab row 0
-        if (a.out_f32) {
-          // lane = slab row: 8 x 16-byte units, unit j of row r at (j ^ (r & 7))
-#pragma unroll
-          for (int j = 0; j < 8; ++j)
-            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(stg + lane * 128 + ((j ^ (lane & 7)) << 4)), "f"(f[4 * j]),
-                         "f"(f[4 * j + 1]), "f"(f[4 * j + 2]), "f"(f[4 * j + 3])
-                         : "memory");
-          __syncwarp();
-          float* dst = reinterpret_cast<float*>(a.y) + col0 + c;
-#pragma unroll
-          for (int t = 0; t < 8; ++t) {
-            const int r = t * 4 + (lane >> 3), j = lane & 7;
-            float4 o;
-            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(o.x), "=f"(o.y), "=f"(o.z), "=f"(o.w)
-                         : "r"(stg + r * 128 + ((j ^ (r & 7)) << 4)));
-            if (grow0 + r < a.M) *reinterpret_cast<float4*>(dst + (size_t)(grow0 + r) * a.ldy + j * 4) = o;
-          }
-          if (a.stats) sk_slab_stats(a, stg, lane, col0 + c, grow0);
-        } else {
-          sk_store_chunk_bf16(a, stg, lane, f, col0 + c, grow0);
-        }
-        __syncwarp();                                           // staging tile free for the next chunk
-      }
-      if (tail) {
-        __threadfence();                                       // my partial is visible device-wide ...
-        asm volatile("bar.sync 1, 256;" ::: "memory");          // ... and so is everybody else's
-        if (et == 0) {
-          int one = 1;
-          asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(a.ws_flags + blockIdx.x), "r"(one) : "memory");
-        }
-      }
-      u += k1 - k0;
-      ++seg;
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 9) {
-    __syncwarp();
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// CTA-pair variant (tcgen05 cta_group::2).  Why: with cta_group::1 every MMA fetches its whole A (128 x 16) and B
-// (N x 16) slice from the issuing SM's shared memory, and that operand path moves ~64 B/clk: 12 KB = 192 clk for a
-// 128 x 256 x 16 MMA whose arithmetic takes 128 clk.  ncu on the single-CTA kernels (profiles/r1c): 101 / 146 / 192 clk
-// per MMA at N = 64 / 128 / 256, i.e. (4096 + 32 N) / 64 -- the tensor pipe tops out at 67 % however the loop is
-// written.  A CTA pair computes one 256 x 256 tile with M = 256 MMAs: each SM supplies its own 128 rows of A and HALF
-// of the B rows (8 KB per MMA = the 128 clk of arithmetic) and accumulates its 128 rows in its own TMEM.
-//   * both CTAs run a TMA producer (own A half, own B half) that signals the LEADER's full barrier (cta_group::2 loads,
-//     leader-mapped barrier address); the leader alone expects the 64 KB of both;
-//   * the leader's MMA warp issues tcgen05.mma.cta_group::2 and commits with a multicast arrive to the empty / tmem_full
-//     barriers of both CTAs; the follower's MMA warp only allocates / frees TMEM;
-//   * each CTA's 8 epilogue warps drain their own 128 x 256 accumulator and arrive on the leader's tmem_empty.
-// The accumulator is 256 of the 512 TMEM columns, so segments alternate between two buffers and the epilogue of one
-// segment overlaps the MMAs of the next.  Stream-K split, partial hand-over and epilogue as above, per CTA pair:
-// pair c's head waits for the partials of pair c + 1 (same rank: same rows), slots / flags indexed by blockIdx.x.
-// ------------------------------------------------------------------------------------------------------------------
-// HALVES = 1: 256 x 256 pair tiles, the two accumulator buffers alternate between segments (above).
-// HALVES = 2: 512 x 256 pair tiles -- each CTA carries TWO 128-row halves (two accumulators = all 512 TMEM columns,
-//   single-buffered) that share its half of the filters: 48 KB per K step for twice the flops of 32 KB.  The HALVES = 1
-//   kernel runs at the L2 -> SM delivery limit (ncu: 1.64 GB in 143 us = 11.5 TB/s, tensor pipe 77 % busy, the issuer
-//   waiting on TMA), so fewer delivered bytes per flop is what is left; the price is an un-overlapped epilogue (~150 k clk
-//   of MMAs per drain at K = 9 x 1024, so a few per cent).  MEASURED: slower (see the launcher) -- kept as an opt-in.
+// 512 x 256 pair tiles (two 128-row halves per CTA sharing its half of the filters, 48 KB per K step for twice the flops
+// of 32 KB) were measured SLOWER on B200 (L19 149 vs 137 us, L6 116 vs 89 us): the un-overlapped epilogue, the shallower
+// 4-stage ring and the coarser tile quantisation cost more than the 1.33x fewer delivered bytes per flop bring.
 constexpr uint32_t SK2_A_BYTES = 128 * 128;
-// X3 (the bf16x3 precision mode, HALVES == 1 only): one pipeline stage holds BOTH halves of a 64-channel chunk of the pixels
+// X3 (the bf16x3 precision mode): one pipeline stage holds BOTH halves of a 64-channel chunk of the pixels
 // (hi, lo) and of the filters (w_hi, w_lo) -- 64 KB per CTA -- and feeds three MMAs per K = 16 slice (hi*w_hi, lo*w_hi,
 // hi*w_lo): 64 KB delivered per 12 MMAs instead of the 96 KB the generic K walk over [hi | lo | hi] x [w_hi | w_hi | w_lo]
 // needs.  The kernel is bound by exactly that delivery (above), and the bf16x3 operands (144 MB per head layer) no longer
 // fit the L2 beside the output, so fewer re-fetched bytes is what counts.  Same packed weights: w_hi = first, w_lo = third
 // block of a tap.
-template <int HALVES, bool X3 = false> struct Sk2Cfg {
-  static constexpr uint32_t STAGE = X3 ? 4 * SK2_A_BYTES : (HALVES + 1) * SK2_A_BYTES;   // per CTA: pixels (+ lo) + 128 filters (+ lo)
-  static constexpr int STAGES = X3 ? 3 : (HALVES == 1 ? 6 : 4);          // 192 KB of operands either way
+template <bool X3> struct Sk2Cfg {
+  static constexpr uint32_t STAGE = X3 ? 4 * SK2_A_BYTES : 2 * SK2_A_BYTES;   // per CTA: pixels (+ lo) + 128 filters (+ lo)
+  static constexpr int STAGES = X3 ? 3 : 6;                                  // 192 KB of operands either way
 };
+constexpr size_t SK2_SMEM = (size_t)Sk2Cfg<false>::STAGES * Sk2Cfg<false>::STAGE + 8 * SK_STG_WARP + 1024;
+static_assert(Sk2Cfg<true>::STAGES * Sk2Cfg<true>::STAGE == Sk2Cfg<false>::STAGES * Sk2Cfg<false>::STAGE, "operand smem");
 
-template <int HALVES, bool X3 = false>
+template <bool X3>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(SK_THREADS, 1)
 conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const SkArgs a) {
-  static_assert(!X3 || HALVES == 1, "bf16x3 stages: 256-row pair tiles only");
-  constexpr int SK2_STAGES = Sk2Cfg<HALVES, X3>::STAGES;
-  constexpr uint32_t SK2_STAGE = Sk2Cfg<HALVES, X3>::STAGE;
-  constexpr int NCHUNK = 4 * HALVES;                           // 32-column chunks per epilogue warp and segment
-  constexpr uint32_t TILE_ROWS = 256u * HALVES;
+  constexpr int SK2_STAGES = Sk2Cfg<X3>::STAGES;
+  constexpr uint32_t SK2_STAGE = Sk2Cfg<X3>::STAGE;
+  constexpr int NCHUNK = 4;                                    // 32-column chunks per epilogue warp and segment
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ __align__(8) uint64_t full_bar[SK2_STAGES], empty_bar[SK2_STAGES], tmem_full[2], tmem_empty[2];
   __shared__ uint32_t s_tmem_base;
@@ -457,17 +208,12 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
         const int k1 = (int)min((long long)a.ksteps, k0 + (u_end - u));
         const uint32_t mt = fdiv(tile, a.fd_nt_mul, a.fd_nt_shr);
         const int nrow0 = (int)(tile - mt * (uint32_t)a.n_tiles) * 256 + (int)rank * 128;   // my half of the filters
-        int w0[HALVES], h0[HALVES], n0[HALVES];
-#pragma unroll
-        for (int h = 0; h < HALVES; ++h) {
-          uint32_t m = mt * TILE_ROWS + (uint32_t)h * 256u + rank * 128u;                   // my rows of half h
-          if ((long long)m >= a.M) m = 0;                      // entirely past the end: load valid pixels, rows are masked
-          const uint32_t row = fdiv(m, a.fd_w_mul, a.fd_w_shr);
-          w0[h] = (int)(m - row * (uint32_t)a.W);
-          const uint32_t img = fdiv(row, a.fd_h_mul, a.fd_h_shr);
-          h0[h] = (int)(row - img * (uint32_t)a.H);
-          n0[h] = (int)img;
-        }
+        uint32_t m = mt * 256u + rank * 128u;                   // my rows
+        if ((long long)m >= a.M) m = 0;                        // entirely past the end: load valid pixels, rows are masked
+        const uint32_t row = fdiv(m, a.fd_w_mul, a.fd_w_shr);
+        const int w0 = (int)(m - row * (uint32_t)a.W);
+        const uint32_t img = fdiv(row, a.fd_h_mul, a.fd_h_shr);
+        const int h0 = (int)(row - img * (uint32_t)a.H), n0 = (int)img;
         for (int k = k0; k < k1; ++k) {
           mbar_wait(&empty_bar[stage], phase ^ 1u);             // my own copy: the leader's commit arrives on both
           if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * SK2_STAGE);
@@ -477,20 +223,16 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
           const uint32_t sA = smem_base + stage * SK2_STAGE;
           const uint32_t bar = smem_u32(&full_bar[stage]) & PEER_BIT_MASK;      // the leader's barrier
           if constexpr (X3) {
-            // stage = [pixels hi | pixels lo | filters hi | filters lo]; lo channels sit a_wrap/2 chunks further, w_lo two
-            // blocks (of cin_p / 3) further
-            const int lo_c = (a.a_wrap >> 1) * 64, lo_k = 2 * (a.cin_p / 3);
-            tma_load_im2col_4d_2sm(sA, &tmA, bar, a_c0, w0[0] - a.pad, h0[0] - a.pad, n0[0], (uint16_t)kw, (uint16_t)kh);
-            tma_load_im2col_4d_2sm(sA + SK2_A_BYTES, &tmA, bar, a_c0 + lo_c, w0[0] - a.pad, h0[0] - a.pad, n0[0], (uint16_t)kw,
-                                   (uint16_t)kh);
+            // stage = [pixels hi | pixels lo | filters hi | filters lo]; the lo channels sit one block (of cin_p / 3 = Cin)
+            // further, w_lo two blocks further
+            const int lo_c = a.cin_p / 3, lo_k = 2 * lo_c;
+            tma_load_im2col_4d_2sm(sA, &tmA, bar, a_c0, w0 - a.pad, h0 - a.pad, n0, (uint16_t)kw, (uint16_t)kh);
+            tma_load_im2col_4d_2sm(sA + SK2_A_BYTES, &tmA, bar, a_c0 + lo_c, w0 - a.pad, h0 - a.pad, n0, (uint16_t)kw, (uint16_t)kh);
             tma_load_2d_2sm(sA + 2 * SK2_A_BYTES, &tmB, bar, b_k, nrow0);
             tma_load_2d_2sm(sA + 3 * SK2_A_BYTES, &tmB, bar, b_k + lo_k, nrow0);
           } else {
-#pragma unroll
-            for (int h = 0; h < HALVES; ++h)
-              tma_load_im2col_4d_2sm(sA + (uint32_t)h * SK2_A_BYTES, &tmA, bar, a_c0, w0[h] - a.pad, h0[h] - a.pad, n0[h], (uint16_t)kw,
-                                     (uint16_t)kh);
-            tma_load_2d_2sm(sA + HALVES * SK2_A_BYTES, &tmB, bar, b_k, nrow0);
+            tma_load_im2col_4d_2sm(sA, &tmA, bar, a_c0, w0 - a.pad, h0 - a.pad, n0, (uint16_t)kw, (uint16_t)kh);
+            tma_load_2d_2sm(sA + SK2_A_BYTES, &tmB, bar, b_k, nrow0);
           }
           if (++stage == SK2_STAGES) { stage = 0; phase ^= 1u; }
         }
@@ -505,7 +247,7 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       // D=f32, A=B=bf16, K-major both, N = 256, M = 256 (the pair)
       constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
       const uint64_t adesc0 = make_smem_desc(smem_base, 16u, 8u * 128u, 2u);                    // SWIZZLE_128B, K-major
-      const uint64_t bdesc0 = make_smem_desc(smem_base + (X3 ? 2 : HALVES) * SK2_A_BYTES, 16u, 8u * 128u, 2u);
+      const uint64_t bdesc0 = make_smem_desc(smem_base + (X3 ? 2 : 1) * SK2_A_BYTES, 16u, 8u * 128u, 2u);
       const uint32_t empty0 = smem_u32(&empty_bar[0]), tfull0 = smem_u32(&tmem_full[0]);
       int stage = 0;
       uint32_t phase = 0, seg = 0;
@@ -514,8 +256,7 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
         const uint32_t tile = (uint32_t)fdiv((uint32_t)u, a.fd_ks_mul, a.fd_ks_shr);
         const int k0 = (int)(u - (long long)tile * a.ksteps);
         const int k1 = (int)min((long long)a.ksteps, k0 + (u_end - u));
-        const uint32_t buf = HALVES == 1 ? (seg & 1u) : 0u;
-        const uint32_t par = HALVES == 1 ? ((seg >> 1) & 1u) : (seg & 1u);
+        const uint32_t buf = seg & 1u, par = (seg >> 1) & 1u;
         mbar_wait(&tmem_empty[buf], par ^ 1u);                   // both CTAs drained this buffer's previous segment
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + buf * 256u;
@@ -538,10 +279,7 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
             } else {
 #pragma unroll
               for (int ks = 0; ks < 4; ++ks) {
-#pragma unroll
-                for (int h = 0; h < HALVES; ++h)
-                  umma_bf16_2sm(tmem_d + (uint32_t)(h * 256), adesc0 + soff + (uint32_t)(h * (SK2_A_BYTES >> 4)) + (uint32_t)(ks * 2),
-                                bdesc0 + soff + (uint32_t)(ks * 2), idesc, accum);
+                umma_bf16_2sm(tmem_d, adesc0 + soff + (uint32_t)(ks * 2), bdesc0 + soff + (uint32_t)(ks * 2), idesc, accum);
                 accum = 1;
               }
             }
@@ -570,8 +308,7 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       const bool head = k0 == 0 && k1 < a.ksteps;              // owner: add the partial of CTA blockIdx.x + 2, finalise
       const uint32_t mt = fdiv(tile, a.fd_nt_mul, a.fd_nt_shr);
       const int col0 = (int)(tile - mt * (uint32_t)a.n_tiles) * 256 + chalf * 128;
-      const uint32_t buf = HALVES == 1 ? (seg & 1u) : 0u;
-      const uint32_t par = HALVES == 1 ? ((seg >> 1) & 1u) : (seg & 1u);
+      const uint32_t buf = seg & 1u, par = (seg >> 1) & 1u;
       if (head) {
         if (et == 0) {
           const int* f = a.ws_flags + blockIdx.x + 2;
@@ -591,8 +328,8 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       mbar_wait(&tmem_full[buf], par);
       tc_fence_after();
       const uint32_t stg = smem_base + SK2_STAGES * SK2_STAGE + (uint32_t)warp * SK_STG_WARP;
-      float4* part = reinterpret_cast<float4*>(a.ws_partial + (size_t)(tail ? blockIdx.x : blockIdx.x + 2) * (32768 * HALVES)) +
-                     (size_t)warp * (1024 * HALVES) + lane;        // + hc * 256 + i * 32
+      float4* part = reinterpret_cast<float4*>(a.ws_partial + (size_t)(tail ? blockIdx.x : blockIdx.x + 2) * 32768) +
+                     (size_t)warp * 1024 + lane;                   // + hc * 256 + i * 32
       float4 pv[8];
       if (head) {
 #pragma unroll
@@ -600,10 +337,9 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       }
 #pragma unroll 1
       for (int hc = 0; hc < NCHUNK; ++hc) {
-        const int h = hc >> 2, c = (hc & 3) * 32;
-        const int row0 = h * 256 + (int)rank * 128 + q * 32;      // first tile row of this warp's 32-row slab
-        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (HALVES == 1 ? buf * 256u : (uint32_t)(h * 256)) +
-                               (uint32_t)(chalf * 128 + c);
+        const int c = hc * 32;
+        const int row0 = (int)rank * 128 + q * 32;                // first tile row of this warp's 32-row slab
+        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + buf * 256u + (uint32_t)(chalf * 128 + c);
         uint32_t v[32];
         tmem_ld32(taddr, v);
         tmem_ld_wait();
@@ -639,7 +375,7 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
 #pragma unroll
           for (int i = 0; i < 32; ++i) f[i] = fmaxf(f[i], a.alpha * f[i]);
         }
-        const long long grow0 = (long long)mt * TILE_ROWS + row0; // global row of slab row 0
+        const long long grow0 = (long long)mt * 256 + row0;       // global row of slab row 0
         if (a.out_f32) {
           // lane = slab row: 8 x 16-byte units, unit j of row r at (j ^ (r & 7))
 #pragma unroll
@@ -693,11 +429,11 @@ constexpr size_t SK_FLAG_BYTES = 4096;
 static size_t sk_workspace_bytes(int sms) { return SK_FLAG_BYTES + (size_t)sms * 256 * 256 * sizeof(float); }
 
 // returns Y2_OK and sets *handled = 1 when the layer was issued on this path
-// dry != 0: only decide (*handled = 2 when the launch would be the CTA-pair kernel, whose float32 epilogue can emit the
-// batch-norm slab statistics; 1 for the single-CTA kernel) -- nothing is enqueued
+// dry != 0: only decide (*handled = 1 when the layer would take this path, whose float32 epilogue can emit the batch-norm
+// slab statistics) -- nothing is enqueued
 int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int dry) {
   *handled = 0;
-  if (env().conv_no_streamk || g_sk_ws == nullptr) return Y2_OK;
+  if (env().conv_no_streamk || g_sk_ws == nullptr || g_num_sms < 2) return Y2_OK;
   if ((p->flags & Y2_CONV_POOL2) != 0) return Y2_OK;
   if (!(p->ksize == 1 || p->ksize == 3) || p->Cin % 64 != 0 || p->Cout % 256 != 0) return Y2_OK;
   if (p->H >= 64 && p->W >= 64) return Y2_OK;                   // large maps: the halo-patch mode of conv_tc_kernel wins
@@ -709,13 +445,11 @@ int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int
   const bool split_in = (p->flags & Y2_CONV_IN_SPLIT) != 0;
   const bool split_out = (p->flags & Y2_CONV_OUT_SPLIT) != 0 && !out_f32;
   const int a_cin = split_in ? 2 * p->Cin : p->Cin, b_cin = split_in ? 3 * p->Cin : p->Cin;
-  const bool two_cta_pre = !env().conv_streamk_1cta && g_num_sms >= 2;
-  const bool x3 = split_in && two_cta_pre && !env().conv_streamk_512 && !env().conv_streamk_x3_generic;   // shared-operand stages
+  const bool x3 = split_in;                                     // bf16x3: shared-operand stages
   const int taps = p->ksize * p->ksize, cchunks = (x3 ? p->Cin : b_cin) / 64, ksteps = taps * cchunks;
   const int lo_off = split_out ? (p->lo_off > 0 ? p->lo_off : p->Cout) : 0;
   if (split_out && ((lo_off & 7) != 0 || ldy < lo_off + p->Cout)) return Y2_OK;
-  int min_ksteps = x3 ? 6 : 18;                                 // short K: the epilogue starts to show (bf16x3 steps are 3x heavier)
-  if (env().conv_streamk_min_ksteps >= 0) min_ksteps = env().conv_streamk_min_ksteps;
+  const int min_ksteps = x3 ? 6 : 18;                           // short K: the epilogue starts to show (bf16x3 steps are 3x heavier)
   if (ksteps < min_ksteps || ksteps > SK_MAX_UNITS) return Y2_OK;
   int rc = load_driver_entry_points();
   if (rc != Y2_OK) return rc;
@@ -730,28 +464,18 @@ int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int
   a.M = (long long)p->N * p->H * p->W;
   a.H = p->H; a.W = p->W; a.ldy = ldy; a.pad = p->ksize / 2;
   a.cin_p = b_cin; a.cchunks = cchunks; a.ksteps = ksteps;
-  a.a_wrap = a_cin / 64;
   a.split_out = split_out ? 1 : 0;
   a.lo_off = lo_off;
   a.stats = out_f32 ? p->stats_slabs : nullptr;
   a.cout = p->Cout;
   fastdiv_init((uint32_t)cchunks, &a.fd_cc_mul, &a.fd_cc_shr);
   a.n_tiles = p->Cout / 256;
-  // CTA-pair kernel (cta_group::2) unless disabled; 512-row pair tiles (two halves per CTA) unless disabled or too few tiles
-  const bool two_cta = !env().conv_streamk_1cta && g_num_sms >= 2;
-  int halves = 1;
-  // 512-row pair tiles are opt-in (Y2_CONV_STREAMK_512=1): measured SLOWER on B200 (L19 149 vs 137 us, L6 116 vs 89 us) --
-  // the un-overlapped epilogue, the shallower 4-stage ring and the coarser tile quantisation cost more than the 1.33x
-  // fewer delivered bytes per flop bring
-  if (two_cta && env().conv_streamk_512) halves = 2;
-  const long long m_tiles = (a.M + 256 * halves - 1) / (256 * halves);
+  const long long m_tiles = (a.M + 255) / 256;
   a.tiles = (int)(m_tiles * a.n_tiles);
   a.units = (long long)a.tiles * ksteps;
   if ((a.tiles < g_num_sms / 2 && !env().conv_force_streamk) || a.units >= (1ll << 31) || a.M + 256 >= (1ll << 31)) return Y2_OK;
-  // every CTA's range must be at least one tile long (a tile is then shared by at most two CTAs)
-  // 74 pairs, every pair's range at least one tile long
+  // 74 pairs, every pair's range at least one tile long (a tile is then shared by at most two pairs)
   const int npairs = a.tiles < g_num_sms / 2 ? a.tiles : g_num_sms / 2;
-  const int grid = two_cta ? 2 * npairs : (a.tiles < g_num_sms ? a.tiles : g_num_sms);
   if (g_sk_ws_bytes < sk_workspace_bytes(g_num_sms)) return Y2_OK;
   a.ws_flags = reinterpret_cast<int*>(g_sk_ws);
   a.ws_partial = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(g_sk_ws) + SK_FLAG_BYTES);
@@ -761,12 +485,8 @@ int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int
   fastdiv_init((uint32_t)ksteps, &a.fd_ks_mul, &a.fd_ks_shr);
 
   if (dry) {
-    *handled = two_cta ? 2 : 1;
+    *handled = 1;
     return Y2_OK;
-  }
-  if (a.stats && !two_cta) {
-    set_error("y2_conv_fwd_bf16: stats_slabs needs the CTA-pair stream-K kernel (query y2_conv_stats_slab_rows first)");
-    return Y2_ERR_UNSUPPORTED;
   }
   CUtensorMap tmA, tmB;
   {
@@ -787,7 +507,7 @@ int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int
     const int Kp = taps * b_cin;
     cuuint64_t bdims[2] = {(cuuint64_t)Kp, (cuuint64_t)p->Cout};
     cuuint64_t bstrides[1] = {(cuuint64_t)Kp * 2};
-    cuuint32_t bbox[2] = {64, two_cta ? 128u : 256u};          // pair kernel: each CTA loads its half of the filters
+    cuuint32_t bbox[2] = {64, 128u};                           // each CTA of the pair loads its half of the filters
     cuuint32_t bestr[2] = {1, 1};
     r = g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p->w_packed), bdims, bstrides, bbox, bestr,
                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -798,42 +518,21 @@ int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int
     }
   }
   // (the flag area was zero when the workspace was registered -- the caller's contract -- and every launch leaves it zero)
-  if (two_cta) {
-    const size_t smem = (size_t)Sk2Cfg<1>::STAGES * Sk2Cfg<1>::STAGE + 8 * SK_STG_WARP + 1024;     // same for both variants
-    static_assert(Sk2Cfg<1>::STAGES * Sk2Cfg<1>::STAGE == Sk2Cfg<2>::STAGES * Sk2Cfg<2>::STAGE, "operand smem");
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(SK_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    cfg.attrs = attr;
-    cfg.numAttrs = fill_launch_attrs(attr, 2u);                 // (matches the kernels' __cluster_dims__)
-    if (x3) {
-      static_assert(Sk2Cfg<1, true>::STAGES * Sk2Cfg<1, true>::STAGE == Sk2Cfg<1>::STAGES * Sk2Cfg<1>::STAGE, "operand smem");
-      Y2_CUDA(cudaFuncSetAttribute((conv_streamk2_kernel<1, true>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      Y2_CUDA(cudaLaunchKernelEx(&cfg, (conv_streamk2_kernel<1, true>), tmA, tmB, a));
-    } else if (halves == 2) {
-      Y2_CUDA(cudaFuncSetAttribute(conv_streamk2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk2_kernel<2>, tmA, tmB, a));
-    } else {
-      Y2_CUDA(cudaFuncSetAttribute(conv_streamk2_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk2_kernel<1>, tmA, tmB, a));
-    }
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3((unsigned)(2 * npairs));
+  cfg.blockDim = dim3(SK_THREADS);
+  cfg.dynamicSmemBytes = SK2_SMEM;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[2];
+  cfg.attrs = attr;
+  cfg.numAttrs = fill_launch_attrs(attr, 2u);                   // (matches the kernel's __cluster_dims__)
+  if (x3) {
+    Y2_CUDA(cudaFuncSetAttribute(conv_streamk2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK2_SMEM));
+    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk2_kernel<true>, tmA, tmB, a));
   } else {
-    const size_t smem = (size_t)SK_STAGES * SK_STAGE + 8 * SK_STG_WARP + 1024;
-    Y2_CUDA(cudaFuncSetAttribute(conv_streamk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(SK_THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    cfg.attrs = attr;
-    cfg.numAttrs = fill_launch_attrs(attr, 1u);
-    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk_kernel, tmA, tmB, a));
+    Y2_CUDA(cudaFuncSetAttribute(conv_streamk2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK2_SMEM));
+    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk2_kernel<false>, tmA, tmB, a));
   }
   Y2_LAUNCHED();
   *handled = 1;

@@ -52,7 +52,6 @@ struct ConvArgs {
   uint32_t a_stage_bytes, b_stage_bytes;
   uint32_t a_sbo, a_lbo, b_sbo, b_lbo, layout_type, kstep_bytes;   // UMMA smem-descriptor fields (bytes)
   int first_layer;        // Cin_p == 8 special case (all taps in one stage, no swizzle)
-  int cluster;            // CTAs per cluster (1 or 2): B tile loaded in slices and multicast to the cluster
   int b_stationary;       // whole B operand resident in smem for the CTA's lifetime (n_tiles == 1, small B)
   uint32_t b_total_bytes;
   int sps;                // (tap, channel-chunk) sub-blocks per pipeline stage
@@ -85,12 +84,13 @@ struct TileCoord {
   long long m0;          // im2col: first flattened pixel index
 };
 
-// `unit` = scheduling unit (cluster == 1: tile index; cluster == 2: super-tile index), `crank` = CTA rank in cluster
+// `unit` = scheduling unit (CS == 1: tile index; CTA pair, CS == 2: index of two consecutive M tiles), `crank` = CTA rank
+template <int CS>
 __device__ __forceinline__ TileCoord decode_tile(const ConvArgs& a, int unit, uint32_t crank) {
   TileCoord t;
   const uint32_t mg = fdiv((uint32_t)unit, a.fd_ntiles_mul, a.fd_ntiles_shr);
   t.n_tile = unit - (int)mg * a.n_tiles;
-  const uint32_t mt = mg * (uint32_t)a.cluster + crank;      // may be >= m_tiles for the last group: all rows masked
+  const uint32_t mt = mg * (uint32_t)CS + crank;             // may be >= m_tiles for the last group: all rows masked
   if (a.a_mode == 0) {
     t.m0 = (long long)mt * TILE_M;                       // < 2^31 (checked on the host)
     const uint32_t m = t.m0 < a.M ? (uint32_t)t.m0 : 0u; // the empty half of a last pair loads valid pixels; its rows are masked
@@ -115,18 +115,12 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvArgs& a, int unit, ui
 // ------------------------------------------------------------------------------------------
 // the kernel
 // ------------------------------------------------------------------------------------------
-#ifndef Y2_EPI_GROUPS
-#define Y2_EPI_GROUPS 4
-#endif
-#ifndef Y2_PRODUCER_SINGLE
-#define Y2_PRODUCER_SINGLE 1
-#endif
 // Warp roles.  Epilogue = EPI_GROUPS groups of 4 warps (one warp per TMEM lane quarter, so the warp id modulo 4
 // must equal the quarter: epilogue warps come first).  The accumulator is multi-buffered in TMEM (NBUF tiles);
 // TP groups work on DIFFERENT tiles at the same time and CP groups split the columns of one tile
 // (EPI_GROUPS = TP * CP).  The SM's warp arbiter favours the highest warp id (B300_MICROARCH.md): the two
 // roles that feed the tensor pipe (TMA producer, MMA issuer) get the top ids so the epilogue cannot starve them.
-constexpr int EPI_GROUPS = Y2_EPI_GROUPS;
+constexpr int EPI_GROUPS = 4;
 constexpr int EPI_WARPS = 4 * EPI_GROUPS;
 constexpr int TC_THREADS = 64 + EPI_WARPS * 32;
 constexpr int WARP_PRODUCER = EPI_WARPS;
@@ -379,20 +373,17 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const uint32_t smem_base = smem_b_stat + (a.b_stationary ? ((a.b_total_bytes + 1023u) & ~1023u) : 0u);
   const uint32_t stage_bytes = a.a_stage_bytes + (a.b_stationary ? 0u : a.b_stage_bytes);
   const uint32_t tx_bytes = a.tx_bytes + (a.b_stationary ? 0u : a.b_stage_bytes);
-  // Work distribution.  cluster == 1: CTA b takes tiles b, b+grid, ...  cluster == 2: the CTA pair takes
-  // "super tiles" (two consecutive M tiles x one N tile); each CTA loads half of the B tile and multicasts
-  // it to both, which removes a third of the L2->SM operand traffic the kernel is bound by.
-  const int CS = a.cluster;
-  // CTA pair on one M = 256 MMA (see conv_streamk2_kernel for the why: the 64 B/clk smem operand path).  Each CTA keeps
-  // its own 128-pixel tile and HALF of the resident filter bank; the leader (rank 0) issues, both run producer + epilogue.
+  // Work distribution.  Single CTA: CTA b takes tiles b, b+grid, ...  CTA pair on one M = 256 MMA (see
+  // conv_streamk2_kernel for the why: the 64 B/clk smem operand path): the pair takes two consecutive M tiles x one N tile.
+  // Each CTA keeps its own 128-pixel tile and HALF of the filters; the leader (rank 0) issues, both run producer + epilogue.
   constexpr bool cta2 = CTA2;
+  constexpr int CS = CTA2 ? 2 : 1;                      // CTAs per cluster
   static_assert(!CTA2 || !FIRST, "no CTA-pair variant of the first-layer paths");
-  const uint32_t crank = CS > 1 ? cluster_ctarank() : 0u;
-  const int sched_first = CS > 1 ? (int)(blockIdx.x / CS) : (int)blockIdx.x;
-  const int sched_step = CS > 1 ? (int)(gridDim.x / CS) : (int)gridDim.x;
+  const uint32_t crank = CTA2 ? cluster_ctarank() : 0u;
+  const int sched_first = (int)(blockIdx.x / CS);
+  const int sched_step = (int)(gridDim.x / CS);
   const int m_groups = (a.m_tiles + CS - 1) / CS;
   const int total_tiles = m_groups * a.n_tiles;        // scheduling units (per cluster)
-  const uint16_t mc_mask = (uint16_t)((1u << CS) - 1u);
 
   if (warp == WARP_PRODUCER) {
     if (lane == 0) {
@@ -400,7 +391,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmB)) : "memory");
       for (int s = 0; s < a.stages; ++s) {
         mbar_init(&full_bar[s], 1);
-        mbar_init(&empty_bar[s], cta2 ? 1 : CS);        // every CTA of the cluster must release the stage (pair: one multicast commit)
+        mbar_init(&empty_bar[s], 1);                    // (pair: one multicast commit releases both CTAs' copies)
       }
       for (int b = 0; b < NBUF; ++b) {
         mbar_init(&tmem_full_bar[b], 1);
@@ -446,7 +437,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
   tc_fence_before();
   __syncthreads();
-  if (CS > 1) cluster_sync_all();                       // partner's barriers are initialised before any remote arrive
+  if constexpr (CTA2) cluster_sync_all();               // partner's barriers are initialised before any remote arrive
   tc_fence_after();
   const uint32_t tmem_base = s_tmem_base;
   pdl_wait();                                           // everything above overlapped the previous kernel's tail
@@ -480,7 +471,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int spt = (int)opaque((uint32_t)a.stages_per_tile);
     uint32_t ustage = 0, soffb = 0;                      // stage index and its byte offset
     for (int tile = sched_first; tile < total_tiles; tile += sched_step) {
-      const TileCoord t = decode_tile(a, tile, crank);
+      const TileCoord t = decode_tile<CS>(a, tile, crank);
       const int nrow0 = t.n_tile * BLOCK_N;
       for (int st = 0; st < spt; ++st) {
         const uint32_t bar = cta2 ? ((full0 + 8u * ustage) & PEER_BIT_MASK) : full0 + 8u * ustage;   // pair: the leader's barrier
@@ -527,15 +518,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               const int kh = lane - 1;
               if constexpr (cta2)      // pair, streamed filters: my half of the rows of tap (kh, kw), counted on the leader's barrier
                 tma_load_2d_2sm(sB + kh * a.b_sub_bytes, &tmB, bar, d.b_k + kh * 3 * a.cin_p, nrow0 + (int)crank * (BLOCK_N / 2));
-              else if (CS > 1)
-                tma_load_2d_mc(sB + kh * a.b_sub_bytes + crank * (a.b_sub_bytes / CS), &tmB, bar, d.b_k + kh * 3 * a.cin_p,
-                               nrow0 + (int)crank * (BLOCK_N / CS), mc_mask);
               else
                 tma_load_2d(sB + kh * a.b_sub_bytes, &tmB, bar, d.b_k + kh * 3 * a.cin_p, nrow0);
             }
           }
         } else {
-#if Y2_PRODUCER_SINGLE
           if (lane == 0) {
             for (int j = 0; j < sps; ++j) {
               const UnitDesc d = s_units[st * sps + j];
@@ -554,34 +541,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                                    (uint16_t)d.kw, (uint16_t)d.kh);
               else
                 tma_load_4d(sA + j * a.a_sub_bytes, &tmA, bar, d.a_c0, t.w0 + d.kw - a.pad, t.h0 + d.kh - a.pad, t.n0);
-              if (!a.b_stationary) {
-                if (CS > 1)
-                  tma_load_2d_mc(sB + j * a.b_sub_bytes + crank * (a.b_sub_bytes / CS), &tmB, bar, d.b_k,
-                                 nrow0 + (int)crank * (BLOCK_N / CS), mc_mask);
-                else
-                  tma_load_2d(sB + j * a.b_sub_bytes, &tmB, bar, d.b_k, nrow0);
-              }
+              if (!a.b_stationary) tma_load_2d(sB + j * a.b_sub_bytes, &tmB, bar, d.b_k, nrow0);
             }
           }
-#else
-          if (lane < 2 * sps) {
-            const int j = lane < sps ? lane : lane - sps;
-            const UnitDesc d = s_units[st * sps + j];
-            if (lane < sps) {
-              if constexpr (A_MODE == 0)
-                tma_load_im2col_4d(sA + j * a.a_sub_bytes, &tmA, bar, d.a_c0, t.w0 - a.pad, t.h0 - a.pad, t.n0,
-                                   (uint16_t)d.kw, (uint16_t)d.kh);
-              else
-                tma_load_4d(sA + j * a.a_sub_bytes, &tmA, bar, d.a_c0, t.w0 + d.kw - a.pad, t.h0 + d.kh - a.pad, t.n0);
-            } else if (!a.b_stationary) {
-              if (CS > 1)
-                tma_load_2d_mc(sB + j * a.b_sub_bytes + crank * (a.b_sub_bytes / CS), &tmB, bar, d.b_k,
-                               nrow0 + (int)crank * (BLOCK_N / CS), mc_mask);
-              else
-                tma_load_2d(sB + j * a.b_sub_bytes, &tmB, bar, d.b_k, nrow0);
-            }
-          }
-#endif
         }
         __syncwarp();
         ++ustage;
@@ -724,7 +686,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
         if (is_leader) {
           if constexpr (cta2) umma_commit_2sm_mc(empty_addr, (uint16_t)3);    // the pair's MMAs retired: both CTAs' copies of the stage are free
-          else if (CS > 1) umma_commit_mc_a(empty_addr, mc_mask);   // release the stage in every CTA of the cluster
           else umma_commit_a(empty_addr);                           // frees the smem stage when these MMAs retire
         }
         __syncwarp();
@@ -764,16 +725,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // scale/shift stalling (short scoreboard), the MMA warp's own LDS delayed, tensor pipe 48 % vs 71 %.
     constexpr bool tma_store = TMAST;
     static_assert(!TMAST || A_MODE == 2, "TMA-store epilogue: halo-patch mode only");
-    // a.tma_store == 2: ONE 8 KB buffer per group (32 KB instead of 64 KB of staging, one more operand stage for the bf16x3 layer
-    // 3); every box store then waits for the previous one's smem read
-    const bool stg_single = a.tma_store == 2;
-    const uint32_t stg_group = smem_b_stat + a.stg_offset + (uint32_t)gi * (stg_single ? 8192u : 16384u);
+    const uint32_t stg_group = smem_b_stat + a.stg_offset + (uint32_t)gi * 16384u;   // two 8 KB buffers per group
     uint32_t nstore = 0;
     for (int it = tp;; it += TP) {
       const int tile = sched_first + it * sched_step;
       if (tile >= total_tiles) break;
       const int buf = it % NBUF;
-      const TileCoord t = decode_tile(a, tile, crank);
+      const TileCoord t = decode_tile<CS>(a, tile, crank);
       const int nbase = t.n_tile * BLOCK_N;
       // ---- per-channel scale/shift of this n-tile -> smem (once per change of n-tile, per tile-parallel set) ----
       if (t.n_tile != staged_ntile) {
@@ -856,58 +814,42 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             ++nstore;
           }
          } else {
-          // bf16x3 output: the chunk leaves as TWO boxes, the hi halves at channel c0 and the lo halves at lo_off + c0 (the affine
-          // is evaluated again for the second box -- cheaper than keeping 32 more packed registers live)
-          const int nparts = a.split_out ? 2 : 1;
-#pragma unroll 1
-          for (int part = 0; part < nparts; ++part) {
-            const uint32_t stg = stg_group + (stg_single ? 0u : (nstore & 1u) * 8192u);
-            if (r == 0) {                                        // the store that last used this buffer has read it
-              if (stg_single) bulk_wait_group_read<0>();
-              else bulk_wait_group_read<1>();
-            }
-            asm volatile("bar.sync %0, 128;" ::"r"(8 + gi) : "memory");
-            // row r = h * 8 + w of the box, 64 B per row; 16-byte unit j (8 channels) at j ^ ((r >> 1) & 3)  (SWIZZLE_64B);
-            // one unit at a time: affine + leaky + pack + store, so that only the 32 accumulators stay live
+          // bf16 rows (not bf16x3: the hi / lo halves as two boxes per chunk were measured slower, see DESIGN.md)
+          const uint32_t stg = stg_group + (nstore & 1u) * 8192u;
+          if (r == 0) bulk_wait_group_read<1>();               // the store that last used this buffer has read it
+          asm volatile("bar.sync %0, 128;" ::"r"(8 + gi) : "memory");
+          // row r = h * 8 + w of the box, 64 B per row; 16-byte unit j (8 channels) at j ^ ((r >> 1) & 3)  (SWIZZLE_64B);
+          // one unit at a time: affine + leaky + pack + store, so that only the 32 accumulators stay live
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              float f[8];
+          for (int j = 0; j < 4; ++j) {
+            float f[8];
 #pragma unroll
-              for (int h = 0; h < 2; ++h) {
-                const int i = 8 * j + 4 * h;
-                const float4 sc = *reinterpret_cast<const float4*>(&my_scale[cc + i]);
-                const float4 sh = *reinterpret_cast<const float4*>(&my_shift[cc + i]);
-                float f0 = fmaf(__uint_as_float(v[i + 0]), sc.x, sh.x), f1 = fmaf(__uint_as_float(v[i + 1]), sc.y, sh.y);
-                float f2 = fmaf(__uint_as_float(v[i + 2]), sc.z, sh.z), f3 = fmaf(__uint_as_float(v[i + 3]), sc.w, sh.w);
-                if (leaky_on) {
-                  f0 = fmaxf(f0, a.alpha * f0); f1 = fmaxf(f1, a.alpha * f1);
-                  f2 = fmaxf(f2, a.alpha * f2); f3 = fmaxf(f3, a.alpha * f3);
-                }
-                f[4 * h] = f0; f[4 * h + 1] = f1; f[4 * h + 2] = f2; f[4 * h + 3] = f3;
+            for (int h = 0; h < 2; ++h) {
+              const int i = 8 * j + 4 * h;
+              const float4 sc = *reinterpret_cast<const float4*>(&my_scale[cc + i]);
+              const float4 sh = *reinterpret_cast<const float4*>(&my_shift[cc + i]);
+              float f0 = fmaf(__uint_as_float(v[i + 0]), sc.x, sh.x), f1 = fmaf(__uint_as_float(v[i + 1]), sc.y, sh.y);
+              float f2 = fmaf(__uint_as_float(v[i + 2]), sc.z, sh.z), f3 = fmaf(__uint_as_float(v[i + 3]), sc.w, sh.w);
+              if (leaky_on) {
+                f0 = fmaxf(f0, a.alpha * f0); f1 = fmaxf(f1, a.alpha * f1);
+                f2 = fmaxf(f2, a.alpha * f2); f3 = fmaxf(f3, a.alpha * f3);
               }
-              uint4 pk;
-              if (a.split_out) {
-                uint4 hi, lo;
-                split8_bf16(f, hi, lo);
-                pk = part ? lo : hi;
-              } else {
-                const __nv_bfloat162 h0 = __floats2bfloat162_rn(f[0], f[1]), h1 = __floats2bfloat162_rn(f[2], f[3]);
-                const __nv_bfloat162 h2 = __floats2bfloat162_rn(f[4], f[5]), h3 = __floats2bfloat162_rn(f[6], f[7]);
-                pk = make_uint4(*reinterpret_cast<const uint32_t*>(&h0), *reinterpret_cast<const uint32_t*>(&h1),
-                                *reinterpret_cast<const uint32_t*>(&h2), *reinterpret_cast<const uint32_t*>(&h3));
-              }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + (uint32_t)r * 64u + (uint32_t)((j ^ ((r >> 1) & 3)) << 4)),
-                           "r"(pk.x), "r"(pk.y), "r"(pk.z), "r"(pk.w)
-                           : "memory");
+              f[4 * h] = f0; f[4 * h + 1] = f1; f[4 * h + 2] = f2; f[4 * h + 3] = f3;
             }
-            fence_proxy_async_smem();
-            asm volatile("bar.sync %0, 128;" ::"r"(8 + gi) : "memory");
-            if (r == 0) {
-              tma_store_4d(&tmY, stg, c0 + part * a.lo_off, t.w0, t.h0, t.n0);   // rows / pixels outside the tensor are clipped by the TMA unit
-              bulk_commit_group();
-            }
-            ++nstore;
+            const __nv_bfloat162 h0 = __floats2bfloat162_rn(f[0], f[1]), h1 = __floats2bfloat162_rn(f[2], f[3]);
+            const __nv_bfloat162 h2 = __floats2bfloat162_rn(f[4], f[5]), h3 = __floats2bfloat162_rn(f[6], f[7]);
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stg + (uint32_t)r * 64u + (uint32_t)((j ^ ((r >> 1) & 3)) << 4)),
+                         "r"(*reinterpret_cast<const uint32_t*>(&h0)), "r"(*reinterpret_cast<const uint32_t*>(&h1)),
+                         "r"(*reinterpret_cast<const uint32_t*>(&h2)), "r"(*reinterpret_cast<const uint32_t*>(&h3))
+                         : "memory");
           }
+          fence_proxy_async_smem();
+          asm volatile("bar.sync %0, 128;" ::"r"(8 + gi) : "memory");
+          if (r == 0) {
+            tma_store_4d(&tmY, stg, c0, t.w0, t.h0, t.n0);     // rows / pixels outside the tensor are clipped by the TMA unit
+            bulk_commit_group();
+          }
+          ++nstore;
          }
         } else if (A_MODE != 0 && pool && !out_f32 && c0 + 32 <= a.Cout && (a.ldy & 7) == 0 && (a.lo_off & 7) == 0) {
           epilogue_chunk_pooled_bf16(a, v, my_scale, my_shift, cc, c0, valid_px, orow, leaky_on, lane);
@@ -925,7 +867,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   // ---- teardown ----
   tc_fence_before();
   __syncthreads();
-  if (CS > 1) cluster_sync_all();                       // nobody exits while a partner may still write/signal here
+  if constexpr (CTA2) cluster_sync_all();               // nobody exits while a partner may still write/signal here
   if (warp == WARP_MMA) {
     __syncwarp();
     tc_fence_after();
@@ -1278,7 +1220,7 @@ template <int BLOCK_N, int A_MODE, int KIND, bool CTA2 = false, bool TMAST = fal
 static int launch_conv3(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmY, const ConvArgs& a, size_t smem, cudaStream_t st) {
   Y2_CUDA(cudaFuncSetAttribute((conv_tc_kernel<BLOCK_N, A_MODE, KIND, CTA2, TMAST>), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                (int)smem));
-  const int CS = a.cluster;
+  constexpr int CS = CTA2 ? 2 : 1;
   long long units = (long long)((a.m_tiles + CS - 1) / CS) * a.n_tiles;
   long long want = units * CS;
   int grid = (int)(want < g_num_sms ? want : g_num_sms);
@@ -1386,7 +1328,7 @@ static int conv_is_try(const y2_conv_params* p, cudaStream_t st, int* handled) {
   // un-pooled outputs leave through 32 KB of staging + TMA box stores when at least three ring stages remain next to it
   const size_t IS_STG = 4 * 8192;
   a.tma_store = 0;
-  if (!pool && !env().conv_is_no_tma_store && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(p->y) & 15) == 0 &&
+  if (!pool && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(p->y) & 15) == 0 &&
       (!split_out || a.lo_off % 8 == 0) && (SMEM_BUDGET - b_region - IS_STG) / stage_bytes >= 3)
     a.tma_store = 1;
   const size_t stg_bytes = a.tma_store ? IS_STG : 0;
@@ -1462,7 +1404,7 @@ extern "C" int y2_conv_stats_slab_rows(const y2_conv_params* p) {
   if (!p || !(p->flags & Y2_CONV_OUT_F32) || load_driver_entry_points() != Y2_OK) return 0;
   int handled = 0;
   if (conv_streamk_try(p, nullptr, &handled, 1) != Y2_OK) return 0;
-  return handled == 2 ? 32 : 0;
+  return handled ? 32 : 0;
 }
 
 extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
@@ -1537,8 +1479,7 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   if (env().conv_force_tiled) a.a_mode = 1;
   // halo-patch mode for 3x3 layers on large maps: an 8 x 16 pixel tile whose (16+2)-row neighbourhood is
   // loaded once per horizontal tap (first layer: once in total) instead of once per tap
-  if (p->ksize == 3 && p->H >= 64 && p->W >= 64 && !env().conv_no_patch) a.a_mode = 2;
-  if (env().conv_force_patch && p->ksize == 3) a.a_mode = 2;
+  if (p->ksize == 3 && p->H >= 64 && p->W >= 64) a.a_mode = 2;
   int TW = 1, TH = 1, NB = 128;
   if (a.a_mode == 2) {
     TW = 8; TH = 16; NB = 1;
@@ -1567,10 +1508,6 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   }
   // halo-patch mode keeps three taps of B per stage: 256-wide tiles would leave room for a single stage
   if (a.a_mode == 2 && block_n == 256) block_n = 128;
-  if (env().conv_block_n) {
-    int v = env().conv_block_n;
-    if ((v == 128 || v == 256) && cout_p >= v && !a.first_layer) block_n = v;
-  }
   a.n_tiles = (cout_p + block_n - 1) / block_n;
   if (a.first_layer) {
     a.a_stage_bytes = 10 * TILE_M * 16;
@@ -1628,7 +1565,7 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
       a.cta2 = 1;
       a.b_sub_bytes = half;
       a.b_stage_bytes = 3 * half;
-    } else if (!env().conv_no_bstat) {
+    } else {
       // the bank does not fit (bf16x3: three times the K extent): still a pair, each CTA STREAMING its half of the three
       // taps' filter rows next to its patch -- (4096 + 16 N) / 64 clk per MMA instead of the single CTA's (4096 + 32 N) / 64
       a.cta2 = 1;
@@ -1639,37 +1576,28 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   }
   // ... and for the im2col / tiled-box modes with 128-byte rows and >= 128-wide tiles (pooled 52x52 / 26x26 layers, the
   // 1x1 layers): the filter tile is streamed, each CTA fetching its half of the rows per stage
-  if (a.a_mode != 2 && !a.first_layer && a.row_bytes == 128 && block_n >= 128 && a.m_tiles >= 2 && !env().conv_no_cta2 &&
-      !env().conv_no_cta2_generic && !env().conv_cluster) {
+  if (a.a_mode != 2 && !a.first_layer && a.row_bytes == 128 && block_n >= 128 && a.m_tiles >= 2 && !env().conv_no_cta2) {
     a.cta2 = 1;
     a.b_sub_bytes = (uint32_t)(block_n / 2) * a.row_bytes;
     a.b_stage_bytes = (uint32_t)a.sps * a.b_sub_bytes;
   }
   // B-stationary: with a single N tile and a small filter bank, every tile of the CTA needs the same B
   a.b_total_bytes = a.first_layer ? a.b_sub_bytes : (uint32_t)a.kblocks * a.b_sub_bytes;
-  a.b_stationary = (a.n_tiles == 1 && a.b_total_bytes + 4 * (size_t)a.a_stage_bytes <= SMEM_BUDGET &&
-                    !env().conv_no_bstat && !cta2_streamed) ? 1 : 0;
+  a.b_stationary = (a.n_tiles == 1 && a.b_total_bytes + 4 * (size_t)a.a_stage_bytes <= SMEM_BUDGET && !cta2_streamed) ? 1 : 0;
   // halo-patch mode with a resident filter bank and a single channel chunk (layer 2: Cin = 32): the three
   // horizontally shifted patches share ONE stage, so the MMA warp issues all 9 taps behind one barrier round trip.
   // With one patch per stage that warp's ~800 clk of per-stage bookkeeping hid 192 clk of tensor work (ncu, r1c).
   if (a.a_mode == 2 && !a.first_layer && a.b_stationary && (a.cchunks == 1 || split_in) &&
-      a.b_total_bytes + 3 * (size_t)(3 * a.a_sub_bytes) <= SMEM_BUDGET && !env().conv_no_kwmerge) {
+      a.b_total_bytes + 3 * (size_t)(3 * a.a_sub_bytes) <= SMEM_BUDGET) {
     a.kw_merge = 1;                                      // (several chunks -- the bf16x3 K extent -- : one merged stage per chunk)
     a.a_stage_bytes = 3 * a.a_sub_bytes;
     a.stages_per_tile = a.cchunks;
     a.tx_bytes = a.a_stage_bytes;
   }
-  // CTA pairs with B multicast (opt-in, Y2_CONV_CLUSTER=1): each CTA fetches half of the B tile for both.
-  // Measured on B200 it is ~15% SLOWER than independent CTAs: the kernel is bound by bytes delivered into
-  // each SM (~49 B/clk/SM), which multicast does not reduce -- see DESIGN.md.
-  a.cluster = a.cta2 ? 2 : 1;
   if (a.cta2 && a.a_mode == 2 && !a.b_stationary && !cta2_streamed) {
     set_error("y2_conv_fwd_bf16: internal: halo-patch CTA-pair mode without a resident filter bank");
     return Y2_ERR_UNSUPPORTED;
   }
-  if (!a.first_layer && !a.b_stationary && a.m_tiles >= 2 && (a.b_sub_bytes / 2) % 1024 == 0 && block_n >= 64 &&
-      env().conv_cluster)
-    a.cluster = 2;
   // stages: B-stage must stay 1024-byte aligned for the 128B swizzle atoms
   uint32_t stage_bytes = a.a_stage_bytes + (a.b_stationary ? 0u : a.b_stage_bytes);
   Y2_ARG(a.first_layer || (a.a_stage_bytes % 1024 == 0 && a.b_stage_bytes % 1024 == 0));
@@ -1677,13 +1605,13 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   // TMA-store epilogue for the un-pooled 128-channel bf16 output of the halo-patch pair kernel (layer 3): 4 groups x 2 x 8 KB
   // of staging.  (Measured: layer 3 108 -> 93 us; the 64-channel layer 4 got slower -- two chunks per tile do not amortise
   // the per-chunk group barriers and the ring loses four stages -- so it keeps the direct stores.)
-  // (bf16x3: the hi / lo halves as two boxes per chunk -- implemented, opt-in Y2_CONV_TMA_STORE_SPLIT=1: the 64 KB of staging
-  // leaves 3 instead of 5 operand stages next to the streamed filters and layer 3 got SLOWER, 308 -> 325 us.)
+  // (bf16x3: the hi / lo halves as two boxes per chunk were measured: the 64 KB of staging leaves 3 instead of 5 operand
+  // stages next to the streamed filters and layer 3 got SLOWER, 308 -> 325 us -- it keeps the direct stores.)
   const size_t STG_BYTES = 4 * 2 * 8192;
   a.tma_store = 0;
   {
     const bool common = a.a_mode == 2 && !pool && p->Cout % 32 == 0 && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(p->y) & 15) == 0 &&
-                        EPI_GROUPS == 4 && b_region + 3 * (size_t)stage_bytes + STG_BYTES <= SMEM_BUDGET && !env().conv_no_tma_store;
+                        b_region + 3 * (size_t)stage_bytes + STG_BYTES <= SMEM_BUDGET;
     // bf16 rows: the 128-channel pair kernel (layer 3); float32 rows (training forward): also the first layer and the 64-channel
     // pair kernel (layer 2), whose 16-byte per-lane stores cost far more than the bf16 ones
     const bool shape_bf16 = !a.first_layer && block_n == 128 && a.row_bytes == 128 && a.cta2;
@@ -1691,15 +1619,9 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
                            (!a.first_layer && block_n == 64 && a.row_bytes == 64 && a.cta2 && p->Cout == 64);
     // (64 columns on 128-byte operand rows -- layer 4 without the input-stationary kernel: 131 -> 141 us, not enabled)
     if (common && !out_f32 && shape_bf16 && !split_out) a.tma_store = 1;
-    if (!out_f32 && split_out && shape_bf16 && a.lo_off % 8 == 0 && env().conv_tma_store_split) {
-      const size_t stg = env().conv_tma_store_split == 2 ? STG_BYTES / 2 : STG_BYTES;
-      if (a.a_mode == 2 && !pool && p->Cout % 32 == 0 && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(p->y) & 15) == 0 &&
-          EPI_GROUPS == 4 && b_region + 3 * (size_t)stage_bytes + stg <= SMEM_BUDGET && !env().conv_no_tma_store)
-        a.tma_store = env().conv_tma_store_split == 2 ? 2 : 1;
-    }
     if (common && out_f32 && shape_f32 && !env().conv_no_tma_store_f32) a.tma_store = 1;
   }
-  const size_t stg_bytes = a.tma_store == 2 ? STG_BYTES / 2 : (a.tma_store ? STG_BYTES : 0);
+  const size_t stg_bytes = a.tma_store ? STG_BYTES : 0;
   int stages = (int)((SMEM_BUDGET - b_region - stg_bytes) / stage_bytes);
   if (stages > 12) stages = 12;
   if (stages < 2) {
@@ -1776,7 +1698,7 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
       const int Kp = taps * a.cin_p;
       cuuint64_t dims[2] = {(cuuint64_t)Kp, (cuuint64_t)cout_p};
       cuuint64_t strides[1] = {(cuuint64_t)Kp * 2};
-      cuuint32_t box[2] = {(cuuint32_t)a.kchunk, (cuuint32_t)(block_n / a.cluster)};   // per-CTA slice of the B tile
+      cuuint32_t box[2] = {(cuuint32_t)a.kchunk, (cuuint32_t)(a.cta2 ? block_n / 2 : block_n)};   // per-CTA slice of the B tile
       r = g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p->w_packed), dims, strides, box,
                         estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1792,7 +1714,7 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
     // output [N, H, W, Cout] with row stride ldy: boxes of 32 channels x the 8 x 16 pixel tile, 64-byte swizzled rows
     // (float32 rows: boxes of 16 channels -- the same 64 bytes per row)
     const cuuint64_t es = out_f32 ? 4 : 2;
-    cuuint64_t dims[4] = {(cuuint64_t)(split_out ? a.lo_off + p->Cout : p->Cout), (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
+    cuuint64_t dims[4] = {(cuuint64_t)p->Cout, (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
     cuuint64_t strides[3] = {(cuuint64_t)a.ldy * es, (cuuint64_t)p->W * a.ldy * es, (cuuint64_t)p->H * p->W * a.ldy * es};
     cuuint32_t box[4] = {out_f32 ? 16u : 32u, 8, 16, 1};
     cuuint32_t estr[4] = {1, 1, 1, 1};

@@ -41,23 +41,16 @@ __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, 
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
-// CTA2: CTA-pair variant (tcgen05 cta_group::2, see conv_streamk_tcgen05.cu for the why).  The pair computes TWO M tiles
-// (rank r: tile 2 * mp + r) against the SAME dh columns with M = 256 MMAs: each CTA loads its own (tap, channel) atoms and
-// HALF of the dh atoms, so a K stage delivers 32 KB per SM instead of 48 KB for the same flops (the single-CTA kernel asks
-// the L2 for 17 TB/s at N = 256 -- more than it delivers) and an MMA fetches 8 KB instead of 12 KB of operands from smem.
-// Both producers signal the LEADER's full barrier; the leader issues and commits with a multicast to both CTAs; each CTA's
-// epilogue drains its own 128 accumulator rows.
 // G: M tiles per scheduling unit that share ONE pass over the dh columns (G accumulators of BLOCK_N columns per TMEM buffer).
 // The early layers have few output rows (taps x Cin = 288 .. 1152) and millions of pixels: with one M tile per unit the
 // activations are fetched once per tap group and dh once per M tile -- 2.6 GB of DRAM traffic for layer 2's 0.5 GB of operands
 // (x and dh no longer fit the L2), which made those layers HBM-bound at 250-500 TFLOP/s.  With G tiles per unit a K stage
 // loads dh once and the G tiles' (spatially overlapping) taps of the same pixels together.
-template <int BLOCK_N, int ATOM_BYTES, bool CTA2 = false, int G = 1>
+template <int BLOCK_N, int ATOM_BYTES, int G = 1>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmG, const WgradArgs a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   constexpr int NBUF = 2;
-  static_assert(!CTA2 || G == 1, "tile groups: single-CTA kernel only");
   static_assert(NBUF * G * BLOCK_N <= 512, "TMEM has 512 columns");
   constexpr uint32_t TMEM_COLS = NBUF * G * BLOCK_N <= 128 ? 128 : (NBUF * G * BLOCK_N <= 256 ? 256 : 512);
   __shared__ __align__(8) uint64_t full_bar[WG_MAX_STAGES];
@@ -68,35 +61,25 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t smem_base = (smem_u32(smem) + 1023u) & ~1023u;
-  const uint32_t stage_bytes = a.a_stage_bytes + a.b_stage_bytes;          // per CTA (pair: own A atoms + half of the dh atoms)
-  const uint32_t crank = CTA2 ? cluster_ctarank() : 0u;
-  const int m_groups = CTA2 ? (a.m_tiles + 1) / 2 : (a.m_tiles + G - 1) / G;   // scheduling units along M (pair: two tiles; G tiles)
+  const uint32_t stage_bytes = a.a_stage_bytes + a.b_stage_bytes;
+  const int m_groups = (a.m_tiles + G - 1) / G;                            // scheduling units along M (G tiles each)
   const int total_units = m_groups * a.n_tiles * a.splits;
-  const int unit0 = CTA2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, unit_step = CTA2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-  const int my_atoms = CTA2 ? a.n_atoms / 2 : a.n_atoms;                   // dh atoms this CTA loads
+  const int unit0 = (int)blockIdx.x, unit_step = (int)gridDim.x;
 
   if (warp == WG_WARP_PRODUCER && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmX)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmG)) : "memory");
     for (int s = 0; s < a.stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-    for (int b = 0; b < NBUF; ++b) { mbar_init(&tmem_full_bar[b], 1); mbar_init(&tmem_empty_bar[b], CTA2 ? 8 : 4); }
+    for (int b = 0; b < NBUF; ++b) { mbar_init(&tmem_full_bar[b], 1); mbar_init(&tmem_empty_bar[b], 4); }
     fence_barrier_init();
   }
   if (warp == WG_WARP_MMA) {
-    if constexpr (CTA2) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem_base)), "r"(TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem_base)),
-                   "r"(TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem_base)), "r"(TMEM_COLS)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (CTA2) cluster_sync_all();               // the partner's barriers exist before anything signals them
   tc_fence_after();
   const uint32_t tmem_base = s_tmem_base;
 
@@ -108,9 +91,9 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
       const uint32_t q1 = fdiv((uint32_t)unit, a.fd_nt_mul, a.fd_nt_shr);
       const int nt = unit - (int)q1 * a.n_tiles;
       const uint32_t sp = fdiv(q1, a.fd_mt_mul, a.fd_mt_shr);
-      const int mt = ((int)q1 - (int)sp * m_groups) * (CTA2 ? 2 : G) + (int)crank;        // first M tile of the unit
+      const int mt = ((int)q1 - (int)sp * m_groups) * G;                                 // first M tile of the unit
       const int ks0 = (int)(((long long)sp * a.kstages) / a.splits), ks1 = (int)(((long long)(sp + 1) * a.kstages) / a.splits);
-      // my load: lanes [0, G * slots) fetch A atoms (tile mt + lane / slots), the next my_atoms lanes fetch B atoms
+      // my load: lanes [0, G * slots) fetch A atoms (tile mt + lane / slots), the next n_atoms lanes fetch B atoms
       const int a_lanes = G * a.slots;
       int kw = 0, kh = 0, c0 = 0;
       if (lane < a_lanes) {
@@ -121,32 +104,26 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
         kh = (int)fdiv((uint32_t)tap, a.fd_k_mul, a.fd_k_shr);
         kw = tap - kh * a.ksize;
       } else {
-        c0 = nt * BLOCK_N + ((int)crank * my_atoms + (lane - a_lanes)) * 64;        // pair: my half of the dh columns
+        c0 = nt * BLOCK_N + (lane - a_lanes) * 64;
       }
       for (int ks = ks0; ks < ks1; ++ks) {
         if (lane == 0) {
           mbar_wait(&empty_bar[stage], phase ^ 1u);
-          if (!CTA2) mbar_expect_tx(&full_bar[stage], stage_bytes);
-          else if (crank == 0) mbar_expect_tx(&full_bar[stage], 2u * stage_bytes);   // both CTAs' loads land on the leader's barrier
+          mbar_expect_tx(&full_bar[stage], stage_bytes);
         }
         __syncwarp();
         const uint32_t p0 = (uint32_t)ks * (uint32_t)a.kp;
         const uint32_t sA = smem_base + stage * stage_bytes;
-        const uint32_t bar = CTA2 ? (smem_u32(&full_bar[stage]) & PEER_BIT_MASK) : smem_u32(&full_bar[stage]);
+        const uint32_t bar = smem_u32(&full_bar[stage]);
         if (lane < a_lanes) {
           const uint32_t row = fdiv(p0, a.fd_w_mul, a.fd_w_shr);          // n*H + h
           const int w0 = (int)(p0 - row * (uint32_t)a.W);
           const uint32_t img = fdiv(row, a.fd_h_mul, a.fd_h_shr);
           const int h0 = (int)(row - img * (uint32_t)a.H);
-          if constexpr (CTA2)
-            tma_load_im2col_4d_2sm(sA + lane * (a.kp * ATOM_BYTES), &tmX, bar, c0, w0 - a.pad, h0 - a.pad, (int)img, (uint16_t)kw,
-                                   (uint16_t)kh);
-          else
-            tma_load_im2col_4d(sA + lane * (a.kp * ATOM_BYTES), &tmX, bar, c0, w0 - a.pad, h0 - a.pad, (int)img, (uint16_t)kw,
-                               (uint16_t)kh);
-        } else if (lane < a_lanes + my_atoms) {
-          if constexpr (CTA2) tma_load_2d_2sm(sA + a.a_stage_bytes + (lane - a_lanes) * (a.kp * 128), &tmG, bar, c0, (int)p0);
-          else tma_load_2d(sA + a.a_stage_bytes + (lane - a_lanes) * (a.kp * 128), &tmG, bar, c0, (int)p0);
+          tma_load_im2col_4d(sA + lane * (a.kp * ATOM_BYTES), &tmX, bar, c0, w0 - a.pad, h0 - a.pad, (int)img, (uint16_t)kw,
+                             (uint16_t)kh);
+        } else if (lane < a_lanes + a.n_atoms) {
+          tma_load_2d(sA + a.a_stage_bytes + (lane - a_lanes) * (a.kp * 128), &tmG, bar, c0, (int)p0);
         }
         __syncwarp();
         if (++stage == a.stages) { stage = 0; phase ^= 1u; }
@@ -158,7 +135,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
     asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(is_leader));
     // D = f32, A = B = bf16, both MN-major (bits 15, 16), N, M = 128
     constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
-                               ((uint32_t)(BLOCK_N >> 3) << 17) | ((uint32_t)((CTA2 ? 256 : 128) >> 4) << 24);
+                               ((uint32_t)(BLOCK_N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
     constexpr uint32_t a_layout = ATOM_BYTES == 128 ? 2u : 4u;
     // MN-major canonical layout: LBO = byte distance between swizzle atoms along M/N, SBO = between 8-pixel groups
     const uint64_t adesc0 = make_smem_desc(smem_base, (uint32_t)(a.kp * ATOM_BYTES), 8u * ATOM_BYTES, a_layout);
@@ -169,7 +146,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
     int stage = 0;
     uint32_t phase = 0;
     int it = 0;
-    for (int unit = unit0; unit < ((!CTA2 || crank == 0) ? total_units : 0); unit += unit_step, ++it) {     // pair: the leader issues
+    for (int unit = unit0; unit < total_units; unit += unit_step, ++it) {
       const uint32_t q1 = fdiv((uint32_t)unit, a.fd_nt_mul, a.fd_nt_shr);
       const uint32_t sp = fdiv(q1, a.fd_mt_mul, a.fd_mt_shr);
       const int ks0 = (int)(((long long)sp * a.kstages) / a.splits), ks1 = (int)(((long long)(sp + 1) * a.kstages) / a.splits);
@@ -185,26 +162,18 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
         if (is_leader) {
           const uint64_t ad = adesc0 + (uint32_t)stage * stage16, bd = bdesc0 + (uint32_t)stage * stage16;
           for (int k = 0; k < ksteps; ++k) {
-            if constexpr (CTA2) {
-              umma_bf16_2sm(tmem_d, ad + (uint32_t)k * a_kstep, bd + (uint32_t)k * b_kstep, idesc, accum);
-            } else {
 #pragma unroll
-              for (int gi = 0; gi < G; ++gi)
-                umma_bf16(tmem_d + (uint32_t)(gi * BLOCK_N), ad + (uint32_t)gi * a_tile16 + (uint32_t)k * a_kstep,
-                          bd + (uint32_t)k * b_kstep, idesc, accum);
-            }
+            for (int gi = 0; gi < G; ++gi)
+              umma_bf16(tmem_d + (uint32_t)(gi * BLOCK_N), ad + (uint32_t)gi * a_tile16 + (uint32_t)k * a_kstep,
+                        bd + (uint32_t)k * b_kstep, idesc, accum);
             accum = 1;
           }
-          if constexpr (CTA2) umma_commit_2sm_mc(smem_u32(&empty_bar[stage]), (uint16_t)3);   // both CTAs' copies of the stage are free
-          else umma_commit(&empty_bar[stage]);
+          umma_commit(&empty_bar[stage]);
         }
         __syncwarp();
         if (++stage == a.stages) { stage = 0; phase ^= 1u; }
       }
-      if (is_leader) {
-        if constexpr (CTA2) umma_commit_2sm_mc(smem_u32(&tmem_full_bar[buf]), (uint16_t)3);
-        else umma_commit(&tmem_full_bar[buf]);
-      }
+      if (is_leader) umma_commit(&tmem_full_bar[buf]);
       __syncwarp();
     }
   } else {
@@ -217,7 +186,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
       const uint32_t q1 = fdiv((uint32_t)unit, a.fd_nt_mul, a.fd_nt_shr);
       const int nt = unit - (int)q1 * a.n_tiles;
       const uint32_t sp = fdiv(q1, a.fd_mt_mul, a.fd_mt_shr);
-      const int mt0 = ((int)q1 - (int)sp * m_groups) * (CTA2 ? 2 : G) + (int)crank;
+      const int mt0 = ((int)q1 - (int)sp * m_groups) * G;
       const int buf = it & 1;
       mbar_wait(&tmem_full_bar[buf], ((uint32_t)it >> 1) & 1u);
       tc_fence_after();
@@ -238,10 +207,7 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
         if (cc + 32 >= BLOCK_N && gi == G - 1) {
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) {
-            if constexpr (CTA2) mbar_arrive_cluster(smem_u32(&tmem_empty_bar[buf]) & PEER_BIT_MASK);   // the leader's barrier counts both CTAs
-            else mbar_arrive(&tmem_empty_bar[buf]);
-          }
+          if (lane == 0) mbar_arrive(&tmem_empty_bar[buf]);
         }
         const int col0 = nt * BLOCK_N + cc;
         if (valid && col0 < a.Cout) {
@@ -264,50 +230,23 @@ conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_const
 
   tc_fence_before();
   __syncthreads();
-  if constexpr (CTA2) cluster_sync_all();               // nobody frees TMEM / exits while the partner's MMAs or arrives are in flight
   if (warp == WG_WARP_MMA) {
     __syncwarp();
     tc_fence_after();
-    if constexpr (CTA2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
   }
 }
 
 template <int BLOCK_N, int ATOM_BYTES>
-static int launch_wgrad(const CUtensorMap& tmX, const CUtensorMap& tmG, const WgradArgs& a, size_t smem, cudaStream_t st, bool cta2,
-                        int group) {
+static int launch_wgrad(const CUtensorMap& tmX, const CUtensorMap& tmG, const WgradArgs& a, size_t smem, cudaStream_t st, int group) {
   if constexpr (BLOCK_N <= 128) {
     constexpr int GG = BLOCK_N == 64 ? 3 : 2;
     if (group == GG) {
-      Y2_CUDA(cudaFuncSetAttribute((conv_wgrad_tc_kernel<BLOCK_N, ATOM_BYTES, false, GG>), cudaFuncAttributeMaxDynamicSharedMemorySize,
+      Y2_CUDA(cudaFuncSetAttribute((conv_wgrad_tc_kernel<BLOCK_N, ATOM_BYTES, GG>), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)smem));
       const int units = ((a.m_tiles + GG - 1) / GG) * a.n_tiles * a.splits;
       const int grid = units < g_num_sms ? units : g_num_sms;
-      conv_wgrad_tc_kernel<BLOCK_N, ATOM_BYTES, false, GG><<<grid, WG_THREADS, smem, st>>>(tmX, tmG, a);
-      Y2_LAUNCHED();
-      return Y2_OK;
-    }
-  }
-  if constexpr (BLOCK_N >= 128) {
-    if (cta2) {
-      Y2_CUDA(cudaFuncSetAttribute((conv_wgrad_tc_kernel<BLOCK_N, ATOM_BYTES, true>), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)smem));
-      const int units = ((a.m_tiles + 1) / 2) * a.n_tiles * a.splits;
-      const int pairs = units < g_num_sms / 2 ? units : g_num_sms / 2;
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3((unsigned)(2 * pairs));
-      cfg.blockDim = dim3(WG_THREADS);
-      cfg.dynamicSmemBytes = smem;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];                   // (cluster only: this kernel has no griddepcontrol.wait, so no programmatic launch)
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 2;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      Y2_CUDA(cudaLaunchKernelEx(&cfg, (conv_wgrad_tc_kernel<BLOCK_N, ATOM_BYTES, true>), tmX, tmG, a));
+      conv_wgrad_tc_kernel<BLOCK_N, ATOM_BYTES, GG><<<grid, WG_THREADS, smem, st>>>(tmX, tmG, a);
       Y2_LAUNCHED();
       return Y2_OK;
     }
@@ -353,36 +292,31 @@ extern "C" int y2_conv_wgrad_bf16(const void* x, const void* dh, int ld_dh, floa
   a.n_atoms = block_n / 64;
   a.kp = 64;
   a.kstages = (int)((a.M + a.kp - 1) / a.kp);
-  // CTA pairs (two M tiles against the same dh columns, each CTA loading half of the dh atoms) when there are two atoms to
-  // share and two M tiles to pair
   // tile groups for the narrow layers (block_n 64: three M tiles per unit, 128: two) with many pixels per output row
   int group = 1;
-  if (!env().wgrad_no_group && ksize == 3 && a.m_tiles >= 2 && a.M >= 2048) group      // (1x1 layers: measured slower)
+  if (ksize == 3 && a.m_tiles >= 2 && a.M >= 2048) group      // (1x1 layers: measured slower)
     = block_n == 64 ? 3 : (block_n == 128 ? 2 : 1);
-  const bool cta2 = group == 1 && block_n >= 128 && a.m_tiles >= 2 && g_num_sms >= 2 && env().wgrad_cta2;   // opt-in: no gain measured
   a.a_stage_bytes = (uint32_t)(group * a.slots * a.kp * atom_bytes);
-  a.b_stage_bytes = (uint32_t)((cta2 ? a.n_atoms / 2 : a.n_atoms) * a.kp * 128);
+  a.b_stage_bytes = (uint32_t)(a.n_atoms * a.kp * 128);
   const size_t SMEM_BUDGET = 200 * 1024;
   int stages = (int)(SMEM_BUDGET / (a.a_stage_bytes + a.b_stage_bytes));
   if (stages > WG_MAX_STAGES) stages = WG_MAX_STAGES;
   a.stages = stages;
   const size_t smem = (size_t)stages * (a.a_stage_bytes + a.b_stage_bytes) + 1024;
   // split-K: enough units to fill the machine ~3 times unless the tiles alone already do
-  const int tiles = (cta2 ? (a.m_tiles + 1) / 2 : (a.m_tiles + group - 1) / group) * a.n_tiles;   // scheduling units before the K split
-  const int workers = cta2 ? g_num_sms / 2 : g_num_sms;
+  const int tiles = ((a.m_tiles + group - 1) / group) * a.n_tiles;   // scheduling units before the K split
   int splits = 1;
-  if (tiles < workers * 3 / 2) splits = (workers * 3 + tiles - 1) / tiles;
+  if (tiles < g_num_sms * 3 / 2) splits = (g_num_sms * 3 + tiles - 1) / tiles;
   int max_splits = a.kstages / 8;
   if (max_splits < 1) max_splits = 1;
   if (splits > max_splits) splits = max_splits;
-  if (env().wgrad_splits) { int v = env().wgrad_splits; if (v >= 1 && v <= a.kstages) splits = v; }
   a.splits = splits;
   fastdiv_init((uint32_t)W, &a.fd_w_mul, &a.fd_w_shr);
   fastdiv_init((uint32_t)H, &a.fd_h_mul, &a.fd_h_shr);
   fastdiv_init((uint32_t)a.cchunks, &a.fd_cch_mul, &a.fd_cch_shr);
   fastdiv_init((uint32_t)ksize, &a.fd_k_mul, &a.fd_k_shr);
   fastdiv_init((uint32_t)a.n_tiles, &a.fd_nt_mul, &a.fd_nt_shr);
-  fastdiv_init((uint32_t)(cta2 ? (a.m_tiles + 1) / 2 : (a.m_tiles + group - 1) / group), &a.fd_mt_mul, &a.fd_mt_shr);
+  fastdiv_init((uint32_t)((a.m_tiles + group - 1) / group), &a.fd_mt_mul, &a.fd_mt_shr);
 
   CUtensorMap tmX, tmG;
   {
@@ -418,14 +352,14 @@ extern "C" int y2_conv_wgrad_bf16(const void* x, const void* dh, int ld_dh, floa
   cudaStream_t st = (cudaStream_t)stream;
   if (atom_bytes == 128) {
     switch (block_n) {
-      case 64: return launch_wgrad<64, 128>(tmX, tmG, a, smem, st, cta2, group);
-      case 128: return launch_wgrad<128, 128>(tmX, tmG, a, smem, st, cta2, group);
-      default: return launch_wgrad<256, 128>(tmX, tmG, a, smem, st, cta2, group);
+      case 64: return launch_wgrad<64, 128>(tmX, tmG, a, smem, st, group);
+      case 128: return launch_wgrad<128, 128>(tmX, tmG, a, smem, st, group);
+      default: return launch_wgrad<256, 128>(tmX, tmG, a, smem, st, group);
     }
   }
   switch (block_n) {
-    case 64: return launch_wgrad<64, 64>(tmX, tmG, a, smem, st, cta2, group);
-    case 128: return launch_wgrad<128, 64>(tmX, tmG, a, smem, st, cta2, group);
-    default: return launch_wgrad<256, 64>(tmX, tmG, a, smem, st, cta2, group);
+    case 64: return launch_wgrad<64, 64>(tmX, tmG, a, smem, st, group);
+    case 128: return launch_wgrad<128, 64>(tmX, tmG, a, smem, st, group);
+    default: return launch_wgrad<256, 64>(tmX, tmG, a, smem, st, group);
   }
 }

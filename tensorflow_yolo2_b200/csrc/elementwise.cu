@@ -877,13 +877,13 @@ static int bn_stats_impl(const float* x, int M, int C, int ld, float* mean, floa
     // tile assignment balances any number of splits.  Layer 1 at batch 64 (1.4 GB): 382 -> 237 us = 6.0 TB/s.
     {
       const int tx = cg <= 8 ? 8 : (cg <= 16 ? 16 : 32);
-      const int wave = g_sms_elementwise() * ((env().bn_stats_variant & 2) ? 4 : 5) / ((cg + tx - 1) / tx);
-      if (!env().bn_stats_unr4 && splits > wave) splits = wave > 1 ? wave : 1;
+      const int wave = g_sms_elementwise() * 5 / ((cg + tx - 1) / tx);
+      if (splits > wave) splits = wave > 1 ? wave : 1;
     }
     // large maps: eight rows (128 B per thread) in flight -- with four the kernel sat at 3.9 TB/s (ncu r2n: 47 % of DRAM peak, the
     // affine pass with 128 B per thread in flight reaches 5.7); the deep 13x13 layers keep four (measured: no gain there)
-    const bool deep = M >= 32768 && !env().bn_stats_unr4;
-    const int cs = ((size_t)M * ld * 4 > (96u << 20)) && !(env().bn_stats_variant & 1) ? 1 : 0;
+    const bool deep = M >= 32768;
+    const int cs = (size_t)M * ld * 4 > (96u << 20) ? 1 : 0;
 #define Y2_LAUNCH_STATS(TX_)                                                                                                  \
   do {                                                                                                                        \
     if (deep) bn_stats_partial_v4_kernel<TX_, 8><<<dim3((cg + TX_ - 1) / TX_, splits), 256, 0, st>>>(x, M, C, ld, rows, (double*)workspace, cs); \

@@ -99,14 +99,6 @@ __device__ __forceinline__ void tma_load_im2col_4d(uint32_t dst, const CUtensorM
       : "memory");
 }
 
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(tm)), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -131,17 +123,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
 }
 __device__ __forceinline__ void umma_commit_a(uint32_t addr) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(addr) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc_a(uint32_t addr, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(addr),
-               "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
-               : "memory");
 }
 // ---- CTA pairs (tcgen05 cta_group::2): one MMA spans two SMs, each CTA feeds its own 128 rows of A and HALF of B ----
 // shared::cluster addresses carry the CTA rank in bit 24; clearing it addresses the same offset in the pair's leader
