@@ -240,3 +240,25 @@ def test_max_pool_routes_ties_to_first_maximum():
                 want[0, 2 * i + k // 2, 2 * j + k % 2, c] = dy[0, i, j, c]
     np.testing.assert_array_equal(x.grad.numpy(), want.numpy())
     assert want[0, 0, 0, 0] == dy[0, 0, 0, 0] and want[0, 0, 3, 0] == dy[0, 0, 1, 0] and want[0, 1, 4, 0] == dy[0, 0, 2, 0]
+
+
+def test_split_hi_lo_representation_bound():
+    """The bound the full-size inference test allows a bf16x3 output (tests/helpers.py SPLIT_REPR): hi + lo of split_hi_lo(v)
+    is within 2^-16 |v| of v, over every binade of normal bf16 lo parts and at bf16 rounding ties of hi and of lo.  It is
+    within a factor 2 of tight: lo rounds |v - hi| < 2^-8 |v| to 8 bits, so the error reaches 2^-17 |v| when lo is a tie."""
+    from tests.helpers import SPLIT_REPR, split_hi_lo
+    rs = np.random.RandomState(5)
+    mant = rs.uniform(1.0, 2.0, 200000)
+    expo = rs.randint(-100, 120, mant.size)
+    v = (mant * np.exp2(expo) * rs.choice([-1.0, 1.0], mant.size)).astype(np.float32)
+    bits = rs.randint(0, 1 << 23, 4096).astype(np.uint32) | np.uint32(127 << 23)
+    ties = ((bits & ~np.uint32(0xFFFF)) | np.uint32(0x8000)).view(np.float32)       # exactly halfway between two bf16
+    worst = ((bits & ~np.uint32(0xFFFF)) | np.uint32(0x4040)).view(np.float32)      # v - hi = 0x4040 units: lo is a tie
+    v = torch.from_numpy(np.concatenate([v, ties, -ties, worst, np.float32([0.0, 1.0, -2.5, 1e38, 2.0 ** -100])]))
+    hi, lo = split_hi_lo(v)
+    assert hi.dtype == lo.dtype == torch.bfloat16
+    assert torch.equal(hi, v.to(torch.bfloat16))
+    err = (v.double() - hi.double() - lo.double()).abs()
+    ratio = err / (SPLIT_REPR * v.double().abs()).clamp_min(1e-300)
+    assert torch.all(err <= SPLIT_REPR * v.double().abs()), float(ratio.max())
+    assert float(ratio.max()) > 0.45

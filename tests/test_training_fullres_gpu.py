@@ -16,25 +16,19 @@ plus a rel-L2 bound per tensor.
 Half of each batch is the two golden photos letterboxed with constant gray bars, the rest random images with a constant
 rectangle: constant regions give bit-identical pre-BN values, i.e. exact ties in the 2x2 max-pool windows, whose gradient
 must go to the first maximum of the window."""
-import os
-
 import numpy as np
 import pytest
 import torch
 
 from oracle import yolo2_oracle as O
-from tests.helpers import make_store
+from tests.helpers import REL_L2_BF16, REL_L2_ELEM, TAU, _check, _images, _rel_l2, _ulp, make_store
 
 pytestmark = pytest.mark.gpu
 
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
-TAU = 1e-5
 # conv_wgrad_tc_kernel: one float32 accumulator in tensor memory takes a whole K range -- on the 13x13 and 19x19 layers all
 # N*H*W pixels (64 * 169 = 10816: 676 MMAs of K = 16), each step rounding relative to a partial sum bounded by absref, so
 # the worst case is 676 * 2^-24 = 4e-5 of absref (twice that if the accumulation truncates): 1e-4.
 TAU_WGRAD = 1e-4
-REL_L2_BF16 = 2.0 ** -8          # twice the worst relative rounding error of a bf16 output
-REL_L2_ELEM = 0.25               # float32 outputs: RMS error <= a quarter of the RMS element bound
 CONFIGS = {416: dict(IS=416, N=64, loss='v1', OF=45), 608: dict(IS=608, N=32, loss='region', OF=125)}
 NUM_LAYERS = 22
 STAGES = ('conv', 'stats', 'act', 'bnbwd', 'wgrad', 'dgrad')
@@ -62,34 +56,6 @@ _COMMON = {1: [WGRAD_C3, BN_BWD_POOL_ROWS], 2: [HALO_PAIR, WGRAD_TC, BN_BWD_POOL
            14: [STREAMK], 16: [STREAMK], 18: [STREAMK], 19: [STREAMK], 20: [STREAMK], 21: [STREAMK], 22: [IM2COL_PAIR]}
 EXPECTED_BWD = {416: dict(_COMMON), 608: {**_COMMON, 6: [HALO_PAIR], 7: [IM2COL_PAIR], 8: [HALO_PAIR, BN_BWD_POOL_ROWS]}}
 EXPECTED_FWD = {416: [BN_STATS_8ROW], 608: [BN_STATS_8ROW]}
-
-
-# ---- inputs ------------------------------------------------------------------------------------------------------------
-def _images(IS, N, seed):
-    """uint8 BGR [N,IS,IS,3]: the first half letterboxed golden photos (constant gray bars), the rest random noise with a
-    constant-colour rectangle of at least 160 x 160."""
-    import cv2
-    rs = np.random.RandomState(seed)
-    photos = [cv2.imread(os.path.join(GOLDEN, f)) for f in ('testImg1.jpg', 'testImg2.jpg')]
-    out = np.empty((N, IS, IS, 3), dtype=np.uint8)
-    for i in range(N):
-        if i < N // 2:
-            im = photos[i % 2]
-            h, w = im.shape[:2]
-            s = IS / max(h, w) * rs.uniform(0.7, 1.0)
-            nh, nw = int(h * s), int(w * s)
-            img = np.full((IS, IS, 3), (114, 128)[rs.randint(2)], dtype=np.uint8)
-            y0, x0 = rs.randint(0, IS - nh + 1), rs.randint(0, IS - nw + 1)
-            img[y0:y0 + nh, x0:x0 + nw] = cv2.resize(im, (nw, nh))
-            if rs.rand() < 0.5:
-                img = img[:, ::-1]
-        else:
-            img = rs.randint(0, 256, (IS, IS, 3)).astype(np.uint8)
-            hh, ww = rs.randint(160, IS // 2 + 1, 2)
-            y0, x0 = rs.randint(0, IS - hh + 1), rs.randint(0, IS - ww + 1)
-            img[y0:y0 + hh, x0:x0 + ww] = rs.randint(0, 256, 3)
-        out[i] = img
-    return out
 
 
 def _labels_v1(rs, N, S, IS, C=20):
@@ -193,39 +159,7 @@ def rec(request):
     torch.cuda.empty_cache()
 
 
-# ---- float64 references and the element check ----------------------------------------------------------------------------
-def _ulp(x, bits):
-    """Spacing of a float format with `bits` significant bits at |x| (0 at x == 0)."""
-    _, e = torch.frexp(x)
-    return torch.where(x == 0, torch.zeros_like(x), torch.ldexp(torch.ones_like(x), e - bits))
-
-
-def _rel_l2(got, ref):
-    return float(torch.linalg.vector_norm(got.double() - ref) / torch.linalg.vector_norm(ref).clamp_min(1e-300))
-
-
-def _check(tag, got, ref, absref, bf16_out, tau=TAU):
-    """Every element within ulp_out(ref)/2 + tau * absref; rel-L2 within 2^-8 for bf16 outputs, and for float32 outputs
-    within a quarter of the element bound's own rel-L2 (float32 results carry cancellation: |ref| << absref)."""
-    got, ref = got.double(), ref.double()
-    bound = tau * absref.double()
-    if bf16_out:
-        bound = bound + 0.5 * _ulp(ref, 8)
-    err = (got - ref).abs()
-    bad = err > bound
-    worst = float((err / bound.clamp_min(1e-300)).max())
-    rl = _rel_l2(got, ref)
-    print('%-18s max err / bound %.3f   rel-L2 %.3g' % (tag, worst, rl))
-    nbad = int(bad.sum())
-    if nbad:
-        i = int(torch.argmax((err - bound).flatten()))
-        raise AssertionError('%s: %d of %d elements out of bound; worst at flat index %d (of shape %s): got %.9g ref %.9g '
-                             'absref %.4g' % (tag, nbad, got.numel(), i, tuple(got.shape), float(got.flatten()[i]),
-                                              float(ref.flatten()[i]), float(absref.flatten()[i])))
-    limit = REL_L2_BF16 if bf16_out else REL_L2_ELEM * _rel_l2(ref + bound, ref)
-    assert rl <= limit, '%s: rel-L2 %.3g > %.3g' % (tag, rl, limit)
-
-
+# ---- float64 references -------------------------------------------------------------------------------------------------
 def _nchw(t):
     return t.permute(0, 3, 1, 2).contiguous()
 
