@@ -103,13 +103,7 @@ typedef struct y2_conv_params {
   float alpha;
   int ldy;      /* output row stride in elements; 0 -> Cout */
   int lo_off;   /* OUT_SPLIT: column of the lo half (0 -> Cout); must be 0 otherwise */
-  /* OUT_F32 only, optional: batch-norm statistics of the rows this call stores, without a second pass over them.  When
-   * y2_conv_stats_slab_rows(p) returns R > 0 (the layer runs on the stream-K kernel), a non-NULL stats_slabs receives
-   * [ceil(M / R)][3][Cout] float32 = per R-row slab and channel (k, sum(v - k), sum((v - k)^2)) of the stored values v
-   * (k = the slab's first row); y2_bn_stats_from_slabs folds them.  Must be NULL when the query returns 0. */
-  float* stats_slabs;
 } y2_conv_params;
-int y2_conv_stats_slab_rows(const y2_conv_params* p);
 int y2_conv_cin_padded(int Cin);
 size_t y2_conv_packed_weight_elems(int ksize, int Cin, int Cout);
 int y2_pack_weights_bf16(const float* w_hwio, void* w_packed, int ksize, int Cin, int Cout, y2_stream_t stream);
@@ -153,10 +147,6 @@ int y2_conv1_u8_pool_fwd_split(const uint8_t* img, const void* w_packed, const f
 size_t y2_bn_stats_workspace_bytes(int M, int C);
 int y2_bn_stats(const float* x, int M, int C, int ld, float* mean, float* var,
                 void* workspace, size_t workspace_bytes, y2_stream_t stream);
-/* Mean / biased variance (and, with gamma / beta / scale / shift non-NULL, the folded affine of y2_bn_stats_fold) from the
- * slab partials a y2_conv_fwd_bf16 call wrote through y2_conv_params.stats_slabs: Chan's merge in float64, fixed order. */
-int y2_bn_stats_from_slabs(const float* slabs, int M, int C, int slab_rows, float* mean, float* var, const float* gamma,
-                           const float* beta, float eps, float* scale, float* shift, y2_stream_t stream);
 /* y2_bn_stats plus, in the same finalising kernel, the folded affine of the centred form
  * y = (x - mean) * scale + shift: scale = gamma * rsqrt(var + eps), shift = beta (what y2_bn_fold
  * gives for mean = 0, bias = NULL) -- the training=True branch of darknet.py:42-44 in two launches. */

@@ -15,7 +15,7 @@ class ConvParams(C.Structure):
     _fields_ = [('x', C.c_void_p), ('w_packed', C.c_void_p), ('scale', C.c_void_p), ('shift', C.c_void_p),
                 ('y', C.c_void_p), ('N', C.c_int), ('H', C.c_int), ('W', C.c_int), ('Cin', C.c_int),
                 ('Cout', C.c_int), ('ksize', C.c_int), ('flags', C.c_int), ('alpha', C.c_float),
-                ('ldy', C.c_int), ('lo_off', C.c_int), ('stats_slabs', C.c_void_p)]
+                ('ldy', C.c_int), ('lo_off', C.c_int)]
 
 
 class Y2Error(RuntimeError):
@@ -38,8 +38,6 @@ _SIGNATURES = {
     'y2_conv_packed_weight_split_elems': (_sz, [_i, _i, _i]),
     'y2_pack_weights_bf16_split': (_i, [_vp, _vp, _i, _i, _i, _vp]),
     'y2_conv_fwd_bf16': (_i, [C.POINTER(ConvParams), _vp]),
-    'y2_conv_stats_slab_rows': (_i, [C.POINTER(ConvParams)]),
-    'y2_bn_stats_from_slabs': (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _f, _vp, _vp, _vp]),
     'y2_conv_workspace_bytes': (_sz, []),
     'y2_conv_set_workspace': (_i, [_vp, _sz]),
     'y2_conv1_u8_packed_weight_elems': (_sz, []),

@@ -49,7 +49,7 @@ const EnvSwitches& env() {
 }  // namespace y2
 
 extern "C" {
-int y2_version(void) { return 100; }
+int y2_version(void) { return 101; }
 const char* y2_last_error(void) { return y2::g_err; }
 unsigned long long y2_launch_count(void) { return y2::g_launches.load(std::memory_order_relaxed); }
 int y2_reload_env(void) {

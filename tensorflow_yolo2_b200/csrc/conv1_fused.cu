@@ -479,18 +479,12 @@ static int conv1_u8_pool_launch(const uint8_t* img, const void* w_packed, const 
   CUtensorMap tmImg, tmY;
   {
     // pooled output [N, H/2, W/2, 32 | 64] bf16: boxes of one tile (8 x 16 pooled pixels, the whole row), swizzled rows
-    const cuuint64_t cw = split ? 2 * C1_COUT : C1_COUT, Ho = H / 2, Wo = W / 2;
-    cuuint64_t dims[4] = {cw, Wo, Ho, (cuuint64_t)N};
-    cuuint64_t strides[3] = {cw * 2, Wo * cw * 2, Ho * Wo * cw * 2};
-    cuuint32_t box[4] = {(cuuint32_t)cw, (cuuint32_t)C1_TW, (cuuint32_t)C1_TH, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encodeTiled(&tmY, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, y, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                               split ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("y2_conv1_u8_pool_fwd: output tensor map encode failed (CUresult %d)", (int)r);
-      return Y2_ERR_DRIVER;
-    }
+    const int cw = split ? 2 * C1_COUT : C1_COUT;
+    const cuuint32_t box[4] = {(cuuint32_t)cw, (cuuint32_t)C1_TW, (cuuint32_t)C1_TH, 1};
+    rc = tmap_nhwc_box(&tmY, y, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, N, H / 2, W / 2, cw, cw, box,
+                       split ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                       "y2_conv1_u8_pool_fwd", "output");
+    if (rc != Y2_OK) return rc;
   }
   {
     cuuint64_t dims[3] = {(cuuint64_t)W * 3, (cuuint64_t)H, (cuuint64_t)N};

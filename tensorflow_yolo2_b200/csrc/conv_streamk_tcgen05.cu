@@ -55,8 +55,6 @@ struct SkArgs {
   int H, W, ldy, pad;
   int cin_p, cchunks, ksteps;       // K steps per tile = taps * cchunks   (cin_p: K extent per tap of the B operand)
   int split_out, lo_off;            // bf16x3 output: hi at column c, lo at column lo_off + c
-  float* stats;                     // out_f32 only: per 32-row slab and column (k, sum(x - k), sum((x - k)^2)) of the stored rows,
-  int cout;                         //   laid out [slab][3][cout] -- batch-norm statistics without a second pass over the rows
   uint32_t fd_cc_mul, fd_cc_shr;    // division by cchunks
   int n_tiles, tiles;
   long long units;                  // tiles * ksteps
@@ -93,30 +91,6 @@ __device__ __forceinline__ void sk_store_rows_bf16(uint32_t stg, int lane, const
     if (grow0 + r < M) *reinterpret_cast<uint4*>(dst + (size_t)(grow0 + r) * ldy + j * 8) = o;
   }
   __syncwarp();
-}
-
-// Batch-norm statistics of one stored 32-row x 32-column chunk, from its swizzled float32 staging tile: lane = column, shifted
-// by the slab's first row (activations reach 1e9 with |mean| >> std under the reference's initialiser: plain sums would
-// cancel).  (k, sum d, sum d^2) per (slab, column); y2_bn_stats_from_slabs merges the slabs in float64.
-__device__ __forceinline__ void sk_slab_stats(const SkArgs& a, uint32_t stg, int lane, int col, long long grow0) {
-  if (grow0 >= a.M) return;
-  const int nvalid = (int)min((long long)32, a.M - grow0);
-  auto at = [&](int r) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(stg + r * 128 + ((((lane >> 2) ^ (r & 7))) << 4) + ((lane & 3) << 2)));
-    return v;
-  };
-  const float k = at(0);
-  float s1 = 0.0f, s2 = 0.0f;
-#pragma unroll 8
-  for (int r = 0; r < 32; ++r) {
-    const float d = at(r) - k;
-    if (r < nvalid) { s1 += d; s2 = fmaf(d, d, s2); }
-  }
-  float* o = a.stats + (size_t)(grow0 >> 5) * 3 * a.cout + col + lane;          // lane = column within the chunk
-  o[0] = k;
-  o[a.cout] = s1;
-  o[2 * a.cout] = s2;
 }
 
 // affine + leaky done: convert (and, bf16x3, split into hi / lo) and store one 32 x 32 chunk
@@ -393,7 +367,6 @@ conv_streamk2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                          : "r"(stg + r * 128 + ((j ^ (r & 7)) << 4)));
             if (grow0 + r < a.M) *reinterpret_cast<float4*>(dst + (size_t)(grow0 + r) * a.ldy + j * 4) = o;
           }
-          if (a.stats) sk_slab_stats(a, stg, lane, col0 + c, grow0);
         } else {
           sk_store_chunk_bf16(a, stg, lane, f, col0 + c, grow0);
         }
@@ -429,47 +402,34 @@ constexpr size_t SK_FLAG_BYTES = 4096;
 static size_t sk_workspace_bytes(int sms) { return SK_FLAG_BYTES + (size_t)sms * 256 * 256 * sizeof(float); }
 
 // returns Y2_OK and sets *handled = 1 when the layer was issued on this path
-// dry != 0: only decide (*handled = 1 when the layer would take this path, whose float32 epilogue can emit the batch-norm
-// slab statistics) -- nothing is enqueued
-int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int dry) {
+int conv_streamk_try(const ConvCall& c, cudaStream_t st, int* handled) {
   *handled = 0;
   if (env().conv_no_streamk || g_sk_ws == nullptr || g_num_sms < 2) return Y2_OK;
-  if ((p->flags & Y2_CONV_POOL2) != 0) return Y2_OK;
-  if (!(p->ksize == 1 || p->ksize == 3) || p->Cin % 64 != 0 || p->Cout % 256 != 0) return Y2_OK;
-  if (p->H >= 64 && p->W >= 64) return Y2_OK;                   // large maps: the halo-patch mode of conv_tc_kernel wins
-  const bool out_f32 = (p->flags & Y2_CONV_OUT_F32) != 0;
-  const int ldy = p->ldy > 0 ? p->ldy : (((p->flags & Y2_CONV_OUT_SPLIT) != 0 && !out_f32) ? 2 * p->Cout : p->Cout);
-  if (ldy % (out_f32 ? 4 : 8) != 0 || (reinterpret_cast<uintptr_t>(p->y) & 15) != 0) return Y2_OK;
-  if ((p->shift && (reinterpret_cast<uintptr_t>(p->shift) & 15) != 0) || (p->scale && (reinterpret_cast<uintptr_t>(p->scale) & 15) != 0))
+  if (c.pool || c.Cin % 64 != 0 || c.Cout % 256 != 0) return Y2_OK;
+  if (c.H >= 64 && c.W >= 64) return Y2_OK;                     // large maps: the halo-patch mode of conv_tc_kernel wins
+  if (c.ldy % (c.out_f32 ? 4 : 8) != 0 || (reinterpret_cast<uintptr_t>(c.y) & 15) != 0) return Y2_OK;
+  if ((c.shift && (reinterpret_cast<uintptr_t>(c.shift) & 15) != 0) || (c.scale && (reinterpret_cast<uintptr_t>(c.scale) & 15) != 0))
     return Y2_OK;
-  const bool split_in = (p->flags & Y2_CONV_IN_SPLIT) != 0;
-  const bool split_out = (p->flags & Y2_CONV_OUT_SPLIT) != 0 && !out_f32;
-  const int a_cin = split_in ? 2 * p->Cin : p->Cin, b_cin = split_in ? 3 * p->Cin : p->Cin;
-  const bool x3 = split_in;                                     // bf16x3: shared-operand stages
-  const int taps = p->ksize * p->ksize, cchunks = (x3 ? p->Cin : b_cin) / 64, ksteps = taps * cchunks;
-  const int lo_off = split_out ? (p->lo_off > 0 ? p->lo_off : p->Cout) : 0;
-  if (split_out && ((lo_off & 7) != 0 || ldy < lo_off + p->Cout)) return Y2_OK;
+  const bool x3 = c.split_in;                                   // bf16x3: shared-operand stages
+  const int cchunks = (x3 ? c.Cin : c.b_cin) / 64, ksteps = c.taps * cchunks;
+  if (c.split_out && (c.lo_off & 7) != 0) return Y2_OK;
   const int min_ksteps = x3 ? 6 : 18;                           // short K: the epilogue starts to show (bf16x3 steps are 3x heavier)
   if (ksteps < min_ksteps || ksteps > SK_MAX_UNITS) return Y2_OK;
-  int rc = load_driver_entry_points();
-  if (rc != Y2_OK) return rc;
   SkArgs a;
   memset(&a, 0, sizeof(a));
-  a.scale = p->scale;
-  a.shift = p->shift;
-  a.y = p->y;
-  a.alpha = p->alpha;
-  a.leaky = (p->flags & Y2_CONV_LEAKY) != 0;
-  a.out_f32 = out_f32;
-  a.M = (long long)p->N * p->H * p->W;
-  a.H = p->H; a.W = p->W; a.ldy = ldy; a.pad = p->ksize / 2;
-  a.cin_p = b_cin; a.cchunks = cchunks; a.ksteps = ksteps;
-  a.split_out = split_out ? 1 : 0;
-  a.lo_off = lo_off;
-  a.stats = out_f32 ? p->stats_slabs : nullptr;
-  a.cout = p->Cout;
+  a.scale = c.scale;
+  a.shift = c.shift;
+  a.y = c.y;
+  a.alpha = c.alpha;
+  a.leaky = c.leaky;
+  a.out_f32 = c.out_f32;
+  a.M = c.M;
+  a.H = c.H; a.W = c.W; a.ldy = c.ldy; a.pad = c.pad;
+  a.cin_p = c.b_cin; a.cchunks = cchunks; a.ksteps = ksteps;
+  a.split_out = c.split_out ? 1 : 0;
+  a.lo_off = c.lo_off;
   fastdiv_init((uint32_t)cchunks, &a.fd_cc_mul, &a.fd_cc_shr);
-  a.n_tiles = p->Cout / 256;
+  a.n_tiles = c.Cout / 256;
   const long long m_tiles = (a.M + 255) / 256;
   a.tiles = (int)(m_tiles * a.n_tiles);
   a.units = (long long)a.tiles * ksteps;
@@ -480,63 +440,22 @@ int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int
   a.ws_flags = reinterpret_cast<int*>(g_sk_ws);
   a.ws_partial = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(g_sk_ws) + SK_FLAG_BYTES);
   fastdiv_init((uint32_t)a.n_tiles, &a.fd_nt_mul, &a.fd_nt_shr);
-  fastdiv_init((uint32_t)p->W, &a.fd_w_mul, &a.fd_w_shr);
-  fastdiv_init((uint32_t)p->H, &a.fd_h_mul, &a.fd_h_shr);
+  fastdiv_init((uint32_t)c.W, &a.fd_w_mul, &a.fd_w_shr);
+  fastdiv_init((uint32_t)c.H, &a.fd_h_mul, &a.fd_h_shr);
   fastdiv_init((uint32_t)ksteps, &a.fd_ks_mul, &a.fd_ks_shr);
 
-  if (dry) {
-    *handled = 1;
-    return Y2_OK;
-  }
+  static const char* const who = "y2_conv_fwd_bf16 (stream-K)";
   CUtensorMap tmA, tmB;
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)a_cin, (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
-    cuuint64_t strides[3] = {(cuuint64_t)a_cin * 2, (cuuint64_t)p->W * a_cin * 2, (cuuint64_t)p->H * p->W * a_cin * 2};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    int lower[2] = {-a.pad, -a.pad};
-    int upper[2] = {a.pad - (p->ksize - 1), a.pad - (p->ksize - 1)};
-    CUresult r = g_encodeIm2col(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p->x), dims, strides, lower, upper,
-                                64, 128, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r == CUDA_SUCCESS && g_driver_version <= 13010 && (size_t)a.M * a_cin * 2 < 131072)
-      reinterpret_cast<uint64_t*>(&tmA)[1] &= ~(1ull << 21);   // same small-tensor fix-up as conv_tcgen05.cu
-    if (r != CUDA_SUCCESS) {
-      set_error("conv_streamk: tensor map A encode failed (CUresult %d)", (int)r);
-      return Y2_ERR_DRIVER;
-    }
-    const int Kp = taps * b_cin;
-    cuuint64_t bdims[2] = {(cuuint64_t)Kp, (cuuint64_t)p->Cout};
-    cuuint64_t bstrides[1] = {(cuuint64_t)Kp * 2};
-    cuuint32_t bbox[2] = {64, 128u};                           // each CTA of the pair loads its half of the filters
-    cuuint32_t bestr[2] = {1, 1};
-    r = g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p->w_packed), bdims, bstrides, bbox, bestr,
-                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("conv_streamk: tensor map B encode failed (CUresult %d)", (int)r);
-      return Y2_ERR_DRIVER;
-    }
-  }
+  int rc = tmap_im2col_nhwc(&tmA, c.x, c.N, c.H, c.W, c.a_cin, c.ksize, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B, who, "A");
+  if (rc == Y2_OK)      // each CTA of the pair loads its half of the filters
+    rc = tmap_kmajor(&tmB, c.w_packed, c.taps * c.b_cin, c.Cout, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, who, "B");
+  if (rc != Y2_OK) return rc;
   // (the flag area was zero when the workspace was registered -- the caller's contract -- and every launch leaves it zero)
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)(2 * npairs));
-  cfg.blockDim = dim3(SK_THREADS);
-  cfg.dynamicSmemBytes = SK2_SMEM;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  cfg.attrs = attr;
-  cfg.numAttrs = fill_launch_attrs(attr, 2u);                   // (matches the kernel's __cluster_dims__)
-  if (x3) {
-    Y2_CUDA(cudaFuncSetAttribute(conv_streamk2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK2_SMEM));
-    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk2_kernel<true>, tmA, tmB, a));
-  } else {
-    Y2_CUDA(cudaFuncSetAttribute(conv_streamk2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK2_SMEM));
-    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_streamk2_kernel<false>, tmA, tmB, a));
-  }
-  Y2_LAUNCHED();
-  *handled = 1;
-  return Y2_OK;
+  rc = launch_cluster(x3 ? conv_streamk2_kernel<true> : conv_streamk2_kernel<false>, 2 * npairs, SK_THREADS, SK2_SMEM, 2u, st,
+                      tmA, tmB, a);
+  *handled = rc == Y2_OK;
+  return rc;
 }
 
 }  // namespace y2

@@ -1199,6 +1199,51 @@ int load_driver_entry_points() {
   return Y2_OK;
 }
 
+static int tmap_result(CUresult r, const char* who, const char* name) {
+  if (r == CUDA_SUCCESS) return Y2_OK;
+  set_error("%s: tensor map %s encode failed (CUresult %d)", who, name, (int)r);
+  return Y2_ERR_DRIVER;
+}
+
+int tmap_im2col_nhwc(CUtensorMap* tm, const void* x, int N, int H, int W, int C, int ksize, int chans, int pixels,
+                     CUtensorMapSwizzle sw, const char* who, const char* name) {
+  const int pad = ksize / 2;
+  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
+  cuuint32_t estr[4] = {1, 1, 1, 1};
+  int lower[2] = {-pad, -pad};
+  int upper[2] = {pad - (ksize - 1), pad - (ksize - 1)};
+  CUresult r = g_encodeIm2col(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dims, strides, lower, upper,
+                              (cuuint32_t)chans, (cuuint32_t)pixels, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
+                              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  // same small-tensor fix-up CUTLASS applies (cute/atom/copy_traits_sm90_im2col.hpp) for drivers <= 13.1
+  if (r == CUDA_SUCCESS && g_driver_version <= 13010 && (size_t)N * H * W * C * 2 < 131072)
+    reinterpret_cast<uint64_t*>(tm)[1] &= ~(1ull << 21);
+  return tmap_result(r, who, name);
+}
+
+int tmap_nhwc_box(CUtensorMap* tm, const void* base, CUtensorMapDataType dt, int N, int H, int W, int C, int ld,
+                  const cuuint32_t box[4], CUtensorMapSwizzle sw, CUtensorMapL2promotion l2, const char* who, const char* name) {
+  const cuuint64_t es = dt == CU_TENSOR_MAP_DATA_TYPE_FLOAT32 ? 4 : 2;          // float32 or bf16
+  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+  cuuint64_t strides[3] = {(cuuint64_t)ld * es, (cuuint64_t)W * ld * es, (cuuint64_t)H * W * ld * es};
+  cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult r = g_encodeTiled(tm, dt, 4, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw, l2,
+                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return tmap_result(r, who, name);
+}
+
+int tmap_kmajor(CUtensorMap* tm, const void* base, int K, long long rows, int box_k, int box_rows, CUtensorMapSwizzle sw,
+                CUtensorMapL2promotion l2, const char* who, const char* name) {
+  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)K * 2};
+  cuuint32_t box[2] = {(cuuint32_t)box_k, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = g_encodeTiled(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+                             CU_TENSOR_MAP_INTERLEAVE_NONE, sw, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return tmap_result(r, who, name);
+}
+
 
 // choose the pixel box (NB x TH x TW = 128, powers of two) with the least padding waste
 static void choose_box(int N, int H, int W, bool pool, int* tw, int* th, int* nb) {
@@ -1218,25 +1263,12 @@ static void choose_box(int N, int H, int W, bool pool, int* tw, int* th, int* nb
 
 template <int BLOCK_N, int A_MODE, int KIND, bool CTA2 = false, bool TMAST = false>
 static int launch_conv3(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmY, const ConvArgs& a, size_t smem, cudaStream_t st) {
-  Y2_CUDA(cudaFuncSetAttribute((conv_tc_kernel<BLOCK_N, A_MODE, KIND, CTA2, TMAST>), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)smem));
   constexpr int CS = CTA2 ? 2 : 1;
   long long units = (long long)((a.m_tiles + CS - 1) / CS) * a.n_tiles;
   long long want = units * CS;
   int grid = (int)(want < g_num_sms ? want : g_num_sms);
   grid -= grid % CS;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  cfg.attrs = attr;
-  cfg.numAttrs = fill_launch_attrs(attr, (unsigned)CS);
-  Y2_CUDA(cudaLaunchKernelEx(&cfg, (conv_tc_kernel<BLOCK_N, A_MODE, KIND, CTA2, TMAST>), tmA, tmB, tmY, a));
-  Y2_LAUNCHED();
-  return Y2_OK;
+  return launch_cluster(conv_tc_kernel<BLOCK_N, A_MODE, KIND, CTA2, TMAST>, grid, TC_THREADS, smem, (unsigned)CS, st, tmA, tmB, tmY, a);
 }
 
 template <int BLOCK_N, int KIND>
@@ -1279,39 +1311,33 @@ static int launch_conv(int block_n, const CUtensorMap& tmA, const CUtensorMap& t
   }
 }
 
-int conv_streamk_try(const y2_conv_params* p, cudaStream_t st, int* handled, int dry);   // conv_streamk_tcgen05.cu
+int conv_streamk_try(const ConvCall& c, cudaStream_t st, int* handled);   // conv_streamk_tcgen05.cu
 
 // The input-stationary kernel (conv_is_kernel): 3x3, Cout == 64, maps >= 64 x 64, filters resident.  *handled = 1 when issued.
-static int conv_is_try(const y2_conv_params* p, cudaStream_t st, int* handled) {
+static int conv_is_try(const ConvCall& c, cudaStream_t st, int* handled) {
   *handled = 0;
-  if (env().conv_no_is || p->ksize != 3 || p->Cout != IS_COUT || p->H < 64 || p->W < 64 || p->Cin % 32 != 0 || g_num_sms < 2) return Y2_OK;
-  const bool split_in = (p->flags & Y2_CONV_IN_SPLIT) != 0;
-  const bool out_f32 = (p->flags & Y2_CONV_OUT_F32) != 0;
-  const bool split_out = (p->flags & Y2_CONV_OUT_SPLIT) != 0 && !out_f32;
-  const bool pool = (p->flags & Y2_CONV_POOL2) != 0;
+  if (env().conv_no_is || c.ksize != 3 || c.Cout != IS_COUT || c.H < 64 || c.W < 64 || c.Cin % 32 != 0 || g_num_sms < 2) return Y2_OK;
   // Short K (layer 2: 32 channels) is epilogue-bound, and this kernel's epilogue is the heavier one (three accumulator
   // blocks + two shuffles per value): measured 149 vs 115 us there, against 88 vs 114 us on layer 4 (128 channels).
-  if ((split_in ? 3 : 1) * p->Cin < 96 && !env().conv_force_is) return Y2_OK;
+  if (c.b_cin < 96 && !env().conv_force_is) return Y2_OK;
   ConvArgs a;
   memset(&a, 0, sizeof(a));
-  a.scale = p->scale; a.shift = p->shift; a.y = p->y;
-  a.N = p->N; a.H = p->H; a.W = p->W; a.Cout = p->Cout;
-  a.M = (long long)p->N * p->H * p->W;
-  a.split_out = split_out ? 1 : 0;
-  a.lo_off = split_out ? (p->lo_off > 0 ? p->lo_off : p->Cout) : 0;
-  a.ldy = p->ldy > 0 ? p->ldy : (split_out ? 2 * p->Cout : p->Cout);
-  if (a.ldy < p->Cout || (split_out && (a.lo_off < p->Cout || a.ldy < a.lo_off + p->Cout))) return Y2_OK;   // (the generic path reports it)
-  a.flags = p->flags; a.alpha = p->alpha; a.ksize = 3; a.pad = 1;
-  a.cin_p = split_in ? 3 * p->Cin : p->Cin;
-  const int a_cin = split_in ? 2 * p->Cin : p->Cin;
-  a.kchunk = (p->Cin % 64 == 0) ? 64 : 32;
+  a.scale = c.scale; a.shift = c.shift; a.y = c.y;
+  a.N = c.N; a.H = c.H; a.W = c.W; a.Cout = c.Cout;
+  a.M = c.M;
+  a.split_out = c.split_out ? 1 : 0;
+  a.lo_off = c.lo_off;
+  a.ldy = c.ldy;
+  a.flags = c.flags; a.alpha = c.alpha; a.ksize = 3; a.pad = 1;
+  a.cin_p = c.b_cin;
+  a.kchunk = (c.Cin % 64 == 0) ? 64 : 32;
   a.row_bytes = a.kchunk * 2;
   a.cchunks = a.cin_p / a.kchunk;
-  a.a_wrap = a_cin / a.kchunk;
+  a.a_wrap = c.a_cin / a.kchunk;
   a.kblocks = 9 * a.cchunks;
   a.tw_log2 = 4; a.th_log2 = 3; a.nb_log2 = 0;
-  a.tiles_w = (p->W + IS_OUT_W - 1) / IS_OUT_W; a.tiles_h = (p->H + IS_TH - 1) / IS_TH; a.tiles_nb = p->N;
-  const long long tiles = (long long)a.tiles_w * a.tiles_h * p->N;
+  a.tiles_w = (c.W + IS_OUT_W - 1) / IS_OUT_W; a.tiles_h = (c.H + IS_TH - 1) / IS_TH; a.tiles_nb = c.N;
+  const long long tiles = (long long)a.tiles_w * a.tiles_h * c.N;
   if (tiles < 2 || tiles >= (1ll << 30) || a.M >= (1ll << 31)) return Y2_OK;
   a.m_tiles = (int)tiles; a.n_tiles = 1;
   a.a_stage_bytes = (uint32_t)(IS_PROWS * IS_TW * a.row_bytes);
@@ -1328,8 +1354,8 @@ static int conv_is_try(const y2_conv_params* p, cudaStream_t st, int* handled) {
   // un-pooled outputs leave through 32 KB of staging + TMA box stores when at least three ring stages remain next to it
   const size_t IS_STG = 4 * 8192;
   a.tma_store = 0;
-  if (!pool && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(p->y) & 15) == 0 &&
-      (!split_out || a.lo_off % 8 == 0) && (SMEM_BUDGET - b_region - IS_STG) / stage_bytes >= 3)
+  if (!c.pool && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(c.y) & 15) == 0 &&
+      (!c.split_out || a.lo_off % 8 == 0) && (SMEM_BUDGET - b_region - IS_STG) / stage_bytes >= 3)
     a.tma_store = 1;
   const size_t stg_bytes = a.tma_store ? IS_STG : 0;
   int stages = (int)((SMEM_BUDGET - b_region - stg_bytes) / stage_bytes);
@@ -1339,157 +1365,76 @@ static int conv_is_try(const y2_conv_params* p, cudaStream_t st, int* handled) {
   fastdiv_init((uint32_t)a.tiles_w, &a.fd_w_mul, &a.fd_w_shr);
   fastdiv_init((uint32_t)a.tiles_h, &a.fd_h_mul, &a.fd_h_shr);
   const size_t smem = b_region + (size_t)stages * stage_bytes + stg_bytes + 1024;
-  int rc = load_driver_entry_points();
-  if (rc != Y2_OK) return rc;
-  CUtensorMap tmA, tmB;
+  static const char* const who = "y2_conv_fwd_bf16 (input-stationary)";
   const CUtensorMapSwizzle sw = swizzle_for(a.row_bytes);
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)a_cin, (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
-    cuuint64_t strides[3] = {(cuuint64_t)a_cin * 2, (cuuint64_t)p->W * a_cin * 2, (cuuint64_t)p->H * p->W * a_cin * 2};
-    cuuint32_t box[4] = {(cuuint32_t)a.kchunk, (cuuint32_t)IS_TW, (cuuint32_t)IS_PROWS, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encodeTiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p->x), dims, strides, box, estr,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("y2_conv_fwd_bf16 (input-stationary): tensor map A encode failed (CUresult %d)", (int)r); return Y2_ERR_DRIVER; }
-    const int Kp = 9 * a.cin_p;
-    cuuint64_t bdims[2] = {(cuuint64_t)Kp, (cuuint64_t)IS_COUT};
-    cuuint64_t bstrides[1] = {(cuuint64_t)Kp * 2};
-    cuuint32_t bbox[2] = {(cuuint32_t)a.kchunk, 32};
-    cuuint32_t bestr[2] = {1, 1};
-    r = g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p->w_packed), bdims, bstrides, bbox, bestr,
-                      CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("y2_conv_fwd_bf16 (input-stationary): tensor map B encode failed (CUresult %d)", (int)r); return Y2_ERR_DRIVER; }
-  }
-  CUtensorMap tmY;
+  CUtensorMap tmA, tmB, tmY;
+  const cuuint32_t box_a[4] = {(cuuint32_t)a.kchunk, (cuuint32_t)IS_TW, (cuuint32_t)IS_PROWS, 1};
+  int rc = tmap_nhwc_box(&tmA, c.x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, c.N, c.H, c.W, c.a_cin, c.a_cin, box_a, sw,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, who, "A");
+  if (rc == Y2_OK)
+    rc = tmap_kmajor(&tmB, c.w_packed, 9 * a.cin_p, IS_COUT, a.kchunk, 32, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, who, "B");
+  if (rc != Y2_OK) return rc;
   memset(&tmY, 0, sizeof(tmY));
   if (a.tma_store) {
-    const cuuint64_t es = out_f32 ? 4 : 2;
-    cuuint64_t dims[4] = {(cuuint64_t)(split_out ? a.lo_off + p->Cout : p->Cout), (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
-    cuuint64_t strides[3] = {(cuuint64_t)a.ldy * es, (cuuint64_t)p->W * a.ldy * es, (cuuint64_t)p->H * p->W * a.ldy * es};
-    cuuint32_t box[4] = {out_f32 ? 16u : 32u, (cuuint32_t)IS_OUT_W, (cuuint32_t)IS_TH, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encodeTiled(&tmY, out_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, p->y, dims, strides,
-                               box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("y2_conv_fwd_bf16 (input-stationary): tensor map Y encode failed (CUresult %d)", (int)r); return Y2_ERR_DRIVER; }
+    const cuuint32_t box_y[4] = {c.out_f32 ? 16u : 32u, (cuuint32_t)IS_OUT_W, (cuuint32_t)IS_TH, 1};
+    rc = tmap_nhwc_box(&tmY, c.y, c.out_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, c.N, c.H, c.W,
+                       c.split_out ? a.lo_off + c.Cout : c.Cout, a.ldy, box_y, CU_TENSOR_MAP_SWIZZLE_64B,
+                       CU_TENSOR_MAP_L2_PROMOTION_NONE, who, "Y");
+    if (rc != Y2_OK) return rc;
   }
   const int groups = (a.m_tiles + 1) / 2;
   const int npairs = groups < g_num_sms / 2 ? groups : g_num_sms / 2;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)(2 * npairs));
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  cfg.attrs = attr;
-  cfg.numAttrs = fill_launch_attrs(attr, 2u);
-  if (a.row_bytes == 64) {
-    Y2_CUDA(cudaFuncSetAttribute(conv_is_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_is_kernel<1>, tmA, tmB, tmY, a));
-  } else {
-    Y2_CUDA(cudaFuncSetAttribute(conv_is_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    Y2_CUDA(cudaLaunchKernelEx(&cfg, conv_is_kernel<2>, tmA, tmB, tmY, a));
-  }
-  Y2_LAUNCHED();
-  *handled = 1;
-  return Y2_OK;
+  rc = launch_cluster(a.row_bytes == 64 ? conv_is_kernel<1> : conv_is_kernel<2>, 2 * npairs, TC_THREADS, smem, 2u, st, tmA, tmB, tmY, a);
+  *handled = rc == Y2_OK;
+  return rc;
 }
 
-}  // namespace y2
-
-using namespace y2;
-
-extern "C" int y2_conv_stats_slab_rows(const y2_conv_params* p) {
-  if (!p || !(p->flags & Y2_CONV_OUT_F32) || load_driver_entry_points() != Y2_OK) return 0;
-  int handled = 0;
-  if (conv_streamk_try(p, nullptr, &handled, 1) != Y2_OK) return 0;
-  return handled ? 32 : 0;
-}
-
-extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
-  Y2_ARG(p != nullptr);
-  Y2_ARG(p->x && p->w_packed && p->y);
-  const bool split_in = (p->flags & Y2_CONV_IN_SPLIT) != 0;
-  const bool split_out = (p->flags & Y2_CONV_OUT_SPLIT) != 0 && (p->flags & Y2_CONV_OUT_F32) == 0;
-  Y2_ARG(split_out || p->lo_off == 0);
-  if (split_in) Y2_ARG(p->Cin % 32 == 0);
-  Y2_ARG(p->N > 0 && p->H > 0 && p->W > 0 && p->Cin > 0 && p->Cout > 0 && (p->ksize == 1 || p->ksize == 3));
-  const bool pool = (p->flags & Y2_CONV_POOL2) != 0;
-  const bool out_f32 = (p->flags & Y2_CONV_OUT_F32) != 0;
-  if (pool) Y2_ARG(p->H % 2 == 0 && p->W % 2 == 0);
-  int rc = load_driver_entry_points();
-  if (rc != Y2_OK) return rc;
-  {
-    // float32 pre-BN rows of a deep 3x3 layer on a small map: 256x256 stream-K tiles (conv_streamk_tcgen05.cu)
-    int handled = 0;
-    rc = conv_streamk_try(p, (cudaStream_t)stream, &handled, 0);
-    if (rc != Y2_OK || handled) return rc;
-  }
-  if (p->stats_slabs) {
-    set_error("y2_conv_fwd_bf16: stats_slabs is only produced by the stream-K path (query y2_conv_stats_slab_rows first)");
-    return Y2_ERR_UNSUPPORTED;
-  }
-  {
-    int handled = 0;
-    rc = conv_is_try(p, (cudaStream_t)stream, &handled);
-    if (rc != Y2_OK || handled) return rc;
-  }
-
+// conv_tc_kernel: every call the other two paths decline
+static int conv_generic(const ConvCall& c, cudaStream_t st) {
   ConvArgs a;
   memset(&a, 0, sizeof(a));
-  a.scale = p->scale;
-  a.shift = p->shift;
-  a.y = p->y;
-  a.N = p->N; a.H = p->H; a.W = p->W; a.Cout = p->Cout;
-  a.M = (long long)p->N * p->H * p->W;
-  a.split_out = split_out ? 1 : 0;
-  a.lo_off = split_out ? (p->lo_off > 0 ? p->lo_off : p->Cout) : 0;
-  a.ldy = p->ldy > 0 ? p->ldy : (split_out ? 2 * p->Cout : p->Cout);
-  Y2_ARG(a.ldy >= p->Cout);
-  if (split_out) Y2_ARG(a.lo_off >= p->Cout && a.ldy >= a.lo_off + p->Cout);
-  a.flags = p->flags;
-  a.alpha = p->alpha;
-  a.ksize = p->ksize;
-  a.pad = p->ksize / 2;
-  // cin_p: K extent per tap of the B operand; a_cin: channels of the A tensor (bf16x3: [w_hi|w_hi|w_lo] against [hi|lo])
-  a.cin_p = split_in ? 3 * p->Cin : y2_conv_cin_padded(p->Cin);
-  const int a_cin = split_in ? 2 * p->Cin : a.cin_p;
-  Y2_ARG(split_in || a.cin_p == p->Cin || p->Cin < 8);
-  const int cout_p = (p->Cout + 15) / 16 * 16;
-  const int taps = p->ksize * p->ksize;
+  a.scale = c.scale;
+  a.shift = c.shift;
+  a.y = c.y;
+  a.N = c.N; a.H = c.H; a.W = c.W; a.Cout = c.Cout;
+  a.M = c.M;
+  a.split_out = c.split_out ? 1 : 0;
+  a.lo_off = c.lo_off;
+  a.ldy = c.ldy;
+  a.flags = c.flags;
+  a.alpha = c.alpha;
+  a.ksize = c.ksize;
+  a.pad = c.pad;
+  a.cin_p = c.b_cin;
+  const int cout_p = (c.Cout + 15) / 16 * 16;
   a.first_layer = a.cin_p == 8;
   if (a.first_layer) {
-    Y2_ARG(p->ksize == 3);
     a.kchunk = 8; a.row_bytes = 16; a.kblocks = 1; a.cchunks = 1; a.ksteps = 5;
     a.layout_type = 0;                    // no swizzle: core matrices of 8 rows x 16 B
     a.kstep_bytes = 2 * 16;               // x rows -> two 16-byte K groups per MMA (scaled by rows in-kernel)
-  } else if (p->Cin % 64 == 0) {
+  } else if (c.Cin % 64 == 0) {
     a.kchunk = 64; a.row_bytes = 128; a.layout_type = 2; a.ksteps = 4; a.kstep_bytes = 32;
-    a.cchunks = a.cin_p / 64; a.kblocks = taps * a.cchunks;
-  } else if (p->Cin % 32 == 0) {
+    a.cchunks = a.cin_p / 64; a.kblocks = c.taps * a.cchunks;
+  } else {                                // Cin % 32 == 0 (checked with the call)
     a.kchunk = 32; a.row_bytes = 64; a.layout_type = 4; a.ksteps = 2; a.kstep_bytes = 32;
-    a.cchunks = a.cin_p / 32; a.kblocks = taps * a.cchunks;
-  } else {
-    set_error("y2_conv_fwd_bf16: Cin=%d unsupported (need 3, or a multiple of 32)", p->Cin);
-    return Y2_ERR_UNSUPPORTED;
+    a.cchunks = a.cin_p / 32; a.kblocks = c.taps * a.cchunks;
   }
-  a.a_wrap = a.first_layer ? 1 : a_cin / a.kchunk;
-  a.a_mode = pool ? 1 : 0;
+  a.a_wrap = a.first_layer ? 1 : c.a_cin / a.kchunk;
+  a.a_mode = c.pool ? 1 : 0;
   if (env().conv_force_tiled) a.a_mode = 1;
   // halo-patch mode for 3x3 layers on large maps: an 8 x 16 pixel tile whose (16+2)-row neighbourhood is
   // loaded once per horizontal tap (first layer: once in total) instead of once per tap
-  if (p->ksize == 3 && p->H >= 64 && p->W >= 64) a.a_mode = 2;
+  if (c.ksize == 3 && c.H >= 64 && c.W >= 64) a.a_mode = 2;
   int TW = 1, TH = 1, NB = 128;
   if (a.a_mode == 2) {
     TW = 8; TH = 16; NB = 1;
     a.tw_log2 = 3; a.th_log2 = 4; a.nb_log2 = 0;
-    a.tiles_w = (p->W + TW - 1) / TW; a.tiles_h = (p->H + TH - 1) / TH; a.tiles_nb = p->N;
+    a.tiles_w = (c.W + TW - 1) / TW; a.tiles_h = (c.H + TH - 1) / TH; a.tiles_nb = c.N;
     a.m_tiles = a.tiles_w * a.tiles_h * a.tiles_nb;
   } else if (a.a_mode == 1) {
-    choose_box(p->N, p->H, p->W, pool, &TW, &TH, &NB);
+    choose_box(c.N, c.H, c.W, c.pool, &TW, &TH, &NB);
     a.tw_log2 = ilog2(TW); a.th_log2 = ilog2(TH); a.nb_log2 = ilog2(NB);
-    a.tiles_w = (p->W + TW - 1) / TW; a.tiles_h = (p->H + TH - 1) / TH; a.tiles_nb = (p->N + NB - 1) / NB;
+    a.tiles_w = (c.W + TW - 1) / TW; a.tiles_h = (c.H + TH - 1) / TH; a.tiles_nb = (c.N + NB - 1) / NB;
     a.m_tiles = a.tiles_w * a.tiles_h * a.tiles_nb;
   } else {
     a.m_tiles = (int)((a.M + TILE_M - 1) / TILE_M);
@@ -1547,8 +1492,8 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   Y2_ARG(a.M + TILE_M < (1ll << 31));
   Y2_ARG(a.kblocks <= MAX_UNITS);
   fastdiv_init((uint32_t)a.n_tiles, &a.fd_ntiles_mul, &a.fd_ntiles_shr);
-  fastdiv_init((uint32_t)(a.a_mode == 0 ? p->W : a.tiles_w), &a.fd_w_mul, &a.fd_w_shr);
-  fastdiv_init((uint32_t)(a.a_mode == 0 ? p->H : a.tiles_h), &a.fd_h_mul, &a.fd_h_shr);
+  fastdiv_init((uint32_t)(a.a_mode == 0 ? c.W : a.tiles_w), &a.fd_w_mul, &a.fd_w_shr);
+  fastdiv_init((uint32_t)(a.a_mode == 0 ? c.H : a.tiles_h), &a.fd_h_mul, &a.fd_h_shr);
   // bytes per pipeline stage that the TMA unit will report on the stage's mbarrier
   a.tx_bytes = (a.a_mode == 2 && a.first_layer ? a.a_sub_bytes : a.a_stage_bytes);
   fastdiv_init((uint32_t)a.cchunks, &a.fd_cch_mul, &a.fd_cch_shr);
@@ -1587,7 +1532,7 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   // halo-patch mode with a resident filter bank and a single channel chunk (layer 2: Cin = 32): the three
   // horizontally shifted patches share ONE stage, so the MMA warp issues all 9 taps behind one barrier round trip.
   // With one patch per stage that warp's ~800 clk of per-stage bookkeeping hid 192 clk of tensor work (ncu, r1c).
-  if (a.a_mode == 2 && !a.first_layer && a.b_stationary && (a.cchunks == 1 || split_in) &&
+  if (a.a_mode == 2 && !a.first_layer && a.b_stationary && (a.cchunks == 1 || c.split_in) &&
       a.b_total_bytes + 3 * (size_t)(3 * a.a_sub_bytes) <= SMEM_BUDGET) {
     a.kw_merge = 1;                                      // (several chunks -- the bf16x3 K extent -- : one merged stage per chunk)
     a.a_stage_bytes = 3 * a.a_sub_bytes;
@@ -1610,16 +1555,16 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   const size_t STG_BYTES = 4 * 2 * 8192;
   a.tma_store = 0;
   {
-    const bool common = a.a_mode == 2 && !pool && p->Cout % 32 == 0 && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(p->y) & 15) == 0 &&
+    const bool common = a.a_mode == 2 && !c.pool && c.Cout % 32 == 0 && a.ldy % 8 == 0 && (reinterpret_cast<uintptr_t>(c.y) & 15) == 0 &&
                         b_region + 3 * (size_t)stage_bytes + STG_BYTES <= SMEM_BUDGET;
     // bf16 rows: the 128-channel pair kernel (layer 3); float32 rows (training forward): also the first layer and the 64-channel
     // pair kernel (layer 2), whose 16-byte per-lane stores cost far more than the bf16 ones
     const bool shape_bf16 = !a.first_layer && block_n == 128 && a.row_bytes == 128 && a.cta2;
-    const bool shape_f32 = shape_bf16 || (a.first_layer && block_n == 32 && p->Cout == 32) ||
-                           (!a.first_layer && block_n == 64 && a.row_bytes == 64 && a.cta2 && p->Cout == 64);
+    const bool shape_f32 = shape_bf16 || (a.first_layer && block_n == 32 && c.Cout == 32) ||
+                           (!a.first_layer && block_n == 64 && a.row_bytes == 64 && a.cta2 && c.Cout == 64);
     // (64 columns on 128-byte operand rows -- layer 4 without the input-stationary kernel: 131 -> 141 us, not enabled)
-    if (common && !out_f32 && shape_bf16 && !split_out) a.tma_store = 1;
-    if (common && out_f32 && shape_f32 && !env().conv_no_tma_store_f32) a.tma_store = 1;
+    if (common && !c.out_f32 && shape_bf16 && !c.split_out) a.tma_store = 1;
+    if (common && c.out_f32 && shape_f32 && !env().conv_no_tma_store_f32) a.tma_store = 1;
   }
   const size_t stg_bytes = a.tma_store ? STG_BYTES : 0;
   int stages = (int)((SMEM_BUDGET - b_region - stg_bytes) / stage_bytes);
@@ -1633,100 +1578,108 @@ extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
   size_t smem = b_region + (size_t)stages * stage_bytes + stg_bytes + 1024;
 
   // ---- tensor maps ----
-  CUtensorMap tmA, tmB;
+  static const char* const who = "y2_conv_fwd_bf16";
+  CUtensorMap tmA, tmB, tmY;
   const CUtensorMapSwizzle sw = swizzle_for(a.row_bytes);
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)a_cin, (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
-    cuuint64_t strides[3] = {(cuuint64_t)a_cin * 2, (cuuint64_t)p->W * a_cin * 2, (cuuint64_t)p->H * p->W * a_cin * 2};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r;
-    if (a.a_mode == 0) {
-      int lower[2] = {-a.pad, -a.pad};
-      int upper[2] = {a.pad - (p->ksize - 1), a.pad - (p->ksize - 1)};
-      r = g_encodeIm2col(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p->x), dims, strides, lower, upper,
-                         (cuuint32_t)a.kchunk, (cuuint32_t)TILE_M, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      // same small-tensor fix-up CUTLASS applies (cute/atom/copy_traits_sm90_im2col.hpp) for drivers <= 13.1
-      if (r == CUDA_SUCCESS && g_driver_version <= 13010 && (size_t)a.M * a_cin * 2 < 131072)
-        reinterpret_cast<uint64_t*>(&tmA)[1] &= ~(1ull << 21);
-    } else if (a.a_mode == 2 && a.first_layer) {
-      // halo patch of the first layer: (8+2) px x 8 ch = 80 contiguous elements per row, 18 rows
-      cuuint64_t dims3[3] = {(cuuint64_t)p->W * 8, (cuuint64_t)p->H, (cuuint64_t)p->N};
-      cuuint64_t strides3[2] = {(cuuint64_t)p->W * 16, (cuuint64_t)p->H * p->W * 16};
-      cuuint32_t box3[3] = {80, 18, 1};
-      r = g_encodeTiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(p->x), dims3, strides3, box3, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else if (a.a_mode == 2) {
-      cuuint32_t box[4] = {(cuuint32_t)a.kchunk, 8, 18, 1};
-      r = g_encodeTiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p->x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else if (a.first_layer) {
-      // Cin_p == 8: pixels are 16 B, so (channel, w) is one contiguous dimension of W*8 elements.
-      // A [TW*8, TH, NB] box then moves 256-byte rows instead of 16-byte ones (16x fewer TMA requests);
-      // the left/right halo is still zero-filled because the shift is a multiple of one pixel.
-      cuuint64_t dims3[3] = {(cuuint64_t)p->W * 8, (cuuint64_t)p->H, (cuuint64_t)p->N};
-      cuuint64_t strides3[2] = {(cuuint64_t)p->W * 16, (cuuint64_t)p->H * p->W * 16};
-      cuuint32_t box3[3] = {(cuuint32_t)TW * 8, (cuuint32_t)TH, (cuuint32_t)NB};
-      r = g_encodeTiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(p->x), dims3, strides3, box3, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else {
-      cuuint32_t box[4] = {(cuuint32_t)a.kchunk, (cuuint32_t)TW, (cuuint32_t)TH, (cuuint32_t)NB};
-      r = g_encodeTiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p->x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    }
-    if (r != CUDA_SUCCESS) {
-      set_error("y2_conv_fwd_bf16: tensor map A encode failed (CUresult %d, mode %d)", (int)r, a.a_mode);
-      return Y2_ERR_DRIVER;
-    }
-  }
-  {
-    CUresult r;
+  int rc;
+  if (a.a_mode == 0) {
+    rc = tmap_im2col_nhwc(&tmA, c.x, c.N, c.H, c.W, c.a_cin, c.ksize, a.kchunk, TILE_M, sw, who, "A");
+  } else if (a.first_layer) {
+    // Cin_p == 8: pixels are 16 B, so (channel, w) is one contiguous dimension of W*8 elements.  The halo patch is
+    // (8+2) px x 8 ch = 80 contiguous elements per row, 18 rows; a tiled [TW*8, TH, NB] box moves 256-byte rows instead
+    // of 16-byte ones (16x fewer TMA requests), and its left/right halo is still zero-filled because the shift is a
+    // multiple of one pixel.
+    cuuint64_t dims3[3] = {(cuuint64_t)c.W * 8, (cuuint64_t)c.H, (cuuint64_t)c.N};
+    cuuint64_t strides3[2] = {(cuuint64_t)c.W * 16, (cuuint64_t)c.H * c.W * 16};
+    cuuint32_t box3[3] = {80, 18, 1};
+    if (a.a_mode == 1) { box3[0] = (cuuint32_t)TW * 8; box3[1] = (cuuint32_t)TH; box3[2] = (cuuint32_t)NB; }
     cuuint32_t estr[3] = {1, 1, 1};
-    if (a.first_layer) {
-      // packed as [kgroup=10][Cout_p][8]
-      cuuint64_t dims[3] = {8, (cuuint64_t)cout_p, 10};
-      cuuint64_t strides[2] = {16, (cuuint64_t)cout_p * 16};
-      cuuint32_t box[3] = {8, (cuuint32_t)block_n, 10};
-      r = g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(p->w_packed), dims, strides, box,
-                        estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else {
-      const int Kp = taps * a.cin_p;
-      cuuint64_t dims[2] = {(cuuint64_t)Kp, (cuuint64_t)cout_p};
-      cuuint64_t strides[1] = {(cuuint64_t)Kp * 2};
-      cuuint32_t box[2] = {(cuuint32_t)a.kchunk, (cuuint32_t)(a.cta2 ? block_n / 2 : block_n)};   // per-CTA slice of the B tile
-      r = g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p->w_packed), dims, strides, box,
-                        estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    }
-    if (r != CUDA_SUCCESS) {
-      set_error("y2_conv_fwd_bf16: tensor map B encode failed (CUresult %d)", (int)r);
-      return Y2_ERR_DRIVER;
-    }
+    rc = tmap_result(g_encodeTiled(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(c.x), dims3, strides3, box3, estr,
+                                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE),
+                     who, "A");
+  } else {
+    // halo patch (a_mode 2) or tiled box (a_mode 1)
+    const cuuint32_t box[4] = {(cuuint32_t)a.kchunk, a.a_mode == 2 ? 8u : (cuuint32_t)TW, a.a_mode == 2 ? 18u : (cuuint32_t)TH,
+                               a.a_mode == 2 ? 1u : (cuuint32_t)NB};
+    rc = tmap_nhwc_box(&tmA, c.x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, c.N, c.H, c.W, c.a_cin, c.a_cin, box, sw,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, who, "A");
   }
-  CUtensorMap tmY;
+  if (rc != Y2_OK) return rc;
+  if (a.first_layer) {
+    // packed as [kgroup=10][Cout_p][8]
+    cuuint64_t dims[3] = {8, (cuuint64_t)cout_p, 10};
+    cuuint64_t strides[2] = {16, (cuuint64_t)cout_p * 16};
+    cuuint32_t box[3] = {8, (cuuint32_t)block_n, 10};
+    cuuint32_t estr[3] = {1, 1, 1};
+    rc = tmap_result(g_encodeTiled(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(c.w_packed), dims, strides, box,
+                                   estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                                   CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE),
+                     who, "B");
+  } else {
+    // per-CTA slice of the B tile
+    rc = tmap_kmajor(&tmB, c.w_packed, c.taps * a.cin_p, cout_p, a.kchunk, a.cta2 ? block_n / 2 : block_n, sw,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, who, "B");
+  }
+  if (rc != Y2_OK) return rc;
   memset(&tmY, 0, sizeof(tmY));
   if (a.tma_store) {
     // output [N, H, W, Cout] with row stride ldy: boxes of 32 channels x the 8 x 16 pixel tile, 64-byte swizzled rows
     // (float32 rows: boxes of 16 channels -- the same 64 bytes per row)
-    const cuuint64_t es = out_f32 ? 4 : 2;
-    cuuint64_t dims[4] = {(cuuint64_t)p->Cout, (cuuint64_t)p->W, (cuuint64_t)p->H, (cuuint64_t)p->N};
-    cuuint64_t strides[3] = {(cuuint64_t)a.ldy * es, (cuuint64_t)p->W * a.ldy * es, (cuuint64_t)p->H * p->W * a.ldy * es};
-    cuuint32_t box[4] = {out_f32 ? 16u : 32u, 8, 16, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encodeTiled(&tmY, out_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, p->y, dims, strides, box, estr,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("y2_conv_fwd_bf16: tensor map Y encode failed (CUresult %d)", (int)r);
-      return Y2_ERR_DRIVER;
-    }
+    const cuuint32_t box[4] = {c.out_f32 ? 16u : 32u, 8, 16, 1};
+    rc = tmap_nhwc_box(&tmY, c.y, c.out_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, c.N, c.H, c.W,
+                       c.Cout, a.ldy, box, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, who, "Y");
+    if (rc != Y2_OK) return rc;
   }
-  (void)out_f32;
-  cudaStream_t st = (cudaStream_t)stream;
   return launch_conv(block_n, tmA, tmB, tmY, a, smem, st);
+}
+
+}  // namespace y2
+
+using namespace y2;
+
+extern "C" int y2_conv_fwd_bf16(const y2_conv_params* p, y2_stream_t stream) {
+  Y2_ARG(p != nullptr);
+  Y2_ARG(p->x && p->w_packed && p->y);
+  ConvCall c;
+  c.x = p->x; c.w_packed = p->w_packed; c.scale = p->scale; c.shift = p->shift; c.y = p->y;
+  c.alpha = p->alpha;
+  c.flags = p->flags;
+  c.N = p->N; c.H = p->H; c.W = p->W; c.Cin = p->Cin; c.Cout = p->Cout; c.ksize = p->ksize;
+  c.pad = c.ksize / 2;
+  c.taps = c.ksize * c.ksize;
+  c.M = (long long)c.N * c.H * c.W;
+  c.split_in = (p->flags & Y2_CONV_IN_SPLIT) != 0;
+  c.out_f32 = (p->flags & Y2_CONV_OUT_F32) != 0;
+  c.split_out = (p->flags & Y2_CONV_OUT_SPLIT) != 0 && !c.out_f32;
+  c.pool = (p->flags & Y2_CONV_POOL2) != 0;
+  c.leaky = (p->flags & Y2_CONV_LEAKY) != 0;
+  Y2_ARG(c.split_out || p->lo_off == 0);
+  if (c.split_in) Y2_ARG(c.Cin % 32 == 0);
+  Y2_ARG(c.N > 0 && c.H > 0 && c.W > 0 && c.Cin > 0 && c.Cout > 0 && (c.ksize == 1 || c.ksize == 3));
+  if (c.pool) Y2_ARG(c.H % 2 == 0 && c.W % 2 == 0);
+  c.lo_off = c.split_out ? (p->lo_off > 0 ? p->lo_off : c.Cout) : 0;
+  c.ldy = p->ldy > 0 ? p->ldy : (c.split_out ? 2 * c.Cout : c.Cout);
+  Y2_ARG(c.ldy >= c.Cout);
+  if (c.split_out) {
+    Y2_ARG(c.lo_off >= c.Cout);
+    Y2_ARG(c.ldy >= c.lo_off + c.Cout);
+  }
+  c.a_cin = c.split_in ? 2 * c.Cin : y2_conv_cin_padded(c.Cin);
+  c.b_cin = c.split_in ? 3 * c.Cin : c.a_cin;
+  if (c.b_cin == 8) Y2_ARG(c.ksize == 3);         // the first layer (3 channels padded to 8)
+  if (c.b_cin != 8 && c.Cin % 32 != 0) {
+    set_error("y2_conv_fwd_bf16: Cin=%d unsupported (need 3, or a multiple of 32)", c.Cin);
+    return Y2_ERR_UNSUPPORTED;
+  }
+  int rc = load_driver_entry_points();
+  if (rc != Y2_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  int handled = 0;
+  // float32 pre-BN rows of a deep 3x3 layer on a small map: 256x256 stream-K tiles (conv_streamk_tcgen05.cu)
+  rc = conv_streamk_try(c, st, &handled);
+  if (rc != Y2_OK || handled) return rc;
+  rc = conv_is_try(c, st, &handled);
+  if (rc != Y2_OK || handled) return rc;
+  return conv_generic(c, st);
 }

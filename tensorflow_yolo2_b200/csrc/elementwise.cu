@@ -346,52 +346,6 @@ __global__ void bn_update_moving_kernel(float* __restrict__ mm, float* __restric
   mv[c] = mv[c] * momentum + var[c] * (1.0f - momentum);
 }
 
-// Batch statistics from the per-slab partials the stream-K conv epilogue writes (conv_streamk_tcgen05.cu: sk_slab_stats):
-// slabs [nslab][3][C] = (k, sum(x - k), sum((x - k)^2)) over each 32-row slab.  Chan's pairwise merge in float64, slabs
-// folded in a fixed order (deterministic): block (32 columns, FIN_TY slab lanes), then one lane folds the FIN_TY partials.
-__global__ void __launch_bounds__(32 * 32) bn_stats_from_slabs_kernel(const float* __restrict__ slabs, int nslab, int slab_rows, int M,
-                                                                     int C, float* __restrict__ mean, float* __restrict__ var,
-                                                                     const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                                     float eps, float* __restrict__ scale, float* __restrict__ shift) {
-  __shared__ double s_n[32][33], s_mu[32][33], s_m2[32][33];
-  const int c = blockIdx.x * 32 + threadIdx.x;
-  double n = 0.0, mu = 0.0, m2 = 0.0;
-  if (c < C)
-    for (int s = threadIdx.y; s < nslab; s += 32) {
-      const float* p = slabs + (size_t)s * 3 * C + c;
-      const double nb = (double)min(slab_rows, M - s * slab_rows);
-      const double k = (double)p[0], s1 = (double)p[C], s2 = (double)p[2 * C];
-      const double mub = k + s1 / nb, m2b = s2 - s1 * s1 / nb;
-      const double nt = n + nb, delta = mub - mu;
-      mu += delta * nb / nt;
-      m2 += m2b + delta * delta * n * nb / nt;
-      n = nt;
-    }
-  s_n[threadIdx.y][threadIdx.x] = n;
-  s_mu[threadIdx.y][threadIdx.x] = mu;
-  s_m2[threadIdx.y][threadIdx.x] = m2;
-  __syncthreads();
-  if (threadIdx.y != 0 || c >= C) return;
-  for (int y = 1; y < 32; ++y) {
-    const double nb = s_n[y][threadIdx.x];
-    if (nb == 0.0) continue;
-    const double mub = s_mu[y][threadIdx.x], m2b = s_m2[y][threadIdx.x];
-    const double nt = n + nb, delta = mub - mu;
-    mu += delta * nb / nt;
-    m2 += m2b + delta * delta * n * nb / nt;
-    n = nt;
-  }
-  double v = m2 / (double)M;
-  if (v < 0.0) v = 0.0;
-  mean[c] = (float)mu;
-  const float vf = (float)v;
-  var[c] = vf;
-  if (scale) {
-    scale[c] = gamma[c] * rsqrtf(vf + eps);
-    shift[c] = beta[c];
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
 // a2/a3  y = leaky((x - sub)*scale + shift), optional 2x2/2 max-pool (order conv->BN->leaky->pool,
 // darknet.py:150-151), f32 or bf16 output.  One thread per output element group of VEC channels.
@@ -913,17 +867,6 @@ int y2_bn_stats_fold(const float* x, int M, int C, int ld, float* mean, float* v
                      float eps, float* scale, float* shift, void* workspace, size_t workspace_bytes, y2_stream_t stream) {
   Y2_ARG(gamma && beta && scale && shift);
   return bn_stats_impl(x, M, C, ld, mean, var, gamma, beta, eps, scale, shift, workspace, workspace_bytes, stream);
-}
-
-int y2_bn_stats_from_slabs(const float* slabs, int M, int C, int slab_rows, float* mean, float* var, const float* gamma,
-                           const float* beta, float eps, float* scale, float* shift, y2_stream_t stream) {
-  Y2_ARG(slabs && mean && var && M > 0 && C > 0 && slab_rows > 0);
-  Y2_ARG((scale == nullptr) == (shift == nullptr) && (!scale || (gamma && beta)));
-  const int nslab = (M + slab_rows - 1) / slab_rows;
-  bn_stats_from_slabs_kernel<<<(C + 31) / 32, dim3(32, 32), 0, (cudaStream_t)stream>>>(slabs, nslab, slab_rows, M, C, mean, var, gamma,
-                                                                                      beta, eps, scale, shift);
-  Y2_LAUNCHED();
-  return Y2_OK;
 }
 
 int y2_bn_stats_fold_train(const float* x, int M, int C, int ld, float* mean, float* var, const float* gamma, const float* beta,

@@ -221,6 +221,55 @@ extern int g_driver_version;
 
 int load_driver_entry_points();   // defined in conv_tcgen05.cu
 
+// Tensor maps shared by the tensor-core kernels (defined in conv_tcgen05.cu).  Each returns Y2_OK, or sets the error
+// "<who>: tensor map <name> encode failed" and returns Y2_ERR_DRIVER.
+// bf16 NHWC [N][H][W][C] read in im2col mode for a ksize x ksize SAME window: `pixels` rows of `chans` channels per load
+int tmap_im2col_nhwc(CUtensorMap* tm, const void* x, int N, int H, int W, int C, int ksize, int chans, int pixels,
+                     CUtensorMapSwizzle sw, const char* who, const char* name);
+// NHWC [N][H][W][C] of bf16 or float32 whose pixels are `ld` elements apart, read or written in [c, w, h, n] boxes
+int tmap_nhwc_box(CUtensorMap* tm, const void* base, CUtensorMapDataType dt, int N, int H, int W, int C, int ld,
+                  const cuuint32_t box[4], CUtensorMapSwizzle sw, CUtensorMapL2promotion l2, const char* who, const char* name);
+// bf16 K-major rows [rows][K] (packed weights, row-major gradients), read in [box_k, box_rows] boxes
+int tmap_kmajor(CUtensorMap* tm, const void* base, int K, long long rows, int box_k, int box_rows, CUtensorMapSwizzle sw,
+                CUtensorMapL2promotion l2, const char* who, const char* name);
+
+// Launch with a cluster dimension and, unless Y2_NO_PDL is set, programmatic dependent launch (fill_launch_attrs)
+template <typename... KArgs, typename... Args>
+static int launch_cluster(void (*kernel)(KArgs...), int grid, int threads, size_t smem, unsigned cluster, cudaStream_t st,
+                          const Args&... args) {
+  Y2_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3((unsigned)grid);
+  cfg.blockDim = dim3((unsigned)threads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[2];
+  cfg.attrs = attr;
+  cfg.numAttrs = fill_launch_attrs(attr, cluster);
+  Y2_CUDA(cudaLaunchKernelEx(&cfg, kernel, args...));
+  Y2_LAUNCHED();
+  return Y2_OK;
+}
+
+// One y2_conv_fwd_bf16 call, parsed and checked before any kernel path sees it.  The paths (stream-K, input-stationary,
+// generic) only decide whether they can run it.
+struct ConvCall {
+  const void* x;
+  const void* w_packed;
+  const float* scale;
+  const float* shift;
+  void* y;
+  float alpha;
+  int flags;
+  int N, H, W, Cin, Cout, ksize, pad, taps;
+  long long M;                      // N * H * W output rows before pooling
+  bool split_in, split_out, out_f32, pool, leaky;   // split_out: OUT_SPLIT without OUT_F32
+  int ldy, lo_off;                  // resolved: ldy >= Cout; with split_out lo_off >= Cout and ldy >= lo_off + Cout, else 0
+  int a_cin;                        // channels per pixel of x: 2 Cin ([hi | lo]) with IN_SPLIT, else y2_conv_cin_padded(Cin)
+  int b_cin;                        // K extent per tap of w_packed: 3 Cin ([w_hi | w_hi | w_lo]) with IN_SPLIT, else a_cin
+};
+
 static inline CUtensorMapSwizzle swizzle_for(int row_bytes) {
   return row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
                                                                           : CU_TENSOR_MAP_SWIZZLE_NONE;

@@ -115,7 +115,6 @@ class Yolo2Engine:
             self.in_f32 = torch.zeros((N, IS, IS, 3), **f32) if input_kind == 'f32' else None
             self.x0 = torch.empty((N, IS, IS, 8), dtype=torch.bfloat16, device=dev)
             self.acts, self.raw, self.stats = [], {}, {}
-            self.slab_rows, self.slabs = {}, {}           # batch-stat layers whose conv epilogue emits the BN partials
             H = IS
             max_ws = 1
             self.pt_src = None
@@ -248,28 +247,10 @@ class Yolo2Engine:
                 raw = self.raw[li]
                 mean, var, scale, shift, zeros = self.stats[li]
                 bn = L['bn']
-                kw = dict(scale=None, shift=st[L['b']], leaky=False, pool=False, out_f32=True, ldy=raw.shape[1], out=raw, split_in=x3)
-                if li not in self.slab_rows:
-                    # does this layer run on the stream-K kernel, whose epilogue can emit the batch-norm partials?  (decided
-                    # once, outside any graph capture: the first enqueue is the warm-up.)  OPT-IN (Y2_FUSED_BN_STATS=1):
-                    # measured slower on B200 -- 1.74-1.76 vs 1.69-1.70 ms per step in two same-run A/Bs: the column pass
-                    # lengthens the stream-K epilogue, which is only partly hidden behind the next segment's MMAs, by more
-                    # than the 17 us statistics pass it replaces (DESIGN.md section 4.1)
-                    R = 0 if not os.environ.get('Y2_FUSED_BN_STATS') else ops.conv_fwd_bf16(
-                        x, self.packed[li], L['k'], L['cin'], L['cout'], _query_slab_rows=True, **kw)
-                    self.slab_rows[li] = R
-                    if R:
-                        M = raw.shape[0]
-                        self.slabs[li] = torch.empty(((M + R - 1) // R, 3, L['cout']), dtype=torch.float32, device=self.device)
-                R = self.slab_rows[li]
-                if R:
-                    ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], stats_slabs=self.slabs[li], **kw)
-                    ops.bn_stats_from_slabs(self.slabs[li], raw.shape[0], L['cout'], R, st[bn['gamma']], st[bn['beta']],
-                                            mean=mean, var=var, scale=scale, shift=shift)
-                else:
-                    ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], **kw)
-                    ops.bn_stats_fold(raw, L['cout'], st[bn['gamma']], st[bn['beta']], ld=raw.shape[1], workspace=self.ws,
-                                      mean=mean, var=var, scale=scale, shift=shift)
+                ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], scale=None, shift=st[L['b']], leaky=False,
+                                  pool=False, out_f32=True, ldy=raw.shape[1], out=raw, split_in=x3)
+                ops.bn_stats_fold(raw, L['cout'], st[bn['gamma']], st[bn['beta']], ld=raw.shape[1], workspace=self.ws,
+                                  mean=mean, var=var, scale=scale, shift=shift)
                 ops.affine_leaky_pool(raw, self.N, Hl, Hl, L['cout'], ldx=raw.shape[1], sub=mean, scale=scale, shift=shift,
                                       leaky=True, pool=pool, out_bf16=not last, out=out, ldo=ldo, out_col=col,
                                       space_to_depth=s2d, split_out=x3)

@@ -113,8 +113,7 @@ def pack_weights_bf16_split(w_hwio, out=None):
 
 
 def conv_fwd_bf16(x, w_packed, ksize, cin, cout, scale=None, shift=None, leaky=True, pool=False, out_f32=False,
-                  ldy=None, out=None, alpha=ALPHA, out_col=0, split_in=False, split_out=False, lo_off=0, stats_slabs=None,
-                  _query_slab_rows=False):
+                  ldy=None, out=None, alpha=ALPHA, out_col=0, split_in=False, split_out=False, lo_off=0):
     """x bf16 [N,H,W,Cin_p]; returns bf16 [N,Ho,Wo,Cout] or (out_f32) f32 [N*H*W, ldy].
     bf16x3 mode: split_in -> x is [N,H,W,2*Cin] = [hi | lo] and w_packed comes from pack_weights_bf16_split;
     split_out -> the bf16 result is [N,Ho,Wo,2*Cout] = [hi | lo] (lo at column lo_off or Cout of a row of stride ldy)."""
@@ -134,10 +133,7 @@ def conv_fwd_bf16(x, w_packed, ksize, cin, cout, scale=None, shift=None, leaky=T
             out = torch.empty((N, Ho, Wo, ld), dtype=torch.bfloat16, device=x.device)
     prm = ConvParams(x=_p(x, torch.bfloat16), w_packed=_p(w_packed, torch.bfloat16), scale=_p(scale, torch.float32),
                      shift=_p(shift, torch.float32), y=_p_off(out, out_col), N=N, H=H, W=W, Cin=cin, Cout=cout, ksize=ksize,
-                     flags=flags, alpha=alpha, ldy=ld, lo_off=int(lo_off) if split_out else 0,
-                     stats_slabs=_p(stats_slabs, torch.float32))
-    if _query_slab_rows:          # plan only: would this call emit batch-norm slab statistics (and over how many rows each)?
-        return int(_lib.load().y2_conv_stats_slab_rows(C.byref(prm)))
+                     flags=flags, alpha=alpha, ldy=ld, lo_off=int(lo_off) if split_out else 0)
     check(_lib.load().y2_conv_fwd_bf16(C.byref(prm), _stream()), 'y2_conv_fwd_bf16')
     return out
 
@@ -304,19 +300,6 @@ def bn_stats_fold_train(x2d, C_, gamma, beta, moving_mean, moving_var, ld=None, 
                                      _p(beta, torch.float32), eps, _p(scale), _p(shift), _p(moving_mean, torch.float32),
                                      _p(moving_var, torch.float32), momentum, _p(ws), ws.numel(), _stream()),
           'y2_bn_stats_fold_train')
-    return mean, var, scale, shift
-
-
-def bn_stats_from_slabs(slabs, M, C_, slab_rows, gamma=None, beta=None, mean=None, var=None, scale=None, shift=None, eps=BN_EPS):
-    """Fold the slab partials of conv_fwd_bf16(stats_slabs=...) into (mean, biased var[, scale, shift])."""
-    new = lambda: torch.empty((C_,), dtype=torch.float32, device=slabs.device)
-    mean = new() if mean is None else mean
-    var = new() if var is None else var
-    if gamma is not None:
-        scale = new() if scale is None else scale
-        shift = new() if shift is None else shift
-    check(_lib.load().y2_bn_stats_from_slabs(_p(slabs, torch.float32), M, C_, slab_rows, _p(mean), _p(var), _p(gamma, torch.float32),
-                                             _p(beta, torch.float32), eps, _p(scale), _p(shift), _stream()), 'y2_bn_stats_from_slabs')
     return mean, var, scale, shift
 
 

@@ -652,40 +652,25 @@ def test_loss_box_deltas_histogram_inputs(ops, golden_dir):
     np.testing.assert_allclose(got, want, rtol=1e-6, atol=1e-6)
 
 
-# ---------------------------------------------------------------------------------- a2: BN partials out of the conv epilogue
-@pytest.mark.parametrize('N,S,Cin,Cout,k,big_mean', [(32, 13, 512, 1024, 3, False), (70, 13, 512, 512, 3, True)])
-def test_conv_streamk_fused_bn_statistics(ops, N, S, Cin, Cout, k, big_mean):
-    """y2_conv_params.stats_slabs + y2_bn_stats_from_slabs == y2_bn_stats over the stored float32 rows (mean and biased
-    variance), also when |mean| >> std (bias 1e4: the shifted per-slab sums must not cancel) and with a ragged last slab
-    (70 * 169 = 11830 rows)."""
-    rs = np.random.RandomState(Cin + N)
-    x = rs.randn(N, S, S, Cin).astype(np.float32)
-    w = (rs.randn(k, k, Cin, Cout) * 0.05).astype(np.float32)
-    b = (rs.randn(Cout) + (1e4 if big_mean else 0.0)).astype(np.float32)
-    xb, wp, bt = cu(x, torch.bfloat16), ops.pack_weights_bf16(cu(w)), cu(b)
+# ---------------------------------------------------------------------------------- a1: the call is checked before any path
+def test_conv_streamk_shape_with_overlapping_output_rows_is_refused(ops):
+    """A 64x13x13 1024 -> 1024 3x3 layer runs on the stream-K kernel (the default workspace is registered).  Output rows that
+    overlap are refused before that kernel is planned: float32 rows of stride 256 < Cout, and hi | lo bf16 rows whose lo
+    half starts at column 8, inside the hi half.  Each output holds every address such a launch would write, so a call that
+    got through would still stay in bounds."""
+    from tensorflow_yolo2_b200 import _lib
+    N, S, C_ = 64, 13, 1024
     M = N * S * S
-    raw = torch.empty((M, Cout), dtype=torch.float32, device='cuda')
-    kw = dict(scale=None, shift=bt, leaky=False, pool=False, out_f32=True, ldy=Cout, out=raw)
-    R = ops.conv_fwd_bf16(xb, wp, k, Cin, Cout, _query_slab_rows=True, **kw)
-    assert R == 32                                           # these shapes run on the CTA-pair stream-K kernel
-    slabs = torch.full(((M + R - 1) // R, 3, Cout), float('nan'), dtype=torch.float32, device='cuda')
-    ops.conv_fwd_bf16(xb, wp, k, Cin, Cout, stats_slabs=slabs, **kw)
-    gamma, beta = cu(rs.uniform(0.5, 1.5, Cout).astype(np.float32)), cu(rs.randn(Cout).astype(np.float32))
-    mean, var, scale, shift = ops.bn_stats_from_slabs(slabs, M, Cout, R, gamma, beta)
-    m2, v2, sc2, sh2 = ops.bn_stats_fold(raw, Cout, gamma, beta)
-    assert not torch.isnan(slabs).any()
-    np.testing.assert_allclose(mean.cpu().numpy(), m2.cpu().numpy(), rtol=1e-6, atol=1e-6)
-    np.testing.assert_allclose(var.cpu().numpy(), v2.cpu().numpy(), rtol=2e-5)
-    np.testing.assert_allclose(scale.cpu().numpy(), sc2.cpu().numpy(), rtol=2e-5)
-    assert torch.equal(shift, sh2)
-    # and against float64 on the stored rows
-    r64 = raw.double()
-    np.testing.assert_allclose(var.cpu().numpy(), r64.var(dim=0, unbiased=False).cpu().numpy(), rtol=2e-5)
-    # a layer that does not run on stream-K reports 0 and refuses the buffer
-    xs, ws = cu(rs.randn(2, 8, 8, 64).astype(np.float32), torch.bfloat16), ops.pack_weights_bf16(cu(rs.randn(3, 3, 64, 256).astype(np.float32)))
-    assert ops.conv_fwd_bf16(xs, ws, 3, 64, 256, out_f32=True, _query_slab_rows=True) == 0
-    with pytest.raises(Exception):
-        ops.conv_fwd_bf16(xs, ws, 3, 64, 256, out_f32=True, stats_slabs=slabs)
+    x = torch.zeros((N, S, S, C_), dtype=torch.bfloat16, device='cuda')
+    wp = ops.pack_weights_bf16(torch.zeros((3, 3, C_, C_), dtype=torch.float32, device='cuda'))
+    y32 = torch.zeros((M * C_,), dtype=torch.float32, device='cuda')
+    with pytest.raises(_lib.Y2Error, match='ldy >= c.Cout'):
+        ops.conv_fwd_bf16(x, wp, 3, C_, C_, out_f32=True, ldy=256, out=y32)
+    y16 = torch.zeros((M * 2 * C_,), dtype=torch.bfloat16, device='cuda')
+    with pytest.raises(_lib.Y2Error, match='lo_off >= c.Cout'):
+        ops.conv_fwd_bf16(x, wp, 3, C_, C_, split_out=True, lo_off=8, ldy=2 * C_, out=y16)
+    torch.cuda.synchronize()
+    assert not y32.any() and not y16.any()
 
 
 # ---------------------------------------------------------------------------------- a10 / f2: cv2.resize on the GPU
