@@ -1,8 +1,9 @@
 """Batch inference engine: Darknet19 + detection head -> decode -> per-class NMS, all buffers
 pre-allocated, weights pre-packed, inference-mode BN pre-folded, the whole step captured in one
-CUDA graph.  It issues exactly the kernels the eager builders in yolo2_nets/darknet.py issue (same
-C-ABI entry points); it exists because a 22-layer network at >10 k images/s is launch-bound from
-Python otherwise.
+CUDA graph.  Every conv layer except the fused uint8 first one (conv1_u8_pool) goes through
+yolo2_nets.darknet.conv_bn_tc, the routine behind the eager builders' tensor-core path, so the
+engine issues the builders' kernels into its own buffers.  It exists because a 22-layer network at
+>10 k images/s is launch-bound from Python otherwise.
 
 The layer semantics follow the reference scripts (src/pascal/pascal_detect_darknet.py:41-43):
 core with is_training=False (moving statistics), head with is_training=True (batch statistics
@@ -17,40 +18,27 @@ import torch
 
 from . import ops
 from .variables import VariableStore
-from .yolo2_nets.darknet import CORE_PLAN
+from .yolo2_nets.darknet import (CORE_PLAN, PASSTHROUGH_FILTERS, PASSTHROUGH_LAYER, classifier_plan, conv_bn_tc,
+                                  head_plan, raw_ld)
 from .yolo2_nets.net_utils import VOC_ANCHORS
 
-HEAD_SCOPES = ('conv1', 'conv2', 'conv3', 'output')
 
-
-PASSTHROUGH_LAYER = 12       # CORE_PLAN index of the 26x26x512 layer (darknet.py:170); its UN-pooled output is the source
-PASSTHROUGH_FILTERS = 64
+def _layer_variables(store, k, cin, cout, pool=False, **kw):
+    wn, _ = store.weight_variable([k, k, cin, cout])
+    bn_, _ = store.bias_variable([cout])
+    return dict(k=k, cin=cin, cout=cout, pool=pool, W=wn, b=bn_, bn=store.batch_norm_variables(cout), **kw)
 
 
 def create_variables(store, output_filter, passthrough=False):
-    """Create (or find) every variable in the reference's creation order and naming.  passthrough=True adds the
-    YOLOv2 passthrough branch (absent from the reference, SURVEY Appendix A): scope darknet19_detection/passthrough
-    (1x1, 512 -> 64), and conv3 takes 1024 + 256 input channels."""
+    """Create (or find) every variable of darknet19_core + darknet19_detection in the reference's creation order and naming.
+    passthrough=True adds the YOLOv2 passthrough branch of yolo2_nets.darknet.head_plan."""
     store.reset_name_counters()
-    layers = []
     with store.scope('darknet19'):
-        for (k, cin, cout, pool) in CORE_PLAN:
-            wn, _ = store.weight_variable([k, k, cin, cout])
-            bn_, _ = store.bias_variable([cout])
-            layers.append(dict(k=k, cin=cin, cout=cout, pool=pool, W=wn, b=bn_, bn=store.batch_norm_variables(cout),
-                               head=False))
+        layers = [_layer_variables(store, *p, head=False) for p in CORE_PLAN]
     with store.scope('darknet19_detection'):
-        cat = 1024 + 4 * PASSTHROUGH_FILTERS if passthrough else 1024
-        plan = [('conv1', 3, 1024, 1024), ('conv2', 3, 1024, 1024)]
-        if passthrough:
-            plan.append(('passthrough', 1, 512, PASSTHROUGH_FILTERS))
-        plan += [('conv3', 3, cat, 1024), ('output', 1, 1024, output_filter)]
-        for sc, k, cin, cout in plan:
+        for sc, k, cin, cout in head_plan(output_filter, PASSTHROUGH_FILTERS if passthrough else 0):
             with store.scope(sc):
-                wn, _ = store.weight_variable([k, k, cin, cout])
-                bn_, _ = store.bias_variable([cout])
-                layers.append(dict(k=k, cin=cin, cout=cout, pool=False, W=wn, b=bn_,
-                                   bn=store.batch_norm_variables(cout), head=True, role=sc))
+                layers.append(_layer_variables(store, k, cin, cout, head=True, role=sc))
     return layers
 
 
@@ -59,13 +47,9 @@ def create_classifier_variables(store, num_classes=1000):
     19th conv_bn_layer (1x1, 1024 -> num_classes) in the SAME scope, so its names continue the core's numbering
     (darknet19/Variable_36, Variable_37, batch_normalization_18)."""
     store.reset_name_counters()
-    layers = []
     with store.scope('darknet19'):
-        for (k, cin, cout, pool) in list(CORE_PLAN) + [(1, 1024, int(num_classes), False)]:
-            wn, _ = store.weight_variable([k, k, cin, cout])
-            bn_, _ = store.bias_variable([cout])
-            layers.append(dict(k=k, cin=cin, cout=cout, pool=pool, W=wn, b=bn_, bn=store.batch_norm_variables(cout),
-                               head=len(layers) == len(CORE_PLAN), role='logits' if len(layers) == len(CORE_PLAN) else None))
+        layers = [_layer_variables(store, *p, head=False, role=None) for p in CORE_PLAN]
+        layers.append(_layer_variables(store, *classifier_plan(num_classes), head=True, role='logits'))
     return layers
 
 
@@ -138,13 +122,10 @@ class Yolo2Engine:
                     self.acts.append(torch.empty((N, Ho, Ho, cm * L['cout']), dtype=torch.bfloat16, device=dev))
                 if self.passthrough and li == PASSTHROUGH_LAYER:
                     self.pt_src = torch.empty((N, H, H, L['cout']), dtype=torch.bfloat16, device=dev)
-                if training or last or role == 'passthrough':
-                    ld = (L['cout'] + 31) // 32 * 32
-                    self.raw[li] = torch.empty((N * Hin * Hin, ld), **f32)
+                if training or last or role == 'passthrough':                # conv_bn_tc writes float32 conv rows
+                    self.raw[li] = torch.empty((N * Hin * Hin, raw_ld(L['cout'])), **f32)
                 if training:
-                    self.stats[li] = (torch.empty((L['cout'],), **f32), torch.empty((L['cout'],), **f32),
-                                      torch.empty((L['cout'],), **f32), torch.empty((L['cout'],), **f32),
-                                      torch.zeros((L['cout'],), **f32))
+                    self.stats[li] = tuple(torch.empty((L['cout'],), **f32) for _ in range(4))     # mean, var, scale, shift
                     max_ws = max(max_ws, ops.bn_stats_workspace_bytes(N * Hin * Hin, L['cout']))
                 H = Ho
             self.ws = torch.empty((max_ws,), dtype=torch.uint8, device=dev)
@@ -209,56 +190,29 @@ class Yolo2Engine:
         else:
             ops.pad_cast_f32_to_bf16c8(self.in_f32, out=self.x0)
         x = self.x0
-        H = self.IS
         nl = len(self.layers)
         for li, L in enumerate(self.layers):
             training = self.head_training if L['head'] else self.core_training
-            last = li == nl - 1
             out = self.acts[li]
             role = L.get('role')
             pt_source = self.passthrough and li == PASSTHROUGH_LAYER      # un-pooled output wanted too
-            pool = L['pool'] and not pt_source
-            if pt_source:
-                out = self.pt_src
-            # where the layer's activation goes: dense, or a channel slice of the concat buffer
-            ldo, col, s2d = None, 0, False
-            Hl = H
-            if self.passthrough and role == 'conv2':
-                ldo = out.shape[-1]
-            elif role == 'passthrough':
-                x, Hl = self.pt_src, 2 * H
-                ldo, col, s2d = out.shape[-1], 1024, True
-            x3 = self.x3
             if li == 0 and self.fused_conv1:
-                ops.conv1_u8_pool(self.in_u8, self.packed_c1, self.fold[0][1], out=out, split=x3)
-            elif not training:
-                scale, shift = self.fold[li]
-                if last or s2d:
-                    raw = self.raw[li]
-                    ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], scale=scale, shift=shift,
-                                      leaky=True, pool=False, out_f32=True, ldy=raw.shape[1], out=raw, split_in=x3)
-                    # compact the padded rows (detection output) / scatter them space-to-depth (passthrough)
-                    ops.affine_leaky_pool(raw, self.N, Hl, Hl, L['cout'], ldx=raw.shape[1], leaky=False, pool=False,
-                                          out_bf16=not last, out=out, ldo=ldo, out_col=col, space_to_depth=s2d, split_out=x3)
-                else:
-                    ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], scale=scale, shift=shift,
-                                      leaky=True, pool=pool, out=out, ldy=ldo, split_in=x3, split_out=x3)
+                ops.conv1_u8_pool(self.in_u8, self.packed_c1, self.fold[0][1], out=out, split=self.x3)
             else:
-                raw = self.raw[li]
-                mean, var, scale, shift, zeros = self.stats[li]
+                # where the layer's activation goes: dense, or a channel slice of the concat buffer
+                ldo, col, s2d = None, 0, False
+                if self.passthrough and role == 'conv2':
+                    ldo = out.shape[-1]
+                elif role == 'passthrough':
+                    x, ldo, col, s2d = self.pt_src, out.shape[-1], 1024, True
                 bn = L['bn']
-                ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], scale=None, shift=st[L['b']], leaky=False,
-                                  pool=False, out_f32=True, ldy=raw.shape[1], out=raw, split_in=x3)
-                ops.bn_stats_fold(raw, L['cout'], st[bn['gamma']], st[bn['beta']], ld=raw.shape[1], workspace=self.ws,
-                                  mean=mean, var=var, scale=scale, shift=shift)
-                ops.affine_leaky_pool(raw, self.N, Hl, Hl, L['cout'], ldx=raw.shape[1], sub=mean, scale=scale, shift=shift,
-                                      leaky=True, pool=pool, out_bf16=not last, out=out, ldo=ldo, out_col=col,
-                                      space_to_depth=s2d, split_out=x3)
+                conv_bn_tc(x, self.packed[li], L['k'], L['cin'], L['cout'], fold=None if training else self.fold[li],
+                           bias=st[L['b']], gamma=st[bn['gamma']], beta=st[bn['beta']], stats=self.stats.get(li),
+                           workspace=self.ws, pool=L['pool'] and not pt_source, out_f32=li == nl - 1,
+                           out=self.pt_src if pt_source else out, ldo=ldo, col=col, s2d=s2d, x3=self.x3, raw=self.raw.get(li))
             if pt_source:
                 ops.maxpool2x2_bf16(self.pt_src, out=self.acts[li])
             x = self.acts[li]
-            if L['pool']:
-                H //= 2
         if self.decode == 'region':
             if self.C == 20 and self.nbox <= 4095 and self.fused_detect:
                 if self.detect_impl == 'split' and self.A == 5:

@@ -32,6 +32,7 @@ from . import ops
 from .engine import create_classifier_variables, create_variables
 from .parallel import BucketedAllReduce, bucket_segments, make_buckets
 from .variables import VariableStore
+from .yolo2_nets.darknet import conv_bn_tc, raw_ld
 from .yolo2_nets.net_utils import VOC_ANCHORS
 
 
@@ -160,14 +161,13 @@ class Yolo2Trainer:
             Ho = H // 2 if L['pool'] else H
             last = li == nl - 1
             cout, cin, k = L['cout'], L['cin'], L['k']
-            ldh = _round_up(cout, 32)
+            ldh = raw_ld(cout)
             ld_dh = 32 if li == 0 else _round_up(cout, 64)
             self.geom.append(dict(H=H, Ho=Ho, ldh=ldh, ld_dh=ld_dh, M=N * H * H))
             self.acts.append(torch.empty((N, Ho, Ho, cout), **(f32 if last else bf16)))
             self.raw.append(torch.empty((N * H * H, ldh), **f32))
             self.stats.append(dict(mean=torch.empty((cout,), **f32), var=torch.empty((cout,), **f32),
-                                   scale=torch.empty((cout,), **f32), shift=torch.empty((cout,), **f32),
-                                   zeros=torch.zeros((cout,), **f32)))
+                                   scale=torch.empty((cout,), **f32), shift=torch.empty((cout,), **f32)))
             max_ws = max(max_ws, ops.bn_stats_workspace_bytes(N * H * H, cout), ops.bn_bwd_workspace_bytes(N * H * H, cout))
             max_dh = max(max_dh, N * H * H * ld_dh)
             if li > 0:
@@ -233,25 +233,12 @@ class Yolo2Trainer:
         x = self.x0
         nl = len(self.layers)
         for li, L in enumerate(self.layers):
-            g, s, P = self.geom[li], self.stats[li], self.P[li]
-            H, last = g['H'], li == nl - 1
+            s, P, bn = self.stats[li], self.P[li], L['bn']
             ops.pack_weights_bf16(P['W'], out=self.packed[li])
-            raw = self.raw[li]
-            ops.conv_fwd_bf16(x, self.packed[li], L['k'], L['cin'], L['cout'], scale=None, shift=P['b'], leaky=False,
-                              pool=False, out_f32=True, ldy=g['ldh'], out=raw)
-            # batch statistics, the centred affine (scale = gamma * rsqrt(var + eps), shift = beta) and the UPDATE_OPS of the
-            # moving averages: two launches
-            if self.update_moving:
-                bn = L['bn']
-                ops.bn_stats_fold_train(raw, L['cout'], P['gamma'], P['beta'], self.store[bn['moving_mean']],
-                                        self.store[bn['moving_variance']], ld=g['ldh'], workspace=self.ws, mean=s['mean'],
-                                        var=s['var'], scale=s['scale'], shift=s['shift'])
-            else:
-                ops.bn_stats_fold(raw, L['cout'], P['gamma'], P['beta'], ld=g['ldh'], workspace=self.ws, mean=s['mean'],
-                                  var=s['var'], scale=s['scale'], shift=s['shift'])
-            ops.affine_leaky_pool(raw, self.N, H, H, L['cout'], ldx=g['ldh'], sub=s['mean'], scale=s['scale'],
-                                  shift=s['shift'], leaky=True, pool=L['pool'], out_bf16=not last, out=self.acts[li])
-            x = self.acts[li]
+            moving = (self.store[bn['moving_mean']], self.store[bn['moving_variance']]) if self.update_moving else None
+            x = conv_bn_tc(x, self.packed[li], L['k'], L['cin'], L['cout'], bias=P['b'], gamma=P['gamma'], beta=P['beta'],
+                           moving=moving, stats=(s['mean'], s['var'], s['scale'], s['shift']), workspace=self.ws,
+                           pool=L['pool'], out_f32=li == nl - 1, out=self.acts[li], raw=self.raw[li])
         return self.acts[-1]
 
     def loss(self):

@@ -42,6 +42,25 @@ CORE_PLAN = [
     (3, 512, 1024, False),
 ]
 
+PASSTHROUGH_LAYER = 12            # CORE_PLAN index of the 26x26x512 layer (darknet.py:170); its UN-pooled output is the source
+PASSTHROUGH_FILTERS = 64
+
+
+def head_plan(output_filter, passthrough_filters=0):
+    """darknet.py:182-201, the detection head as (scope, ksize, cin, cout) in creation order: conv1..conv3 (3x3, 1024->1024)
+    and output (1x1 -> output_filter).  passthrough_filters > 0 adds the YOLOv2 passthrough branch (absent from the
+    reference, SURVEY Appendix A): a 1x1 conv (scope `passthrough`) on the un-pooled output of CORE_PLAN[PASSTHROUGH_LAYER],
+    whose space_to_depth(2) is concatenated after conv2's 1024 channels, so conv3 takes 1024 + 4 * passthrough_filters."""
+    plan = [('conv1', 3, 1024, 1024), ('conv2', 3, 1024, 1024)]
+    if passthrough_filters:
+        plan.append(('passthrough', 1, CORE_PLAN[PASSTHROUGH_LAYER][2], passthrough_filters))
+    return plan + [('conv3', 3, 1024 + 4 * passthrough_filters, 1024), ('output', 1, 1024, output_filter)]
+
+
+def classifier_plan(num_classes=1000):
+    """The 19th layer of the `darknet19` ImageNet classifier (darknet.py:61-123), as a CORE_PLAN entry: 1x1, 1024 -> classes."""
+    return (1, 1024, int(num_classes), False)
+
 
 def _device():
     return torch.device('cuda', torch.cuda.current_device())
@@ -57,31 +76,20 @@ def _as_param(store, name):
 
 
 # ---------------------------------------------------------------------------------------------
-# packed-weight / folded-BN caches (invalidated when the store changes)
+# packed-weight cache (invalidated when the store changes)
 # ---------------------------------------------------------------------------------------------
 _pack_cache = {}
 
 
-def _packed(store, wname):
-    key = (id(store), wname)
+def _packed(store, wname, split):
+    """pack_weights_bf16 of the variable, or pack_weights_bf16_split (bf16x3) with split=True."""
+    key = (id(store), wname, split)
     hit = _pack_cache.get(key)
     w = _as_param(store, wname)
     if hit is None or hit[0] != store.version or hit[1] != w.data_ptr():
-        hit = (store.version, w.data_ptr(), ops.pack_weights_bf16(w))
+        hit = (store.version, w.data_ptr(), (ops.pack_weights_bf16_split if split else ops.pack_weights_bf16)(w))
         _pack_cache[key] = hit
     return hit[2]
-
-
-_zeros_cache = {}
-
-
-def _zeros(c):
-    key = (c, torch.cuda.current_device())
-    z = _zeros_cache.get(key)
-    if z is None:
-        z = torch.zeros((c,), dtype=torch.float32, device=_device())
-        _zeros_cache[key] = z
-    return z
 
 
 # ---------------------------------------------------------------------------------------------
@@ -150,16 +158,6 @@ def conv_layer(x, filter_size, input_chl, output_chl, stride):
     return ops.conv_fwd_f32(_f32(x), W_conv, b_conv)
 
 
-def _packed_split(store, wname):
-    key = (id(store), wname, 'x3')
-    hit = _pack_cache.get(key)
-    w = _as_param(store, wname)
-    if hit is None or hit[0] != store.version or hit[1] != w.data_ptr():
-        hit = (store.version, w.data_ptr(), ops.pack_weights_bf16_split(w))
-        _pack_cache[key] = hit
-    return hit[2]
-
-
 def conv_bn_layer(x, filter_size, input_chl, output_chl, stride, is_training, _pool=False, _out_f32=None, _out=None,
                   _ldo=None, _col=0, _s2d=False):
     """darknet.py:39-46: conv + bias -> batch norm -> leaky(0.1).
@@ -180,6 +178,7 @@ def conv_bn_layer(x, filter_size, input_chl, output_chl, stride, is_training, _p
     gamma, beta = _as_param(store, bn['gamma']), _as_param(store, bn['beta'])
     mm, mv = _as_param(store, bn['moving_mean']), _as_param(store, bn['moving_variance'])
     training = bool(is_training)
+    moving = (mm, mv) if UPDATE_MOVING_AVERAGES else None
     N, H, Wd, _ = x.shape
     mode = cfg.COMPUTE
     if mode not in ('fp32', 'bf16', 'bf16x3'):
@@ -193,15 +192,13 @@ def conv_bn_layer(x, filter_size, input_chl, output_chl, stride, is_training, _p
     if mode == 'fp32' or (x3 and x.dtype == torch.float32 and input_chl == 3):
         h = ops.conv_fwd_f32(_f32(x), W, b)
         if training:
-            mean, var = ops.bn_stats(h.view(-1, output_chl), output_chl)
-            if UPDATE_MOVING_AVERAGES:
-                ops.bn_update_moving(mm, mv, mean, var)
-        else:
-            mean, var = mm, mv
-        scale, shift = ops.bn_fold(gamma, beta, _zeros(output_chl), var, None)      # shift == beta
+            mean, _, scale, shift = _batch_norm(h.view(-1, output_chl), output_chl, output_chl, gamma, beta, moving)
+        else:                                        # the centred form of _batch_norm, on the moving statistics
+            scale, _ = ops.bn_fold(gamma, beta, mm, mv)
+            mean, shift = mm, beta
         return ops.affine_leaky_pool(h, N, H, Wd, output_chl, sub=mean, scale=scale, shift=shift, leaky=True,
                                      pool=_pool, out_bf16=not out_f32, out=_out, ldo=_ldo, out_col=_col, space_to_depth=_s2d,
-                                     split_out=x3 and not out_f32)
+                                     split_out=x3)
     # ---- tensor-core path ----
     if x.dtype == torch.float32:
         if input_chl == 3:
@@ -214,29 +211,60 @@ def conv_bn_layer(x, filter_size, input_chl, output_chl, stride, is_training, _p
         xb = x
     if x3:
         assert xb.shape[-1] == 2 * input_chl, 'bf16x3: expected a [hi | lo] activation with %d channels' % (2 * input_chl)
-    wp = _packed_split(store, wname) if x3 else _packed(store, wname)
-    if not training:
-        scale, shift = ops.bn_fold(gamma, beta, mm, mv, b)          # bias folded: acc has no bias
-        if out_f32 or _s2d:
-            ld = (output_chl + 31) // 32 * 32
-            raw = ops.conv_fwd_bf16(xb, wp, filter_size, input_chl, output_chl, scale=scale, shift=shift, leaky=True,
-                                    pool=False, out_f32=True, ldy=ld, split_in=x3)
-            # compact the padded rows / pool / scatter them space-to-depth into the concat buffer
-            return ops.affine_leaky_pool(raw, N, H, Wd, output_chl, ldx=ld, leaky=False, pool=_pool, out_bf16=not out_f32,
-                                         out=_out, ldo=_ldo, out_col=_col, space_to_depth=_s2d)
-        return ops.conv_fwd_bf16(xb, wp, filter_size, input_chl, output_chl, scale=scale, shift=shift, leaky=True,
-                                 pool=_pool, out=_out, ldy=_ldo, out_col=_col, split_in=x3, split_out=x3)
-    # batch statistics: raw fp32 conv+bias, stats, then normalise + leaky (+ pool)
-    ld = (output_chl + 31) // 32 * 32
-    raw = ops.conv_fwd_bf16(xb, wp, filter_size, input_chl, output_chl, scale=None, shift=b, leaky=False, pool=False,
-                            out_f32=True, ldy=ld, split_in=x3)
-    mean, var = ops.bn_stats(raw, output_chl, ld=ld)
-    if UPDATE_MOVING_AVERAGES:
-        ops.bn_update_moving(mm, mv, mean, var)
-    scale, shift = ops.bn_fold(gamma, beta, _zeros(output_chl), var, None)
-    return ops.affine_leaky_pool(raw, N, H, Wd, output_chl, ldx=ld, sub=mean, scale=scale, shift=shift, leaky=True,
-                                 pool=_pool, out_bf16=not out_f32, out=_out, ldo=_ldo, out_col=_col, space_to_depth=_s2d,
-                                 split_out=x3 and not out_f32)
+    wp = _packed(store, wname, x3)
+    fold = None if training else ops.bn_fold(gamma, beta, mm, mv, b)          # inference: bias folded, acc has no bias
+    return conv_bn_tc(xb, wp, filter_size, input_chl, output_chl, fold=fold, bias=b, gamma=gamma, beta=beta, moving=moving,
+                      pool=_pool, out_f32=out_f32, out=_out, ldo=_ldo, col=_col, s2d=_s2d, x3=x3)
+
+
+def raw_ld(cout):
+    """Row stride of the float32 conv rows of conv_bn_tc: cout rounded up to 32 columns."""
+    return (cout + 31) // 32 * 32
+
+
+def _batch_norm(rows, cout, ld, gamma, beta, moving=None, stats=None, workspace=None):
+    """Batch statistics of the float32 conv rows [M, ld] and the affine of the centred form y = (x - mean) * scale + shift
+    (scale = gamma * rsqrt(var + eps), shift = beta), plus the moving-average update (UPDATE_OPS) of
+    moving=(moving_mean, moving_variance) when given: two launches either way.  Returns stats=(mean, var, scale, shift)."""
+    if stats is None:
+        stats = tuple(torch.empty((cout,), dtype=torch.float32, device=rows.device) for _ in range(4))
+    mean, var, scale, shift = stats
+    if moving is None:
+        ops.bn_stats_fold(rows, cout, gamma, beta, ld=ld, workspace=workspace, mean=mean, var=var, scale=scale, shift=shift)
+    else:
+        ops.bn_stats_fold_train(rows, cout, gamma, beta, *moving, ld=ld, workspace=workspace, mean=mean, var=var, scale=scale,
+                                shift=shift)
+    return stats
+
+
+def conv_bn_tc(x, wp, k, cin, cout, fold=None, bias=None, gamma=None, beta=None, moving=None, stats=None, workspace=None,
+               pool=False, out_f32=False, out=None, ldo=None, col=0, s2d=False, x3=False, raw=None):
+    """One conv + BN + leaky(0.1) (+ 2x2 max-pool) layer on the tensor cores: the kernels that conv_bn_layer, Yolo2Engine
+    and Yolo2Trainer issue for it.
+
+    x: bf16 [N,H,W,Cin_p] ([N,H,W,2*cin] = [hi | lo] with x3); wp: pack_weights_bf16 (pack_weights_bf16_split with x3).
+    BN: fold=(scale, shift) of bn_fold with the conv bias folded in (inference), or fold=None: batch statistics of conv +
+    `bias`, normalised with `gamma` / `beta` (see _batch_norm for `moving`, `stats` and `workspace`).
+    Output: bf16 [N,Ho,Wo,cout] ([hi | lo] with x3; float32 with out_f32) in `out`, or in channels [col, col + cout) of
+    the rows of stride ldo of `out`, stored space-to-depth(2) with s2d.  raw: the float32 [N*H*W, raw_ld(cout)] conv
+    rows, written unless BN, leaky and pool run in the conv epilogue.  Buffers left None are allocated.  Returns the output."""
+    N, H, W = x.shape[:3]
+    if fold is not None and not (out_f32 or s2d):
+        return ops.conv_fwd_bf16(x, wp, k, cin, cout, scale=fold[0], shift=fold[1], leaky=True, pool=pool, out=out, ldy=ldo,
+                                 out_col=col, split_in=x3, split_out=x3)
+    # float32 rows -- normalised (inference) or conv + bias (batch statistics) -- then one pass that normalises them (batch
+    # statistics), compacts the padded rows, pools and / or scatters them space-to-depth into `out`
+    ld = raw_ld(cout)
+    assert raw is None or tuple(raw.shape) == (N * H * W, ld)
+    batch = fold is None
+    scale, shift = (None, bias) if batch else fold
+    raw = ops.conv_fwd_bf16(x, wp, k, cin, cout, scale=scale, shift=shift, leaky=not batch, pool=False, out_f32=True, ldy=ld,
+                            out=raw, split_in=x3)
+    mean = scale = shift = None
+    if batch:
+        mean, _, scale, shift = _batch_norm(raw, cout, ld, gamma, beta, moving, stats, workspace)
+    return ops.affine_leaky_pool(raw, N, H, W, cout, ldx=ld, sub=mean, scale=scale, shift=shift, leaky=batch, pool=pool,
+                                 out_bf16=not out_f32, out=out, ldo=ldo, out_col=col, space_to_depth=s2d, split_out=x3)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -272,9 +300,6 @@ class _variable_scope:
 
     def __exit__(self, *exc):
         return self.ctx.__exit__(*exc)
-
-
-PASSTHROUGH_LAYER = 12            # CORE_PLAN index of the 26x26x512 layer (darknet.py:170)
 
 
 def space_to_depth(x, block_size=2):
@@ -315,9 +340,10 @@ def darknet19(inputs, num_classes=None, is_training=True, global_pool=True, outp
     with _variable_scope(scope, reuse=reuse):
         for (k, cin, cout, pool) in CORE_PLAN:
             net = conv_bn_layer(net, k, cin, cout, 1, is_training, _pool=pool)
-        net = conv_bn_layer(net, 1, 1024, 1000, 1, is_training, _out_f32=(cfg.COMPUTE == 'bf16x3'))
+        k, cin, cout, _ = classifier_plan()
+        net = conv_bn_layer(net, k, cin, cout, 1, is_training, _out_f32=(cfg.COMPUTE == 'bf16x3'))
         assert net.shape[1] == 7 and net.shape[2] == 7, 'darknet19 classifier expects a 224x224 input (darknet.py:116)'
-        logits = avg_pool(net, 7, 7).reshape(-1, 1000)
+        logits = avg_pool(net, 7, 7).reshape(-1, cout)
     return logits
 
 
@@ -331,28 +357,20 @@ def darknet19_detection(net, output_filter, is_training=True, scope='darknet19_d
     darknet19_core(return_passthrough=True).  It goes through a 1x1 conv_bn_layer (scope `passthrough`, 512 ->
     passthrough_filters), space_to_depth(2), and is concatenated after conv2's 1024 channels; conv3 then takes
     1024 + 4*passthrough_filters input channels."""
+    filters = 0 if passthrough is None else passthrough_filters
     with _variable_scope(scope, reuse=reuse):
-        with _variable_scope('conv1'):
-            net = conv_bn_layer(net, 3, 1024, 1024, 1, is_training)
-        cat = 1024
-        if passthrough is None:
-            with _variable_scope('conv2'):
-                net = conv_bn_layer(net, 3, 1024, 1024, 1, is_training)
-        else:
-            # conv2's 1024 channels and the reorganised passthrough's 4 * filters share ONE [N,S,S,cat] tensor: the concat
-            # and tf.space_to_depth are the two producers' store addresses (as in the batch engine), never a copy
-            N, S = int(net.shape[0]), int(net.shape[1])
-            cat = 1024 + 4 * passthrough_filters
-            fp32 = cfg.COMPUTE == 'fp32'
-            buf = torch.empty((N, S, S, cat), dtype=torch.float32 if fp32 else torch.bfloat16, device=net.device)
-            with _variable_scope('conv2'):
-                conv_bn_layer(net, 3, 1024, 1024, 1, is_training, _out=buf, _ldo=cat, _col=0)
-            with _variable_scope('passthrough'):
-                conv_bn_layer(passthrough, 1, int(passthrough.shape[-1]), passthrough_filters, 1, is_training, _out=buf,
-                              _ldo=cat, _col=1024, _s2d=True)
-            net = buf
-        with _variable_scope('conv3'):
-            net = conv_bn_layer(net, 3, cat, 1024, 1, is_training)
-        with _variable_scope('output'):
-            output = conv_bn_layer(net, 1, 1024, output_filter, 1, is_training, _out_f32=True)
-    return output
+        for sc, k, cin, cout in head_plan(output_filter, filters):
+            with _variable_scope(sc):
+                if sc == 'conv2' and filters:
+                    # conv2's 1024 channels and the reorganised passthrough's 4 * filters share ONE [N,S,S,cat] tensor: the
+                    # concat and tf.space_to_depth are the two producers' store addresses (as in the batch engine), never a copy
+                    N, S, cat = int(net.shape[0]), int(net.shape[1]), cout + 4 * filters
+                    buf = torch.empty((N, S, S, cat), dtype=torch.float32 if cfg.COMPUTE == 'fp32' else torch.bfloat16,
+                                      device=net.device)
+                    conv_bn_layer(net, k, cin, cout, 1, is_training, _out=buf, _ldo=cat)
+                    net = buf
+                elif sc == 'passthrough':
+                    conv_bn_layer(passthrough, k, cin, cout, 1, is_training, _out=net, _ldo=cat, _col=1024, _s2d=True)
+                else:
+                    net = conv_bn_layer(net, k, cin, cout, 1, is_training, _out_f32=sc == 'output')
+    return net

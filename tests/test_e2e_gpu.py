@@ -66,10 +66,14 @@ def test_builders_fp32_vs_oracle_tame_416(fresh, golden_dir):
 
 
 # ---- tensor-core path vs the oracle with bf16 operand rounding at the same points --------------
-@pytest.mark.parametrize('tame', [True, False])
-def test_builders_bf16_vs_oracle(fresh, tame):
+@pytest.mark.parametrize('tame,update_moving', [pytest.param(True, False, id='True'), pytest.param(False, False, id='False'),
+                                                pytest.param(True, True, id='True-update_moving')])
+def test_builders_bf16_vs_oracle(fresh, monkeypatch, tame, update_moving):
+    from tensorflow_yolo2_b200 import ops
+    from tensorflow_yolo2_b200.yolo2_nets import darknet
     from tensorflow_yolo2_b200.yolo2_nets.darknet import darknet19_core, darknet19_detection
     fresh.COMPUTE = 'bf16'
+    monkeypatch.setattr(darknet, 'UPDATE_MOVING_AVERAGES', update_moving)
     st, layers = make_store(125, tame=tame)
     core_p, head_p = oracle_params(st, layers)
     _install(st)
@@ -87,6 +91,25 @@ def test_builders_bf16_vs_oracle(fresh, tame):
     # see DESIGN.md "Numerics".
     assert e_core < 1.5e-2
     assert e_out < 5e-2
+    if update_moving:
+        # the head's UPDATE_OPS: conv1's moving statistics against bn_update_moving of bn_stats of the same float32 conv +
+        # bias rows.  The mean is bit-exact.  bn_stats_fold_train's kernel puts the other product of
+        # mv * momentum + var * (1 - momentum) into the FMA, so the variance may differ by its two float32 roundings (both
+        # terms are >= 0, no cancellation): at most 2 ulp
+        L, p = layers[len(darknet.CORE_PLAN)], head_p[0]
+        rows = ops.conv_fwd_bf16(core, ops.pack_weights_bf16(st[L['W']]), L['k'], L['cin'], L['cout'], shift=st[L['b']],
+                                 leaky=False, out_f32=True)
+        mean, var = ops.bn_stats(rows, L['cout'])
+        mm, mv = p['mm'].cuda(), p['mv'].cuda()                  # the values before the pass
+        ops.bn_update_moving(mm, mv, mean, var)
+        got_mm, got_mv = st[L['bn']['moving_mean']], st[L['bn']['moving_variance']]
+        assert not torch.equal(mm, p['mm'].cuda())
+        assert torch.equal(got_mm, mm)
+        ulp = torch.nextafter(mv, torch.full_like(mv, float('inf'))) - mv
+        worst = ((got_mv - mv).abs() / ulp).max().item()
+        print('moving variance vs bn_update_moving: %d of %d differ, at most %g ulp' % ((got_mv != mv).sum().item(), mv.numel(),
+                                                                                        worst))
+        assert worst <= 2
 
 
 # ---- darknet19 ImageNet classifier (darknet.py:61-123): core + 1x1 -> 1000 + 7x7 average pool -----------------------
