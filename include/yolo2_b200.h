@@ -278,6 +278,22 @@ int y2_bn_leaky_pool_bwd(const float* h_raw, int ldh, const void* dy, int dy_dty
                          const float* gamma, const float* beta, float eps, float alpha, int leaky, int pool, int N,
                          int H, int W, int C, float* dgamma, float* dbeta, void* dh_bf16, int ld_dh, void* workspace,
                          size_t workspace_bytes, y2_stream_t stream);
+/* y2_bn_leaky_pool_bwd_ex: the same, with three ways to read dy (y2_bn_leaky_pool_bwd is this call with ldy = C,
+ * dy_s2d = 0, dy_add = NULL, and gives the same bits):
+ *   ldy     row stride of dy (>= C; >= 4C with dy_s2d); dy points at the layer's first column, so a channel slice of a
+ *           wider gradient (conv2's 1024 columns of the [N,S,S,1280] concat gradient of the YOLOv2 passthrough graph) is
+ *           read in place.
+ *   dy_s2d  (un-pooled layers, H and W even) the layer's output was stored space_to_depth(2) into rows of stride ldy:
+ *           pixel (h, w), channel c is read from row (h/2, w/2), column ((h%2)*2 + w%2)*C + c -- depth_to_space of the
+ *           concat gradient, for the passthrough conv.
+ *   dy_add  (pooled layers; NULL = none) bf16 [N,H,W,C]: the gradient of the UN-pooled output from a second consumer
+ *           (the passthrough branch reads layer 13 before its pool).  Every input row gets its dy_add value, the window's
+ *           first maximum also gets the pooled dy; the float32 sum takes that row's leaky slope. */
+int y2_bn_leaky_pool_bwd_ex(const float* h_raw, int ldh, const void* dy, int dy_dtype, int ldy, int dy_s2d,
+                            const void* dy_add, const float* mean, const float* var, const float* gamma, const float* beta,
+                            float eps, float alpha, int leaky, int pool, int N, int H, int W, int C, float* dgamma,
+                            float* dbeta, void* dh_bf16, int ld_dh, void* workspace, size_t workspace_bytes,
+                            y2_stream_t stream);
 /* Data gradient = the forward convolution of dh with the weights transposed (Cin <-> Cout) and flipped spatially:
  * pack them with this, then call y2_conv_fwd_bf16 with Cin := ld_dh, Cout := Cin, no scale/shift/leaky. */
 size_t y2_conv_packed_weight_dgrad_elems(int ksize, int Cin, int ld_dh);

@@ -73,6 +73,8 @@ _SIGNATURES = {
     'y2_bn_bwd_workspace_bytes': (_sz, [_i, _i]),
     'y2_bn_leaky_pool_bwd': (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _f, _f, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i,
                                   _vp, _sz, _vp]),
+    'y2_bn_leaky_pool_bwd_ex': (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _i, _i, _i, _i, _i, _i, _vp, _vp,
+                                     _vp, _i, _vp, _sz, _vp]),
     'y2_conv_packed_weight_dgrad_elems': (_sz, [_i, _i, _i]),
     'y2_pack_weights_dgrad_bf16': (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
     'y2_conv_wgrad_bf16': (_i, [_vp, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),

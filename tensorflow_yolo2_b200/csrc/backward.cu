@@ -8,6 +8,9 @@
 //                               dh      = gamma*inv_std * (dz - dbeta/M - xhat * dgamma/M)        -> bf16 [M, ld_dh]
 //                            z / xhat / the pooling arg-max are recomputed from the saved fp32 pre-BN rows, so the
 //                            forward stores nothing extra.  Two passes over h (reduce in fp64, then apply).
+//   y2_bn_leaky_pool_bwd_ex  the same, with dy read as a channel slice of wider rows (row stride ldy), through the inverse
+//                            of a space_to_depth(2) store, and / or with an un-pooled addend (a pooled layer whose output
+//                            also feeds a second consumer un-pooled): the YOLOv2 passthrough branch's gradients.
 //   y2_pack_weights_dgrad_bf16   weights packed transposed + spatially flipped: the data gradient of a SAME stride-1
 //                            convolution is the same convolution of dh with those weights, so dgrad runs on
 //                            conv_tc_kernel (conv_tcgen05.cu) unchanged.
@@ -42,8 +45,32 @@ __device__ __forceinline__ float load_dy(const void* dy, int dy_f32, size_t i) {
   return dy_f32 ? reinterpret_cast<const float*>(dy)[i] : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(dy)[i]);
 }
 
+// Where the gradient of output unit u (a pixel of the [N,Hu,Wu] map dy is given on) is read, channel c at + c.  The pointer is
+// pre-offset to the layer's first column.
+//   DY_DENSE  rows of stride C (the layer's own [N,Hu,Wu,C] gradient)
+//   DY_ROWS   rows of stride ldy (a channel slice of a wider gradient: conv2's 1024 columns of the [N,S,S,1280] concat)
+//   DY_S2D    depth-to-space: the layer's output was stored space_to_depth(2) into rows of stride ldy (the passthrough
+//             branch), so pixel (h, w) reads row (h/2, w/2), column ((h%2)*2 + w%2)*C + c -- the inverse of the store
+//             address of affine_leaky_pool_kernel's s2d mode (elementwise.cu)
+enum { DY_DENSE = 0, DY_ROWS = 1, DY_S2D = 2 };
+
+template <int DYM>
+__device__ __forceinline__ size_t dy_row(size_t u, int ldy, int Hu, int Wu, int C) {      // offset of (unit u, channel 0)
+  if (DYM == DY_DENSE) return u * C;
+  if (DYM == DY_ROWS) return u * ldy;
+  const int w = (int)(u % Wu);
+  const size_t t = u / Wu;
+  const int h = (int)(t % Hu);
+  const size_t n = t / Hu;
+  return ((n * (Hu >> 1) + (h >> 1)) * (size_t)(Wu >> 1) + (w >> 1)) * ldy + (size_t)(((h & 1) * 2 + (w & 1)) * C);
+}
+
 // pass 1: grid (ceil(C/32), splits), block (32, 8).  part[split][c][2] = (sum dz, sum dz*xhat)
-__global__ void bn_bwd_reduce_kernel(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32,
+// ADD: dy_add (bf16 [N,H,W,C], one value per input row) is added to every row's gradient in front of the leaky slope; the
+// pooled dy still goes to the window's first maximum only.
+template <int DYM, bool ADD>
+__device__ __forceinline__ void bn_bwd_reduce_body(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+                                     const __nv_bfloat16* __restrict__ dy_add,
                                      const float* __restrict__ mean, const float* __restrict__ var,
                                      const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
                                      float alpha, int leaky_on, int pool, int H, int W, int C, size_t units,
@@ -59,17 +86,35 @@ __global__ void bn_bwd_reduce_kernel(const float* __restrict__ h, int ldh, const
     int cnt = 0;
     for (size_t u = u0 + threadIdx.y; u < u1; u += 8) {
       const UnitRows ur = unit_rows(u, H, W, pool != 0);
-      float best = -INFINITY, bx = 0.0f, bz = 0.0f;
-      for (int k = 0; k < ur.n; ++k) {
-        const float xh = (h[ur.r[k] * ldh + c] - mu) * inv;
-        const float z = xh * g + b;
-        const float a = leaky_on ? fmaxf(z, alpha * z) : z;
-        if (a > best) { best = a; bx = xh; bz = z; }
+      if constexpr (ADD) {
+        float xs[4], zs[4], best = -INFINITY;
+        int arg = 0;
+        for (int k = 0; k < ur.n; ++k) {
+          xs[k] = (h[ur.r[k] * ldh + c] - mu) * inv;
+          zs[k] = xs[k] * g + b;
+          const float a = leaky_on ? fmaxf(zs[k], alpha * zs[k]) : zs[k];
+          if (a > best) { best = a; arg = k; }
+        }
+        const float dp = load_dy(dy, dy_f32, dy_row<DYM>(u, ldy, pool ? H >> 1 : H, pool ? W >> 1 : W, C) + c);
+        for (int k = 0; k < ur.n; ++k) {
+          float d = __bfloat162float(dy_add[ur.r[k] * C + c]) + (k == arg ? dp : 0.0f);
+          if (leaky_on && !(zs[k] > 0.0f)) d *= alpha;
+          f1 += d;
+          f2 += d * xs[k];
+        }
+      } else {
+        float best = -INFINITY, bx = 0.0f, bz = 0.0f;
+        for (int k = 0; k < ur.n; ++k) {
+          const float xh = (h[ur.r[k] * ldh + c] - mu) * inv;
+          const float z = xh * g + b;
+          const float a = leaky_on ? fmaxf(z, alpha * z) : z;
+          if (a > best) { best = a; bx = xh; bz = z; }
+        }
+        float d = load_dy(dy, dy_f32, dy_row<DYM>(u, ldy, pool ? H >> 1 : H, pool ? W >> 1 : W, C) + c);
+        if (leaky_on && !(bz > 0.0f)) d *= alpha;
+        f1 += d;
+        f2 += d * bx;
       }
-      float d = load_dy(dy, dy_f32, u * C + c);
-      if (leaky_on && !(bz > 0.0f)) d *= alpha;
-      f1 += d;
-      f2 += d * bx;
       if (++cnt == 64) { a1 += (double)f1; a2 += (double)f2; f1 = f2 = 0.0f; cnt = 0; }
     }
     a1 += (double)f1;
@@ -84,17 +129,37 @@ __global__ void bn_bwd_reduce_kernel(const float* __restrict__ h, int ldh, const
     part[((size_t)blockIdx.y * C + c) * 2 + 1] = a2;
   }
 }
+__global__ void bn_bwd_reduce_kernel(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32,
+                                     const float* __restrict__ mean, const float* __restrict__ var,
+                                     const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
+                                     float alpha, int leaky_on, int pool, int H, int W, int C, size_t units,
+                                     size_t units_per_split, double* __restrict__ part) {
+  bn_bwd_reduce_body<DY_DENSE, false>(h, ldh, dy, dy_f32, C, nullptr, mean, var, gamma, beta, eps, alpha, leaky_on, pool, H, W,
+                                      C, units, units_per_split, part);
+}
+template <int DYM, bool ADD>
+__global__ void bn_bwd_reduce_ex_kernel(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+                                        const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean,
+                                        const float* __restrict__ var, const float* __restrict__ gamma,
+                                        const float* __restrict__ beta, float eps, float alpha, int leaky_on, int pool, int H,
+                                        int W, int C, size_t units, size_t units_per_split, double* __restrict__ part) {
+  bn_bwd_reduce_body<DYM, ADD>(h, ldh, dy, dy_f32, ldy, dy_add, mean, var, gamma, beta, eps, alpha, leaky_on, pool, H, W, C,
+                               units, units_per_split, part);
+}
 
 // Vectorised pass 1 (C % 4 == 0): a thread owns 4 channels (16-byte loads of h, 8-byte loads of bf16 dy) and keeps
 // UNR units in flight; block = TX channel groups x (256/TX) unit lanes.  Four blocks resident per SM.
-template <bool POOL, int TX>
-__global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
-    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, const float* __restrict__ mean,
+// DYM / ADD: the dy read of bn_bwd_reduce_kernel.
+template <bool POOL, int TX, int DYM, bool ADD>
+__device__ __forceinline__ void bn_bwd_reduce_v4_body(
+    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+    const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean,
     const float* __restrict__ var, const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float alpha,
     int leaky_on, int H, int W, int C, size_t units, size_t units_per_split, double* __restrict__ part) {
   constexpr int TY = 256 / TX;
   constexpr int NR = POOL ? 4 : 1;
   constexpr int UNR = POOL ? 2 : 4;
+  constexpr int NA = ADD ? NR : 1;
   __shared__ double sm[TY][TX][8];
   const int tx = threadIdx.x % TX, ty = threadIdx.x / TX;
   const int c0 = (blockIdx.x * TX + tx) * 4;
@@ -113,6 +178,7 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
     for (size_t ub = (size_t)blockIdx.y * UNR * TY + ty; ub < u1; ub += (size_t)gridDim.y * UNR * TY) {
       float4 hv[UNR][NR];
       float dv[UNR][4];
+      uint2 av[UNR][NA];                                             // (ADD) bf16 addend of each input row
 #pragma unroll
       for (int j = 0; j < UNR; ++j) {
         const size_t u = ub + (size_t)j * TY;
@@ -120,11 +186,17 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
           const UnitRows ur = unit_rows(u, H, W, POOL);
 #pragma unroll
           for (int k = 0; k < NR; ++k) hv[j][k] = __ldg(reinterpret_cast<const float4*>(h + ur.r[k] * ldh + c0));   // (re-read by the apply pass)
+          if constexpr (ADD) {
+#pragma unroll
+            for (int k = 0; k < NR; ++k) av[j][k] = __ldg(reinterpret_cast<const uint2*>(dy_add + ur.r[k] * C + c0));
+          }
           if (dy_f32) {
-            const float4 q = __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(dy) + u * C + c0));
+            const float4 q = __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(dy) +
+                                                                   dy_row<DYM>(u, ldy, POOL ? H >> 1 : H, POOL ? W >> 1 : W, C) + c0));
             dv[j][0] = q.x; dv[j][1] = q.y; dv[j][2] = q.z; dv[j][3] = q.w;
           } else {
-            const uint2 q = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const __nv_bfloat16*>(dy) + u * C + c0));
+            const uint2 q = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const __nv_bfloat16*>(dy) +
+                                                                 dy_row<DYM>(u, ldy, POOL ? H >> 1 : H, POOL ? W >> 1 : W, C) + c0));
             const __nv_bfloat162 lo = *reinterpret_cast<const __nv_bfloat162*>(&q.x), hi = *reinterpret_cast<const __nv_bfloat162*>(&q.y);
             dv[j][0] = __low2float(lo); dv[j][1] = __high2float(lo); dv[j][2] = __low2float(hi); dv[j][3] = __high2float(hi);
           }
@@ -132,25 +204,52 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
 #pragma unroll
           for (int k = 0; k < NR; ++k) hv[j][k] = make_float4(0.f, 0.f, 0.f, 0.f);
           dv[j][0] = dv[j][1] = dv[j][2] = dv[j][3] = 0.0f;          // contributes nothing
+          if constexpr (ADD) {
+#pragma unroll
+            for (int k = 0; k < NR; ++k) av[j][k] = make_uint2(0u, 0u);
+          }
         }
       }
 #pragma unroll
       for (int j = 0; j < UNR; ++j) {
 #pragma unroll
         for (int v = 0; v < 4; ++v) {
-          float best = -INFINITY, bx = 0.0f, bz = 0.0f;
+          if constexpr (ADD) {
+            // every input row of the window has a gradient: the addend, plus the pooled dy at the first maximum; the sum
+            // (float32) takes the row's own leaky slope
+            float xs[NR], zs[NR], best = -INFINITY;
+            int arg = 0;
 #pragma unroll
-          for (int k = 0; k < NR; ++k) {
-            const float t = v == 0 ? hv[j][k].x : (v == 1 ? hv[j][k].y : (v == 2 ? hv[j][k].z : hv[j][k].w));
-            const float xh = (t - pm[v]) * pi[v];
-            const float z = xh * pg[v] + pb[v];
-            const float a = leaky_on ? fmaxf(z, alpha * z) : z;
-            if (a > best) { best = a; bx = xh; bz = z; }
+            for (int k = 0; k < NR; ++k) {
+              const float t = v == 0 ? hv[j][k].x : (v == 1 ? hv[j][k].y : (v == 2 ? hv[j][k].z : hv[j][k].w));
+              xs[k] = (t - pm[v]) * pi[v];
+              zs[k] = xs[k] * pg[v] + pb[v];
+              const float a = leaky_on ? fmaxf(zs[k], alpha * zs[k]) : zs[k];
+              if (a > best) { best = a; arg = k; }
+            }
+#pragma unroll
+            for (int k = 0; k < NR; ++k) {
+              const __nv_bfloat162 p = *reinterpret_cast<const __nv_bfloat162*>(v < 2 ? &av[j][k].x : &av[j][k].y);
+              float d = ((v & 1) ? __high2float(p) : __low2float(p)) + (arg == k ? dv[j][v] : 0.0f);
+              if (leaky_on && !(zs[k] > 0.0f)) d *= alpha;
+              f[v] += d;
+              f[4 + v] = fmaf(d, xs[k], f[4 + v]);
+            }
+          } else {
+            float best = -INFINITY, bx = 0.0f, bz = 0.0f;
+#pragma unroll
+            for (int k = 0; k < NR; ++k) {
+              const float t = v == 0 ? hv[j][k].x : (v == 1 ? hv[j][k].y : (v == 2 ? hv[j][k].z : hv[j][k].w));
+              const float xh = (t - pm[v]) * pi[v];
+              const float z = xh * pg[v] + pb[v];
+              const float a = leaky_on ? fmaxf(z, alpha * z) : z;
+              if (a > best) { best = a; bx = xh; bz = z; }
+            }
+            float d = dv[j][v];
+            if (leaky_on && !(bz > 0.0f)) d *= alpha;
+            f[v] += d;
+            f[4 + v] = fmaf(d, bx, f[4 + v]);
           }
-          float d = dv[j][v];
-          if (leaky_on && !(bz > 0.0f)) d *= alpha;
-          f[v] += d;
-          f[4 + v] = fmaf(d, bx, f[4 + v]);
         }
       }
       if (++cnt == 8) {
@@ -170,6 +269,23 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
     for (int y = 0; y < TY; ++y) a += sm[y][tx][ty];
     part[((size_t)blockIdx.y * C + c0 + (ty & 3)) * 2 + (ty >> 2)] = a;
   }
+}
+template <bool POOL, int TX>
+__global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_kernel(
+    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, const float* __restrict__ mean,
+    const float* __restrict__ var, const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float alpha,
+    int leaky_on, int H, int W, int C, size_t units, size_t units_per_split, double* __restrict__ part) {
+  bn_bwd_reduce_v4_body<POOL, TX, DY_DENSE, false>(h, ldh, dy, dy_f32, C, nullptr, mean, var, gamma, beta, eps, alpha, leaky_on,
+                                                   H, W, C, units, units_per_split, part);
+}
+template <bool POOL, int TX, int DYM, bool ADD>
+__global__ void __launch_bounds__(256, 4) bn_bwd_reduce_v4_ex_kernel(
+    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+    const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean, const float* __restrict__ var,
+    const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float alpha, int leaky_on, int H, int W, int C,
+    size_t units, size_t units_per_split, double* __restrict__ part) {
+  bn_bwd_reduce_v4_body<POOL, TX, DYM, ADD>(h, ldh, dy, dy_f32, ldy, dy_add, mean, var, gamma, beta, eps, alpha, leaky_on, H, W,
+                                            C, units, units_per_split, part);
 }
 
 constexpr int BWD_FIN_TY = 32;   // thread rows folding the splits (8 rows walked up to 128 dependent L2 round trips: 22 us per layer)
@@ -209,9 +325,11 @@ __global__ void __launch_bounds__(32 * BWD_FIN_TY) bn_bwd_final_kernel(const dou
 // registers -- and walks units; 32-bit index arithmetic, 16-byte loads of the pre-BN rows, one 8/16-byte load of dy.
 // The generic kernel below spent 3.5 ms of a 17.4 ms training step (ncu launch list) on 64-bit div/mod per element,
 // scalar bf16 dy loads and six constant loads + two rsqrt per channel per element.
-template <bool POOL>
-__global__ void __launch_bounds__(256, 4) bn_bwd_apply_rows_kernel(
-    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, const float* __restrict__ mean,
+// DYM / ADD: the dy read of bn_bwd_reduce_kernel.
+template <bool POOL, int DYM, bool ADD>
+__device__ __forceinline__ void bn_bwd_apply_rows_body(
+    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+    const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean,
     const float* __restrict__ var, const float* __restrict__ gamma, const float* __restrict__ beta,
     const float* __restrict__ dgamma, const float* __restrict__ dbeta, float eps, float alpha, int leaky_on, int H, int W, int C,
     unsigned units, float invM, __nv_bfloat16* __restrict__ dh, int ld_dh) {
@@ -248,10 +366,12 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_apply_rows_kernel(
     float d[4] = {0.0f, 0.0f, 0.0f, 0.0f};
     if (real) {
       if (dy_f32) {
-        const float4 g = __ldcs(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(dy) + (size_t)u * C + c0));
+        const float4 g = __ldcs(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(dy) +
+                                                                dy_row<DYM>(u, ldy, (int)Ho, (int)Wo, C) + c0));
         d[0] = g.x; d[1] = g.y; d[2] = g.z; d[3] = g.w;
       } else {
-        const uint2 g = __ldcs(reinterpret_cast<const uint2*>(reinterpret_cast<const __nv_bfloat16*>(dy) + (size_t)u * C + c0));
+        const uint2 g = __ldcs(reinterpret_cast<const uint2*>(reinterpret_cast<const __nv_bfloat16*>(dy) +
+                                                              dy_row<DYM>(u, ldy, (int)Ho, (int)Wo, C) + c0));
         const __nv_bfloat162 g0 = *reinterpret_cast<const __nv_bfloat162*>(&g.x), g1 = *reinterpret_cast<const __nv_bfloat162*>(&g.y);
         d[0] = __low2float(g0); d[1] = __high2float(g0); d[2] = __low2float(g1); d[3] = __high2float(g1);
       }
@@ -259,6 +379,7 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_apply_rows_kernel(
     float xh[NP][4];
     int arg[4] = {0, 0, 0, 0};
     float abest[4], zbest[4];
+    float zs[ADD ? NP : 1][4];                                      // (ADD) every row's z: each row takes its own slope
 #pragma unroll
     for (int v = 0; v < 4; ++v) { abest[v] = -INFINITY; zbest[v] = 0.0f; }
 #pragma unroll
@@ -270,30 +391,76 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_apply_rows_kernel(
         const float z = x_ * ga[v] + be[v];
         const float a = leaky_on ? fmaxf(z, alpha * z) : z;
         xh[k][v] = x_;
+        if constexpr (ADD) zs[k][v] = z;
         if (a > abest[v]) { abest[v] = a; arg[v] = k; zbest[v] = z; }      // first maximum wins, as in the generic kernel
       }
     }
+    if constexpr (ADD) {
+      // every row's gradient: the addend, plus the pooled dy at the first maximum; the float32 sum takes the row's slope
 #pragma unroll
-    for (int v = 0; v < 4; ++v)
-      if (leaky_on && !(zbest[v] > 0.0f)) d[v] *= alpha;
+      for (int k = 0; k < NP; ++k) {
+        float a4[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+        if (real) {
+          const uint2 g = __ldcs(reinterpret_cast<const uint2*>(dy_add + rows[k] * C + c0));
+          const __nv_bfloat162 g0 = *reinterpret_cast<const __nv_bfloat162*>(&g.x), g1 = *reinterpret_cast<const __nv_bfloat162*>(&g.y);
+          a4[0] = __low2float(g0); a4[1] = __high2float(g0); a4[2] = __low2float(g1); a4[3] = __high2float(g1);
+        }
+        float o[4];
 #pragma unroll
-    for (int k = 0; k < NP; ++k) {
-      float o[4];
+        for (int v = 0; v < 4; ++v) {
+          float dk = a4[v] + (arg[v] == k ? d[v] : 0.0f);
+          if (leaky_on && !(zs[k][v] > 0.0f)) dk *= alpha;
+          o[v] = gi[v] * (dk - m1[v] - xh[k][v] * m2[v]);
+        }
+        const __nv_bfloat162 a = __floats2bfloat162_rn(o[0], o[1]), b = __floats2bfloat162_rn(o[2], o[3]);
+        uint2 pk;
+        pk.x = *reinterpret_cast<const uint32_t*>(&a);
+        pk.y = *reinterpret_cast<const uint32_t*>(&b);
+        *reinterpret_cast<uint2*>(dh + rows[k] * ld_dh + c0) = pk;
+      }
+    } else {
 #pragma unroll
-      for (int v = 0; v < 4; ++v) o[v] = gi[v] * ((arg[v] == k ? d[v] : 0.0f) - m1[v] - xh[k][v] * m2[v]);
-      const __nv_bfloat162 a = __floats2bfloat162_rn(o[0], o[1]), b = __floats2bfloat162_rn(o[2], o[3]);
-      uint2 pk;
-      pk.x = *reinterpret_cast<const uint32_t*>(&a);
-      pk.y = *reinterpret_cast<const uint32_t*>(&b);
-      *reinterpret_cast<uint2*>(dh + rows[k] * ld_dh + c0) = pk;
+      for (int v = 0; v < 4; ++v)
+        if (leaky_on && !(zbest[v] > 0.0f)) d[v] *= alpha;
+#pragma unroll
+      for (int k = 0; k < NP; ++k) {
+        float o[4];
+#pragma unroll
+        for (int v = 0; v < 4; ++v) o[v] = gi[v] * ((arg[v] == k ? d[v] : 0.0f) - m1[v] - xh[k][v] * m2[v]);
+        const __nv_bfloat162 a = __floats2bfloat162_rn(o[0], o[1]), b = __floats2bfloat162_rn(o[2], o[3]);
+        uint2 pk;
+        pk.x = *reinterpret_cast<const uint32_t*>(&a);
+        pk.y = *reinterpret_cast<const uint32_t*>(&b);
+        *reinterpret_cast<uint2*>(dh + rows[k] * ld_dh + c0) = pk;
+      }
     }
   }
 }
+template <bool POOL>
+__global__ void __launch_bounds__(256, 4) bn_bwd_apply_rows_kernel(
+    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, const float* __restrict__ mean,
+    const float* __restrict__ var, const float* __restrict__ gamma, const float* __restrict__ beta,
+    const float* __restrict__ dgamma, const float* __restrict__ dbeta, float eps, float alpha, int leaky_on, int H, int W, int C,
+    unsigned units, float invM, __nv_bfloat16* __restrict__ dh, int ld_dh) {
+  bn_bwd_apply_rows_body<POOL, DY_DENSE, false>(h, ldh, dy, dy_f32, C, nullptr, mean, var, gamma, beta, dgamma, dbeta, eps, alpha,
+                                                leaky_on, H, W, C, units, invM, dh, ld_dh);
+}
+template <bool POOL, int DYM, bool ADD>
+__global__ void __launch_bounds__(256, 4) bn_bwd_apply_rows_ex_kernel(
+    const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+    const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean, const float* __restrict__ var,
+    const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ dgamma,
+    const float* __restrict__ dbeta, float eps, float alpha, int leaky_on, int H, int W, int C, unsigned units, float invM,
+    __nv_bfloat16* __restrict__ dh, int ld_dh) {
+  bn_bwd_apply_rows_body<POOL, DYM, ADD>(h, ldh, dy, dy_f32, ldy, dy_add, mean, var, gamma, beta, dgamma, dbeta, eps, alpha,
+                                         leaky_on, H, W, C, units, invM, dh, ld_dh);
+}
 
 // pass 2: one thread per (unit, VEC channels); writes dh for every input pixel of the unit.
-template <int VEC>
-__global__ void bn_bwd_apply_kernel(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32,
-                                    const float* __restrict__ mean, const float* __restrict__ var,
+// DYM / ADD: the dy read of bn_bwd_reduce_kernel.
+template <int VEC, int DYM, bool ADD>
+__device__ __forceinline__ void bn_bwd_apply_body(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+                                    const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean, const float* __restrict__ var,
                                     const float* __restrict__ gamma, const float* __restrict__ beta,
                                     const float* __restrict__ dgamma, const float* __restrict__ dbeta, float eps,
                                     float alpha, int leaky_on, int pool, int H, int W, int C, size_t units, float invM,
@@ -308,6 +475,7 @@ __global__ void bn_bwd_apply_kernel(const float* __restrict__ h, int ldh, const 
     const int c0 = cv * VEC;
     const UnitRows ur = unit_rows(u, H, W, pool != 0);
     float xh[4][VEC];
+    float zs[ADD ? 4 : 1][VEC];                      // (ADD) every row's z: each row takes its own slope
     int arg[VEC];
     float zbest[VEC], abest[VEC];
 #pragma unroll
@@ -330,45 +498,89 @@ __global__ void bn_bwd_apply_kernel(const float* __restrict__ h, int ldh, const 
           const float z = x_ * gamma[c] + beta[c];
           const float a = leaky_on ? fmaxf(z, alpha * z) : z;
           xh[k][v] = x_;
+          if constexpr (ADD) zs[k][v] = z;
           if (a > abest[v]) { abest[v] = a; arg[v] = k; zbest[v] = z; }
         } else {
           xh[k][v] = 0.0f;
+          if constexpr (ADD) zs[k][v] = 0.0f;
         }
       }
     }
     float d[VEC], gi[VEC], m1[VEC], m2[VEC];
+    if constexpr (ADD) {
+      // every row's gradient: the addend, plus the pooled dy at the first maximum; the float32 sum takes the row's slope
 #pragma unroll
-    for (int v = 0; v < VEC; ++v) {
-      const int c = c0 + v;
-      if (c < C) {
-        float g = load_dy(dy, dy_f32, u * C + c);
-        if (leaky_on && !(zbest[v] > 0.0f)) g *= alpha;
-        d[v] = g;
-        gi[v] = gamma[c] * rsqrtf(var[c] + eps);
-        m1[v] = dbeta[c] * invM;
-        m2[v] = dgamma[c] * invM;
-      } else {
-        d[v] = 0.0f; gi[v] = 0.0f; m1[v] = 0.0f; m2[v] = 0.0f;
+      for (int v = 0; v < VEC; ++v) {
+        const int c = c0 + v;
+        d[v] = c < C ? load_dy(dy, dy_f32, dy_row<DYM>(u, ldy, pool ? H >> 1 : H, pool ? W >> 1 : W, C) + c) : 0.0f;
+        gi[v] = c < C ? gamma[c] * rsqrtf(var[c] + eps) : 0.0f;
+        m1[v] = c < C ? dbeta[c] * invM : 0.0f;
+        m2[v] = c < C ? dgamma[c] * invM : 0.0f;
       }
-    }
-    for (int k = 0; k < ur.n; ++k) {
-      float o[VEC];
+      for (int k = 0; k < ur.n; ++k) {
+        __nv_bfloat16* po = dh + ur.r[k] * ld_dh + c0;
 #pragma unroll
-      for (int v = 0; v < VEC; ++v) o[v] = gi[v] * ((arg[v] == k ? d[v] : 0.0f) - m1[v] - xh[k][v] * m2[v]);
-      __nv_bfloat16* po = dh + ur.r[k] * ld_dh + c0;
-      if (VEC == 4) {
-        __nv_bfloat162 a = __floats2bfloat162_rn(o[0], o[1 % VEC]);
-        __nv_bfloat162 b = __floats2bfloat162_rn(o[2 % VEC], o[3 % VEC]);
-        uint2 pk;
-        pk.x = *reinterpret_cast<uint32_t*>(&a);
-        pk.y = *reinterpret_cast<uint32_t*>(&b);
-        *reinterpret_cast<uint2*>(po) = pk;
-      } else {
+        for (int v = 0; v < VEC; ++v) {
+          const int c = c0 + v;
+          float dk = c < C ? __bfloat162float(dy_add[ur.r[k] * C + c]) + (arg[v] == k ? d[v] : 0.0f) : 0.0f;
+          if (leaky_on && !(zs[k][v] > 0.0f)) dk *= alpha;
+          po[v] = __float2bfloat16_rn(gi[v] * (dk - m1[v] - xh[k][v] * m2[v]));
+        }
+      }
+    } else {
 #pragma unroll
-        for (int v = 0; v < VEC; ++v) po[v] = __float2bfloat16_rn(o[v]);
+      for (int v = 0; v < VEC; ++v) {
+        const int c = c0 + v;
+        if (c < C) {
+          float g = load_dy(dy, dy_f32, dy_row<DYM>(u, ldy, pool ? H >> 1 : H, pool ? W >> 1 : W, C) + c);
+          if (leaky_on && !(zbest[v] > 0.0f)) g *= alpha;
+          d[v] = g;
+          gi[v] = gamma[c] * rsqrtf(var[c] + eps);
+          m1[v] = dbeta[c] * invM;
+          m2[v] = dgamma[c] * invM;
+        } else {
+          d[v] = 0.0f; gi[v] = 0.0f; m1[v] = 0.0f; m2[v] = 0.0f;
+        }
+      }
+      for (int k = 0; k < ur.n; ++k) {
+        float o[VEC];
+#pragma unroll
+        for (int v = 0; v < VEC; ++v) o[v] = gi[v] * ((arg[v] == k ? d[v] : 0.0f) - m1[v] - xh[k][v] * m2[v]);
+        __nv_bfloat16* po = dh + ur.r[k] * ld_dh + c0;
+        if (VEC == 4) {
+          __nv_bfloat162 a = __floats2bfloat162_rn(o[0], o[1 % VEC]);
+          __nv_bfloat162 b = __floats2bfloat162_rn(o[2 % VEC], o[3 % VEC]);
+          uint2 pk;
+          pk.x = *reinterpret_cast<uint32_t*>(&a);
+          pk.y = *reinterpret_cast<uint32_t*>(&b);
+          *reinterpret_cast<uint2*>(po) = pk;
+        } else {
+#pragma unroll
+          for (int v = 0; v < VEC; ++v) po[v] = __float2bfloat16_rn(o[v]);
+        }
       }
     }
   }
+}
+template <int VEC>
+__global__ void bn_bwd_apply_kernel(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32,
+                                    const float* __restrict__ mean, const float* __restrict__ var,
+                                    const float* __restrict__ gamma, const float* __restrict__ beta,
+                                    const float* __restrict__ dgamma, const float* __restrict__ dbeta, float eps,
+                                    float alpha, int leaky_on, int pool, int H, int W, int C, size_t units, float invM,
+                                    __nv_bfloat16* __restrict__ dh, int ld_dh) {
+  bn_bwd_apply_body<VEC, DY_DENSE, false>(h, ldh, dy, dy_f32, C, nullptr, mean, var, gamma, beta, dgamma, dbeta, eps, alpha,
+                                          leaky_on, pool, H, W, C, units, invM, dh, ld_dh);
+}
+template <int VEC, int DYM, bool ADD>
+__global__ void bn_bwd_apply_ex_kernel(const float* __restrict__ h, int ldh, const void* __restrict__ dy, int dy_f32, int ldy,
+                                       const __nv_bfloat16* __restrict__ dy_add, const float* __restrict__ mean,
+                                       const float* __restrict__ var, const float* __restrict__ gamma,
+                                       const float* __restrict__ beta, const float* __restrict__ dgamma,
+                                       const float* __restrict__ dbeta, float eps, float alpha, int leaky_on, int pool, int H,
+                                       int W, int C, size_t units, float invM, __nv_bfloat16* __restrict__ dh, int ld_dh) {
+  bn_bwd_apply_body<VEC, DYM, ADD>(h, ldh, dy, dy_f32, ldy, dy_add, mean, var, gamma, beta, dgamma, dbeta, eps, alpha, leaky_on,
+                                   pool, H, W, C, units, invM, dh, ld_dh);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -664,33 +876,19 @@ static int bwd_splits(size_t units) {
   return (int)(s > 1024 ? 1024 : (s < 1 ? 1 : s));
 }
 
-}  // namespace y2
-
-using namespace y2;
-
-extern "C" {
-
-size_t y2_bn_bwd_workspace_bytes(int M, int C) { return (size_t)bwd_splits((size_t)M) * C * 2 * sizeof(double); }
-
-int y2_bn_leaky_pool_bwd(const float* h_raw, int ldh, const void* dy, int dy_dtype, const float* mean, const float* var,
-                         const float* gamma, const float* beta, float eps, float alpha, int leaky_on, int pool, int N,
-                         int H, int W, int C, float* dgamma, float* dbeta, void* dh_bf16, int ld_dh, void* workspace,
-                         size_t workspace_bytes, y2_stream_t stream) {
-  Y2_ARG(h_raw && dy && mean && var && gamma && beta && dgamma && dbeta && dh_bf16);
-  Y2_ARG(N > 0 && H > 0 && W > 0 && C > 0 && ldh >= C && ld_dh >= C && (dy_dtype == 0 || dy_dtype == 1));
-  if (pool) Y2_ARG(H % 2 == 0 && W % 2 == 0);
-  const size_t M = (size_t)N * H * W;
-  const size_t units = pool ? M / 4 : M;
-  if (!workspace || workspace_bytes < y2_bn_bwd_workspace_bytes((int)M, C)) {
-    set_error("y2_bn_leaky_pool_bwd: workspace too small (%zu < %zu)", workspace_bytes, y2_bn_bwd_workspace_bytes((int)M, C));
-    return Y2_ERR_WORKSPACE;
-  }
-  Y2_ARG(((uintptr_t)workspace & 15) == 0);
+// The launches of y2_bn_leaky_pool_bwd_ex for one dy read mode (arguments checked by the caller).
+template <int DYM, bool ADD>
+static int bn_bwd_launch(const float* h_raw, int ldh, const void* dy, int dy_dtype, int ldy, const __nv_bfloat16* dy_add,
+                         const float* mean, const float* var, const float* gamma, const float* beta, float eps, float alpha,
+                         int leaky_on, int pool, int H, int W, int C, size_t M, size_t units, float* dgamma, float* dbeta,
+                         void* dh_bf16, int ld_dh, void* workspace, y2_stream_t stream) {
+  constexpr bool DENSE = DYM == DY_DENSE && !ADD;         // the mode of y2_bn_leaky_pool_bwd: its own kernels
   cudaStream_t st = (cudaStream_t)stream;
   int splits = bwd_splits(units);
   size_t ups = (units + splits - 1) / splits;
   splits = (int)((units + ups - 1) / ups);
-  if (C % 4 == 0 && ldh % 4 == 0 && (((uintptr_t)h_raw) & 15) == 0 && (((uintptr_t)dy) & 15) == 0) {
+  if (C % 4 == 0 && ldh % 4 == 0 && (((uintptr_t)h_raw) & 15) == 0 && (((uintptr_t)dy) & 15) == 0 && ldy % 4 == 0 &&
+      (((uintptr_t)dy_add) & 7) == 0) {
     const int cg = C / 4;
     {   // one wave of blocks (see bn_stats_impl); tiles are dealt round-robin, so any number of splits is balanced
       const int tx = cg <= 8 ? 8 : (cg <= 16 ? 16 : 32);
@@ -698,22 +896,42 @@ int y2_bn_leaky_pool_bwd(const float* h_raw, int ldh, const void* dy, int dy_dty
       if (splits > wave) splits = wave > 1 ? wave : 1;
     }
 #define Y2_LAUNCH_RED(POOL_, TX_)                                                                                     \
-  bn_bwd_reduce_v4_kernel<POOL_, TX_><<<dim3((cg + TX_ - 1) / TX_, splits), 256, 0, st>>>(                            \
-      h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on, H, W, C, units, ups, (double*)workspace)
-    if (pool) { if (cg <= 8) Y2_LAUNCH_RED(true, 8); else if (cg <= 16) Y2_LAUNCH_RED(true, 16); else Y2_LAUNCH_RED(true, 32); }
-    else      { if (cg <= 8) Y2_LAUNCH_RED(false, 8); else if (cg <= 16) Y2_LAUNCH_RED(false, 16); else Y2_LAUNCH_RED(false, 32); }
+  if constexpr (DENSE)                                                                                                \
+    bn_bwd_reduce_v4_kernel<POOL_, TX_><<<dim3((cg + TX_ - 1) / TX_, splits), 256, 0, st>>>(                          \
+        h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on, H, W, C, units, ups, (double*)workspace); \
+  else                                                                                                                \
+    bn_bwd_reduce_v4_ex_kernel<POOL_, TX_, DYM, ADD><<<dim3((cg + TX_ - 1) / TX_, splits), 256, 0, st>>>(             \
+        h_raw, ldh, dy, dy_dtype == 0, ldy, dy_add, mean, var, gamma, beta, eps, alpha, leaky_on, H, W, C, units, ups,        \
+        (double*)workspace)
+    if (pool) { if (cg <= 8) { Y2_LAUNCH_RED(true, 8); } else if (cg <= 16) { Y2_LAUNCH_RED(true, 16); } else { Y2_LAUNCH_RED(true, 32); } }
+    else      { if (cg <= 8) { Y2_LAUNCH_RED(false, 8); } else if (cg <= 16) { Y2_LAUNCH_RED(false, 16); } else { Y2_LAUNCH_RED(false, 32); } }
 #undef Y2_LAUNCH_RED
   } else {
     dim3 grid((C + 31) / 32, splits), block(32, 8);
-    bn_bwd_reduce_kernel<<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on,
-                                                 pool, H, W, C, units, ups, (double*)workspace);
+    if constexpr (DENSE)
+      bn_bwd_reduce_kernel<<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, eps, alpha, leaky_on,
+                                                   pool, H, W, C, units, ups, (double*)workspace);
+    else
+      bn_bwd_reduce_ex_kernel<DYM, ADD><<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, ldy, dy_add, mean, var, gamma,
+                                                                beta, eps, alpha, leaky_on, pool, H, W, C, units, ups,
+                                                                (double*)workspace);
   }
   Y2_LAUNCHED();
   bn_bwd_final_kernel<<<(C + 31) / 32, dim3(32, BWD_FIN_TY), 0, st>>>((const double*)workspace, splits, C, dgamma, dbeta);
   Y2_LAUNCHED();
   const bool vec4 = (ld_dh % 4 == 0) && (ldh % 4 == 0) && (((uintptr_t)h_raw & 15) == 0) && (((uintptr_t)dh_bf16 & 7) == 0);
   const float invM = 1.0f / (float)M;
-  if (vec4 && C % 4 == 0 && units < (1ull << 31) && (((uintptr_t)dy) & 15) == 0 && !env().bn_bwd_generic) {
+#define Y2_LAUNCH_APPLY(VEC_)                                                                                         \
+  if constexpr (DENSE)                                                                                                \
+    bn_bwd_apply_kernel<VEC_><<<(int)g, 256, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, dgamma, dbeta, \
+                                                      eps, alpha, leaky_on, pool, H, W, C, units, invM,                     \
+                                                      (__nv_bfloat16*)dh_bf16, ld_dh);                                      \
+  else                                                                                                                \
+    bn_bwd_apply_ex_kernel<VEC_, DYM, ADD><<<(int)g, 256, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, ldy, dy_add, mean, var,   \
+                                                                   gamma, beta, dgamma, dbeta, eps, alpha, leaky_on, pool,  \
+                                                                   H, W, C, units, invM, (__nv_bfloat16*)dh_bf16, ld_dh)
+  if (vec4 && C % 4 == 0 && units < (1ull << 31) && (((uintptr_t)dy) & 15) == 0 && ldy % 4 == 0 &&
+      (((uintptr_t)dy_add) & 7) == 0 && !env().bn_bwd_generic) {
     const int cg = ld_dh / 4;
     const int bx = cg >= 64 ? 64 : (cg >= 32 ? 32 : (cg >= 16 ? 16 : 8));        // channel-group lanes per block
     const int by = 256 / bx;
@@ -722,27 +940,81 @@ int y2_bn_leaky_pool_bwd(const float* h_raw, int ldh, const void* dy, int dy_dty
     if (gx > need) gx = need;
     if (gx < 1) gx = 1;
     const dim3 grid((unsigned)gx, (unsigned)((cg + bx - 1) / bx)), block(bx, by);
-    if (pool)
-      bn_bwd_apply_rows_kernel<true><<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, dgamma, dbeta, eps,
-                                                             alpha, leaky_on, H, W, C, (unsigned)units, invM, (__nv_bfloat16*)dh_bf16, ld_dh);
-    else
-      bn_bwd_apply_rows_kernel<false><<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, dgamma, dbeta, eps,
-                                                              alpha, leaky_on, H, W, C, (unsigned)units, invM, (__nv_bfloat16*)dh_bf16, ld_dh);
+#define Y2_LAUNCH_ROWS(POOL_)                                                                                         \
+  if constexpr (DENSE)                                                                                                \
+    bn_bwd_apply_rows_kernel<POOL_><<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, dgamma,   \
+                                                            dbeta, eps, alpha, leaky_on, H, W, C, (unsigned)units, invM,    \
+                                                            (__nv_bfloat16*)dh_bf16, ld_dh);                                \
+  else                                                                                                                \
+    bn_bwd_apply_rows_ex_kernel<POOL_, DYM, ADD><<<grid, block, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, ldy, dy_add, mean,   \
+                                                                         var, gamma, beta, dgamma, dbeta, eps, alpha,       \
+                                                                         leaky_on, H, W, C, (unsigned)units, invM,          \
+                                                                         (__nv_bfloat16*)dh_bf16, ld_dh)
+    if (pool) {
+      Y2_LAUNCH_ROWS(true);
+    } else {
+      Y2_LAUNCH_ROWS(false);
+    }
+#undef Y2_LAUNCH_ROWS
   } else if (vec4) {
     size_t total = units * (ld_dh / 4);
     size_t g = (total + 255) / 256;
     if (g > 148 * 32) g = 148 * 32;
-    bn_bwd_apply_kernel<4><<<(int)g, 256, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, dgamma, dbeta, eps,
-                                                   alpha, leaky_on, pool, H, W, C, units, invM, (__nv_bfloat16*)dh_bf16, ld_dh);
+    Y2_LAUNCH_APPLY(4);
   } else {
     size_t total = units * ld_dh;
     size_t g = (total + 255) / 256;
     if (g > 148 * 32) g = 148 * 32;
-    bn_bwd_apply_kernel<1><<<(int)g, 256, 0, st>>>(h_raw, ldh, dy, dy_dtype == 0, mean, var, gamma, beta, dgamma, dbeta, eps,
-                                                   alpha, leaky_on, pool, H, W, C, units, invM, (__nv_bfloat16*)dh_bf16, ld_dh);
+    Y2_LAUNCH_APPLY(1);
   }
+#undef Y2_LAUNCH_APPLY
   Y2_LAUNCHED();
   return Y2_OK;
+}
+
+}  // namespace y2
+
+using namespace y2;
+
+extern "C" {
+
+size_t y2_bn_bwd_workspace_bytes(int M, int C) { return (size_t)bwd_splits((size_t)M) * C * 2 * sizeof(double); }
+
+int y2_bn_leaky_pool_bwd_ex(const float* h_raw, int ldh, const void* dy, int dy_dtype, int ldy, int dy_s2d,
+                            const void* dy_add, const float* mean, const float* var, const float* gamma, const float* beta,
+                            float eps, float alpha, int leaky_on, int pool, int N, int H, int W, int C, float* dgamma,
+                            float* dbeta, void* dh_bf16, int ld_dh, void* workspace, size_t workspace_bytes,
+                            y2_stream_t stream) {
+  Y2_ARG(h_raw && dy && mean && var && gamma && beta && dgamma && dbeta && dh_bf16);
+  Y2_ARG(N > 0 && H > 0 && W > 0 && C > 0 && ldh >= C && ld_dh >= C && (dy_dtype == 0 || dy_dtype == 1));
+  if (pool) Y2_ARG(H % 2 == 0 && W % 2 == 0);
+  Y2_ARG(ldy >= (dy_s2d ? 4 * C : C));
+  if (dy_s2d) Y2_ARG(!pool && H % 2 == 0 && W % 2 == 0);
+  if (dy_add) Y2_ARG(pool);
+  const size_t M = (size_t)N * H * W;
+  const size_t units = pool ? M / 4 : M;
+  if (!workspace || workspace_bytes < y2_bn_bwd_workspace_bytes((int)M, C)) {
+    set_error("y2_bn_leaky_pool_bwd: workspace too small (%zu < %zu)", workspace_bytes, y2_bn_bwd_workspace_bytes((int)M, C));
+    return Y2_ERR_WORKSPACE;
+  }
+  Y2_ARG(((uintptr_t)workspace & 15) == 0);
+  const __nv_bfloat16* add = (const __nv_bfloat16*)dy_add;
+#define Y2_BN_BWD(DYM_, ADD_)                                                                                          \
+  return bn_bwd_launch<DYM_, ADD_>(h_raw, ldh, dy, dy_dtype, ldy, add, mean, var, gamma, beta, eps, alpha, leaky_on, pool, H, \
+                                   W, C, M, units, dgamma, dbeta, dh_bf16, ld_dh, workspace, stream)
+  if (dy_s2d) Y2_BN_BWD(DY_S2D, false);
+  if (add) { if (ldy == C) Y2_BN_BWD(DY_DENSE, true); else Y2_BN_BWD(DY_ROWS, true); }
+  if (ldy == C) Y2_BN_BWD(DY_DENSE, false);
+  Y2_BN_BWD(DY_ROWS, false);
+#undef Y2_BN_BWD
+}
+
+int y2_bn_leaky_pool_bwd(const float* h_raw, int ldh, const void* dy, int dy_dtype, const float* mean, const float* var,
+                         const float* gamma, const float* beta, float eps, float alpha, int leaky_on, int pool, int N,
+                         int H, int W, int C, float* dgamma, float* dbeta, void* dh_bf16, int ld_dh, void* workspace,
+                         size_t workspace_bytes, y2_stream_t stream) {
+  return y2_bn_leaky_pool_bwd_ex(h_raw, ldh, dy, dy_dtype, C, 0, nullptr, mean, var, gamma, beta, eps, alpha, leaky_on, pool,
+                                 N, H, W, C, dgamma, dbeta, dh_bf16, ld_dh, workspace, workspace_bytes, stream);
 }
 
 size_t y2_conv_packed_weight_dgrad_elems(int ksize, int Cin, int ld_dh) {

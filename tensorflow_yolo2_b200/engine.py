@@ -19,7 +19,7 @@ import torch
 from . import ops
 from .variables import VariableStore
 from .yolo2_nets.darknet import (CORE_PLAN, PASSTHROUGH_FILTERS, PASSTHROUGH_LAYER, classifier_plan, conv_bn_tc,
-                                  head_plan, raw_ld)
+                                  head_plan, layer_route, raw_ld)
 from .yolo2_nets.net_utils import VOC_ANCHORS
 
 
@@ -194,24 +194,18 @@ class Yolo2Engine:
         for li, L in enumerate(self.layers):
             training = self.head_training if L['head'] else self.core_training
             out = self.acts[li]
-            role = L.get('role')
-            pt_source = self.passthrough and li == PASSTHROUGH_LAYER      # un-pooled output wanted too
             if li == 0 and self.fused_conv1:
                 ops.conv1_u8_pool(self.in_u8, self.packed_c1, self.fold[0][1], out=out, split=self.x3)
             else:
-                # where the layer's activation goes: dense, or a channel slice of the concat buffer
-                ldo, col, s2d = None, 0, False
-                if self.passthrough and role == 'conv2':
-                    ldo = out.shape[-1]
-                elif role == 'passthrough':
-                    x, ldo, col, s2d = self.pt_src, out.shape[-1], 1024, True
+                # where the layer reads and writes: dense, a channel slice of the concat buffer, or un-pooled to pt_src
+                r = layer_route(L, li, x, out, self.pt_src)
                 bn = L['bn']
-                conv_bn_tc(x, self.packed[li], L['k'], L['cin'], L['cout'], fold=None if training else self.fold[li],
+                conv_bn_tc(r['x'], self.packed[li], L['k'], L['cin'], L['cout'], fold=None if training else self.fold[li],
                            bias=st[L['b']], gamma=st[bn['gamma']], beta=st[bn['beta']], stats=self.stats.get(li),
-                           workspace=self.ws, pool=L['pool'] and not pt_source, out_f32=li == nl - 1,
-                           out=self.pt_src if pt_source else out, ldo=ldo, col=col, s2d=s2d, x3=self.x3, raw=self.raw.get(li))
-            if pt_source:
-                ops.maxpool2x2_bf16(self.pt_src, out=self.acts[li])
+                           workspace=self.ws, pool=r['pool'], out_f32=li == nl - 1, out=r['out'], ldo=r['ldo'], col=r['col'],
+                           s2d=r['s2d'], x3=self.x3, raw=self.raw.get(li))
+                if r['pooled'] is not None:
+                    ops.maxpool2x2_bf16(self.pt_src, out=r['pooled'])
             x = self.acts[li]
         if self.decode == 'region':
             if self.C == 20 and self.nbox <= 4095 and self.fused_detect:

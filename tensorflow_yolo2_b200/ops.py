@@ -578,9 +578,15 @@ def bn_bwd_workspace_bytes(M, C_):
 
 
 def bn_leaky_pool_bwd(h_raw, dy, mean, var, gamma, beta, N, H, W, C_, ldh=None, leaky=True, pool=False, ld_dh=None,
-                      dgamma=None, dbeta=None, dh=None, workspace=None, alpha=ALPHA, eps=BN_EPS):
+                      dgamma=None, dbeta=None, dh=None, workspace=None, alpha=ALPHA, eps=BN_EPS, ldy=None, dy_col=0,
+                      dy_s2d=False, dy_add=None):
     """Backward of max_pool(leaky(batch_norm(h_raw))) (batch statistics).  dy: grad of the layer output
-    [N,Ho,Wo,C] (f32 or bf16).  Returns (dgamma[C], dbeta[C], dh bf16 [N*H*W, ld_dh])."""
+    [N,Ho,Wo,C] (f32 or bf16).  Returns (dgamma[C], dbeta[C], dh bf16 [N*H*W, ld_dh]).
+
+    The defaults read dy as dense [N,Ho,Wo,C] rows.  Otherwise (y2_bn_leaky_pool_bwd_ex): dy is a wider tensor whose rows
+    of stride `ldy` hold the layer's gradient from column `dy_col` on; dy_s2d=True reads it through depth_to_space(2)
+    (the layer's output was stored space_to_depth(2) there: the passthrough branch); dy_add (bf16 [N,H,W,C], pooled layers)
+    is the gradient of the un-pooled output from a second consumer, added to every input row before the leaky slope."""
     ldh = ldh or C_
     ld_dh = ld_dh or (C_ + 63) // 64 * 64
     dev = h_raw.device
@@ -597,11 +603,17 @@ def bn_leaky_pool_bwd(h_raw, dy, mean, var, gamma, beta, N, H, W, C_, ldh=None, 
     lib = _lib.load()
     need = int(lib.y2_bn_bwd_workspace_bytes(M, C_))
     ws = workspace if workspace is not None else _workspace(need, dev)
-    check(lib.y2_bn_leaky_pool_bwd(_p(h_raw, torch.float32), ldh, _p(dy), 0 if dy.dtype == torch.float32 else 1,
-                                   _p(mean, torch.float32), _p(var, torch.float32), _p(gamma, torch.float32),
-                                   _p(beta, torch.float32), eps, alpha, 1 if leaky else 0, 1 if pool else 0, N, H, W, C_,
-                                   _p(dgamma, torch.float32), _p(dbeta, torch.float32), _p(dh, torch.bfloat16), ld_dh,
-                                   _p(ws), ws.numel(), _stream()), 'y2_bn_leaky_pool_bwd')
+    args = (_p(mean, torch.float32), _p(var, torch.float32), _p(gamma, torch.float32), _p(beta, torch.float32), eps, alpha,
+            1 if leaky else 0, 1 if pool else 0, N, H, W, C_, _p(dgamma, torch.float32), _p(dbeta, torch.float32),
+            _p(dh, torch.bfloat16), ld_dh, _p(ws), ws.numel(), _stream())
+    dy_code = 0 if dy.dtype == torch.float32 else 1
+    if ldy is None and not dy_col and not dy_s2d and dy_add is None:
+        check(lib.y2_bn_leaky_pool_bwd(_p(h_raw, torch.float32), ldh, _p(dy), dy_code, *args), 'y2_bn_leaky_pool_bwd')
+    else:
+        ldy = ldy or dy.shape[-1]
+        assert dy.numel() % ldy == 0 and (dy_add is None or dy_add.numel() == M * C_)
+        check(lib.y2_bn_leaky_pool_bwd_ex(_p(h_raw, torch.float32), ldh, _p_off(dy, dy_col), dy_code, int(ldy),
+                                          1 if dy_s2d else 0, _p(dy_add, torch.bfloat16), *args), 'y2_bn_leaky_pool_bwd_ex')
     return dgamma, dbeta, dh
 
 

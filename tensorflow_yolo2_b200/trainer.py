@@ -22,6 +22,10 @@ contiguous slice that becomes ready early); the VariableStore entries are views 
 checkpoints (net_utils.save_checkpoint) see the live weights under their TF names.
 The conv bias sits in front of a batch-statistics BN, so its gradient is identically zero (TF computes rounding
 noise there); it is left at exactly 0.
+
+Yolo2Trainer(passthrough=True) trains the YOLOv2 graph instead (23 layers, the passthrough conv between conv2 and conv3, see
+the constructor): the forward pass routes every layer through darknet.layer_route, as Yolo2Engine does, and the backward pass
+reads each layer's incoming gradient where its consumer wrote it (dy_src).
 """
 from __future__ import annotations
 
@@ -32,7 +36,7 @@ from . import ops
 from .engine import create_classifier_variables, create_variables
 from .parallel import BucketedAllReduce, bucket_segments, make_buckets
 from .variables import VariableStore
-from .yolo2_nets.darknet import conv_bn_tc, raw_ld
+from .yolo2_nets.darknet import PASSTHROUGH_FILTERS, PASSTHROUGH_LAYER, conv_bn_tc, layer_route, raw_ld
 from .yolo2_nets.net_utils import VOC_ANCHORS
 
 
@@ -44,11 +48,19 @@ class Yolo2Trainer:
     def __init__(self, batch, image_size=416, output_filter=None, store=None, loss='v1', num_class=20, B=5,
                  anchors=VOC_ANCHORS, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, lambda_coord=None, lambda_noobj=None,
                  max_gt=32, device=None, seed=0, process_group=None, bucket_bytes=48 << 20, update_moving=True,
-                 use_cuda_graph=False, optimizer='adam', momentum=0.9):
+                 use_cuda_graph=False, optimizer='adam', momentum=0.9, passthrough=False):
         """loss: 'v1' (the reference's get_loss), 'region' (YOLOv2 region loss) or 'softmax' -- the ImageNet classifier of
         imagenet_train_darknet.py:46-58: the 18 core layers + the 1x1 conv to `num_class` logits maps + 7x7 average pool,
         sparse softmax cross-entropy (image_size 224, num_class 1000 there).  optimizer: 'adam' (pascal_train_darknet.py:51)
-        or 'momentum' (tf.train.MomentumOptimizer(lr, momentum), imagenet_train_darknet.py:58)."""
+        or 'momentum' (tf.train.MomentumOptimizer(lr, momentum), imagenet_train_darknet.py:58).
+
+        passthrough=True trains the YOLOv2 graph of head_plan(OF, 64) (23 layers; the detection losses only): the un-pooled
+        output of layer 13 goes through a 1x1 conv (512 -> 64) whose space_to_depth(2) fills channels [1024, 1280) of a
+        [N,S,S,1280] concat after conv2's 1024, and conv3 reads all 1280 -- the graph Yolo2Engine(passthrough=True) serves,
+        under the same variable names.  Backward: conv3's data gradient is the [N,S,S,1280] concat gradient; conv2 reads its
+        first 1024 columns in place (row stride 1280), the passthrough conv the last 256 through depth_to_space(2); the
+        passthrough conv's data gradient (the un-pooled [N,2S,2S,512] `d_pt`) is added to every pre-pool row of layer 13
+        inside its batch-norm backward, next to the pooled gradient of layer 14."""
         self.device = torch.device(device) if device is not None else torch.device('cuda', torch.cuda.current_device())
         self.N, self.IS = int(batch), int(image_size)
         assert self.IS % 32 == 0
@@ -71,6 +83,9 @@ class Yolo2Trainer:
             of = self.C
         else:
             raise ValueError('loss must be "v1", "region" or "softmax"')
+        if passthrough and loss == 'softmax':
+            raise ValueError('passthrough=True is the YOLOv2 detection graph: use loss="region" or "v1"')
+        self.passthrough = bool(passthrough)
         if optimizer not in ('adam', 'momentum'):
             raise ValueError('optimizer must be "adam" or "momentum"')
         self.optimizer, self.momentum = optimizer, float(momentum)
@@ -84,7 +99,7 @@ class Yolo2Trainer:
         self.update_moving = update_moving
         self.store = store if store is not None else VariableStore(seed=seed)
         self.layers = (create_classifier_variables(self.store, self.OF) if loss == 'softmax'
-                       else create_variables(self.store, self.OF))
+                       else create_variables(self.store, self.OF, passthrough=self.passthrough))
         self.iteration = 0
         # the whole step (forward, loss, backward, Adam: ~245 launches) replayed as ONE CUDA graph.  With world > 1 the NCCL
         # buckets stay eager launches on NCCL's stream (capturing them too dead-locked in a 2-GPU trial) and the step is cut
@@ -154,24 +169,36 @@ class Yolo2Trainer:
         self.x0 = torch.empty((N, IS, IS, 8), **bf16)
         self.acts, self.raw, self.stats, self.geom = [], [], [], []
         self.packed, self.packed_dgrad = [], []
+        self.pt_src = self.d_cat = self.d_pt = None
         H = IS
         max_ws, max_dh, max_dx = 1, 1, 1
         nl = len(self.layers)
         for li, L in enumerate(self.layers):
+            role = L.get('role')
             Ho = H // 2 if L['pool'] else H
+            Hc = 2 * H if role == 'passthrough' else H          # the map the conv runs on: the passthrough conv's is 2S x 2S
             last = li == nl - 1
             cout, cin, k = L['cout'], L['cin'], L['k']
             ldh = raw_ld(cout)
             ld_dh = 32 if li == 0 else _round_up(cout, 64)
-            self.geom.append(dict(H=H, Ho=Ho, ldh=ldh, ld_dh=ld_dh, M=N * H * H))
-            self.acts.append(torch.empty((N, Ho, Ho, cout), **(f32 if last else bf16)))
-            self.raw.append(torch.empty((N * H * H, ldh), **f32))
+            self.geom.append(dict(H=Hc, Ho=Ho if role != 'passthrough' else Hc, ldh=ldh, ld_dh=ld_dh, M=N * Hc * Hc))
+            if self.passthrough and role == 'conv2':
+                # conv2's 1024 channels and the passthrough branch's 4 * 64 share one [N,S,S,1280] activation (conv3's input)
+                self.acts.append(torch.empty((N, Ho, Ho, cout + 4 * PASSTHROUGH_FILTERS), **bf16))
+            elif role == 'passthrough':
+                self.acts.append(self.acts[-1])
+            else:
+                self.acts.append(torch.empty((N, Ho, Ho, cout), **(f32 if last else bf16)))
+            if self.passthrough and li == PASSTHROUGH_LAYER:
+                self.pt_src = torch.empty((N, H, H, cout), **bf16)             # layer 13 before its pool
+                self.d_pt = torch.empty((N, H, H, cout), **bf16)               # its gradient from the passthrough conv
+            self.raw.append(torch.empty((N * Hc * Hc, ldh), **f32))
             self.stats.append(dict(mean=torch.empty((cout,), **f32), var=torch.empty((cout,), **f32),
                                    scale=torch.empty((cout,), **f32), shift=torch.empty((cout,), **f32)))
-            max_ws = max(max_ws, ops.bn_stats_workspace_bytes(N * H * H, cout), ops.bn_bwd_workspace_bytes(N * H * H, cout))
-            max_dh = max(max_dh, N * H * H * ld_dh)
-            if li > 0:
-                max_dx = max(max_dx, N * H * H * cin)
+            max_ws = max(max_ws, ops.bn_stats_workspace_bytes(N * Hc * Hc, cout), ops.bn_bwd_workspace_bytes(N * Hc * Hc, cout))
+            max_dh = max(max_dh, N * Hc * Hc * ld_dh)
+            if li > 0 and not (self.passthrough and role in ('passthrough', 'conv3')):      # (those two: d_pt, d_cat)
+                max_dx = max(max_dx, N * Hc * Hc * cin)
             self.packed.append(torch.empty((int(ops._lib.load().y2_conv_packed_weight_elems(k, cin, cout)),), **bf16))
             self.packed_dgrad.append(None if li == 0 else torch.empty(
                 (int(ops._lib.load().y2_conv_packed_weight_dgrad_elems(k, cin, ld_dh)),), **bf16))
@@ -180,6 +207,8 @@ class Yolo2Trainer:
         self.conv_ws = ops.new_conv_workspace(dev)          # this trainer's own stream-K scratch (see ops.conv_workspace_scope)
         self.dh = torch.empty((max_dh,), **bf16)
         self.dx = [torch.empty((max_dx,), **bf16), torch.empty((max_dx,), **bf16)]
+        if self.passthrough:
+            self.d_cat = torch.empty(tuple(self.acts[self._index('conv3') - 1].shape), **bf16)     # conv3's data gradient
         S = self.S
         self.terms = torch.zeros((2 if self.loss_kind == 'softmax' else 5,), **f32)
         self.lr_dev = torch.zeros((1,), **f32)              # Adam step size of the current iteration (read by the update kernel)
@@ -199,6 +228,34 @@ class Yolo2Trainer:
             self.gt_boxes = torch.zeros((N, self.max_gt, 4), **f32)
             self.gt_classes = torch.zeros((N, self.max_gt), dtype=torch.int32, device=dev)
             self.gt_counts = torch.zeros((N,), dtype=torch.int32, device=dev)
+        self._build_gradient_routes()
+
+    def _index(self, role):
+        return next(li for li, L in enumerate(self.layers) if L.get('role') == role)
+
+    def _build_gradient_routes(self):
+        """Per layer: where its data gradient goes (dx_out) and where the gradient of its output is read (dy_src: the
+        consumer's data gradient as (tensor, ldy, column, depth_to_space, un-pooled addend), or the loss gradient).  In the
+        chain, layer li writes the ping-pong buffer dx[li & 1] and layer li - 1 reads it; the passthrough graph adds the
+        concat gradient d_cat (conv3 -> conv2 and the passthrough conv) and d_pt (passthrough conv -> layer 13)."""
+        N, nl = self.N, len(self.layers)
+        self.dx_out, self.dy_src = [None] * nl, [None] * nl
+        for li in range(1, nl):
+            g, L = self.geom[li], self.layers[li]
+            if self.passthrough and L.get('role') in ('passthrough', 'conv3'):
+                self.dx_out[li] = self.d_pt if L['role'] == 'passthrough' else self.d_cat
+            else:
+                self.dx_out[li] = self.dx[li & 1][:g['M'] * L['cin']].view(N, g['H'], g['H'], L['cin'])
+        for li in range(nl - 1):
+            self.dy_src[li] = dict(t=self.dx_out[li + 1], ldy=None, col=0, s2d=False, add=None)
+        self.dy_src[nl - 1] = dict(t=self.dnet, ldy=None, col=0, s2d=False, add=None)
+        if not self.passthrough:
+            return
+        i2, ip = self._index('conv2'), self._index('passthrough')
+        ldc = self.d_cat.shape[-1]
+        self.dy_src[i2] = dict(t=self.d_cat, ldy=ldc, col=0, s2d=False, add=None)
+        self.dy_src[ip] = dict(t=self.d_cat, ldy=ldc, col=ldc - 4 * self.layers[ip]['cout'], s2d=True, add=None)
+        self.dy_src[PASSTHROUGH_LAYER]['add'] = self.d_pt
 
     def _build_buckets(self, bucket_bytes):
         """Contiguous arena slices in backward order; a bucket is launched once its last layer's gradients are enqueued."""
@@ -236,9 +293,13 @@ class Yolo2Trainer:
             s, P, bn = self.stats[li], self.P[li], L['bn']
             ops.pack_weights_bf16(P['W'], out=self.packed[li])
             moving = (self.store[bn['moving_mean']], self.store[bn['moving_variance']]) if self.update_moving else None
-            x = conv_bn_tc(x, self.packed[li], L['k'], L['cin'], L['cout'], bias=P['b'], gamma=P['gamma'], beta=P['beta'],
-                           moving=moving, stats=(s['mean'], s['var'], s['scale'], s['shift']), workspace=self.ws,
-                           pool=L['pool'], out_f32=li == nl - 1, out=self.acts[li], raw=self.raw[li])
+            r = layer_route(L, li, x, self.acts[li], self.pt_src)
+            conv_bn_tc(r['x'], self.packed[li], L['k'], L['cin'], L['cout'], bias=P['b'], gamma=P['gamma'], beta=P['beta'],
+                       moving=moving, stats=(s['mean'], s['var'], s['scale'], s['shift']), workspace=self.ws, pool=r['pool'],
+                       out_f32=li == nl - 1, out=r['out'], ldo=r['ldo'], col=r['col'], s2d=r['s2d'], raw=self.raw[li])
+            if r['pooled'] is not None:
+                ops.maxpool2x2_bf16(self.pt_src, out=r['pooled'])
+            x = self.acts[li]
         return self.acts[-1]
 
     def loss(self):
@@ -267,31 +328,45 @@ class Yolo2Trainer:
         self.reducer.finish(scale=False)            # sums; the 1/world of the mean is applied inside the update kernel
 
     def _dy_of(self, li):
-        """Gradient w.r.t. layer li's output: the loss gradient for the last layer, else the data gradient layer li + 1 wrote."""
-        if li == len(self.layers) - 1:
-            return self.dnet
-        g, L = self.geom[li + 1], self.layers[li + 1]
-        return self.dx[(li + 1) & 1][:g['M'] * L['cin']].view(self.N, g['H'], g['H'], L['cin'])
+        """Gradient w.r.t. layer li's output as a dense [N,Ho,Wo,C] tensor: the loss gradient for the last layer, else the
+        data gradient of its consumer -- for the passthrough graph's conv2 a view of the concat gradient's first 1024
+        columns, for the passthrough conv a depth_to_space copy of its last 256 (tests and tools; the backward pass reads
+        them in place).  Layer 13's second, un-pooled gradient (passthrough graph) is self.d_pt."""
+        d = self.dy_src[li]
+        L, t = self.layers[li], d['t']
+        c = L['cout']
+        if d['ldy'] is None:
+            return t
+        v = t[..., d['col']:d['col'] + (4 * c if d['s2d'] else c)]
+        if not d['s2d']:
+            return v
+        n, h, w, _ = v.shape                                    # depth_to_space(2): [N,S,S,4C] -> [N,2S,2S,C]
+        return v.reshape(n, h, w, 2, 2, c).permute(0, 1, 3, 2, 4, 5).reshape(n, 2 * h, 2 * w, c)
 
     def _backward_layer(self, li, capture=None):
         L, g, s, P, G = self.layers[li], self.geom[li], self.stats[li], self.P[li], self.G[li]
         H, M, cout, cin, k = g['H'], g['M'], L['cout'], L['cin'], L['k']
-        dy = self._dy_of(li)
+        d = self.dy_src[li]
         if capture is not None:
-            capture[li] = dy.clone()
+            capture[li] = self._dy_of(li).clone()
+            if d['add'] is not None:
+                capture['d_pt'] = d['add'].clone()
         dh = self.dh[:M * g['ld_dh']].view(M, g['ld_dh'])
-        ops.bn_leaky_pool_bwd(self.raw[li], dy, s['mean'], s['var'], P['gamma'], P['beta'], self.N, H, H, cout,
+        ops.bn_leaky_pool_bwd(self.raw[li], d['t'], s['mean'], s['var'], P['gamma'], P['beta'], self.N, H, H, cout,
                               ldh=g['ldh'], leaky=True, pool=L['pool'], ld_dh=g['ld_dh'], dgamma=G['gamma'],
-                              dbeta=G['beta'], dh=dh, workspace=self.ws)
-        xin = self.x0 if li == 0 else self.acts[li - 1]
+                              dbeta=G['beta'], dh=dh, workspace=self.ws, ldy=d['ldy'], dy_col=d['col'], dy_s2d=d['s2d'],
+                              dy_add=d['add'])
+        if L.get('role') == 'passthrough':
+            xin = self.pt_src
+        else:
+            xin = self.x0 if li == 0 else self.acts[li - 1]
         if li == 0:
             ops.conv_wgrad_c3(xin, dh, cout, G['W'])
         else:
             ops.conv_wgrad_bf16(xin, dh, k, cin, cout, G['W'])
             ops.pack_weights_dgrad_bf16(P['W'], g['ld_dh'], out=self.packed_dgrad[li])
-            dx = self.dx[li & 1][:M * cin].view(self.N, H, H, cin)
             ops.conv_fwd_bf16(dh.view(self.N, H, H, g['ld_dh']), self.packed_dgrad[li], k, g['ld_dh'], cin, scale=None,
-                              shift=None, leaky=False, pool=False, out=dx)
+                              shift=None, leaky=False, pool=False, out=self.dx_out[li])
 
     def _set_lr(self):
         """TF's bias-corrected step size of iteration self.iteration -> device scalar (a 4-byte async copy, outside the graph)."""

@@ -267,6 +267,28 @@ def conv_bn_tc(x, wp, k, cin, cout, fold=None, bias=None, gamma=None, beta=None,
                                  out_bf16=not out_f32, out=out, ldo=ldo, out_col=col, space_to_depth=s2d, split_out=x3)
 
 
+def layer_route(L, li, x, out, pt_src=None):
+    """Where layer li of create_variables' list reads and writes in the YOLOv2 graph -- the routing Yolo2Engine and
+    Yolo2Trainer share.  x: the previous layer's activation; out: this layer's activation buffer (for conv2 and the
+    passthrough conv: the [N,S,S,1280] concat buffer, which both fill); pt_src: the un-pooled bf16 [N,2S,2S,512] output of
+    layer PASSTHROUGH_LAYER when the passthrough branch is on, else None.
+
+    Returns dict(x, out, ldo, col, s2d, pool, pooled): conv_bn_tc's input, output and store address, and whether it pools.
+    `pooled` is None, or -- layer PASSTHROUGH_LAYER -- the buffer maxpool2x2_bf16(pt_src) must fill after the layer, because
+    conv_bn_tc then writes the un-pooled activation to pt_src."""
+    r = dict(x=x, out=out, ldo=None, col=0, s2d=False, pool=L['pool'], pooled=None)
+    if pt_src is None:
+        return r
+    role = L.get('role')
+    if li == PASSTHROUGH_LAYER:
+        r.update(out=pt_src, pool=False, pooled=out)
+    elif role == 'conv2':                            # channels [0, 1024) of the concat
+        r.update(ldo=out.shape[-1])
+    elif role == 'passthrough':                      # space_to_depth(2) into channels [1024, 1280) of the concat
+        r.update(x=pt_src, ldo=out.shape[-1], col=out.shape[-1] - 4 * L['cout'], s2d=True)
+    return r
+
+
 # ---------------------------------------------------------------------------------------------
 # builders (darknet.py:126-201)
 # ---------------------------------------------------------------------------------------------
